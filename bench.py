@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark: synthetic users / second through the FULL T-step reverse chain + VAE decode.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload cfg5] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload cfg5] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" is one sample_ddpm-equivalent pass over one batch of users (SURVEY.md §8d).  Default workload is the
 configuration BASELINE.json quotes its target on: the synthetic scale-up (T=178, VAE 1000/950, 4 hidden layers,
@@ -250,6 +250,25 @@ def run_reference(args, w, rank):
     emit(line)
 
 
+DUMP_BYTES = 60 << 20   # stays under 64 MB in either unit (10^6 or 2^20 bytes), .npy headers included
+
+
+def dump_outputs(path, out, rank, world, row_offset):
+    """Write what the last timed step returned, the float32 logits [n, I] of this rank, to `path` so that two builds can be
+    compared output for output: `logits.npy` holds whole rows (all of them when every rank's rows fit in DUMP_BYTES, else a
+    fixed seeded sample) and `logits_rows.npy` their global row ids; with several ranks each file gets a `_rank<r>` suffix."""
+    import numpy as np
+    import torch
+    n, I = out.shape
+    k = min(n, DUMP_BYTES // world // (4 * I + 8))
+    rows = np.sort(np.random.default_rng(0).choice(n, size=k, replace=False)) if k < n else np.arange(n)
+    logits = out.index_select(0, torch.from_numpy(rows).to(out.device)).cpu().numpy()
+    suffix = f"_rank{rank}" if world > 1 else ""
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, f"logits{suffix}.npy"), logits.astype(np.float32, copy=False))
+    np.save(os.path.join(path, f"logits_rows{suffix}.npy"), (rows + row_offset).astype(np.float64))
+
+
 def run_ours(args, w, rank, world, local_rank):
     import torch
     import torch.distributed as dist
@@ -308,6 +327,8 @@ def run_ours(args, w, rank, world, local_rank):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     total_ms = float(t.item())
     value = world * n * args.steps / (total_ms * 1e-3)
+    if args.dump_outputs:   # before the e2e leg below, which overwrites `out`
+        dump_outputs(args.dump_outputs, out, rank, world, row_offset)
 
     # ---- end to end through the public call with HOST buffers: every step uploads the trained weights from pinned host
     #      memory (the checkpoint a caller holds), re-packs them, samples, and delivers the rows into pinned host memory
@@ -644,7 +665,13 @@ def main():
     ap.add_argument("--eager-rows", type=int, default=None, help="--impl reference: rows of the eager-CUDA sample")
     ap.add_argument("--cluster", type=int, default=0, help="force single CTAs (1), tcgen05 CTA pairs (2) or column-split clusters (4, 8); 0 = auto")
     ap.add_argument("--subtiles", type=int, default=0, help="row tiles a CTA pair interleaves (1, 2); 0 = auto")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the logits of the last step (a fixed sample of rows, <= 64 MB) to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.mode != "sample"):
+        ap.error("--dump-outputs writes the output of the sampling path (--impl ours --mode sample)")
     w = WORKLOADS[args.workload]
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
