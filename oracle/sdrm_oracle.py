@@ -45,7 +45,7 @@ def timestep_embedding(t, dim):
     args = t[:, None].float() * freqs[None]
     emb = torch.cat([torch.cos(args), torch.sin(args)], dim=-1)
     if dim % 2:
-        emb = torch.cat([emb, torch.zeros_like(emb[:, :1])], dim=-1)
+        emb = torch.cat([emb, torch.zeros(emb.shape[0], 1, dtype=emb.dtype)], dim=-1)   # (dim = 1: emb has no column to copy)
     return emb
 
 

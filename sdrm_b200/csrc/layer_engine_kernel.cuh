@@ -929,6 +929,26 @@ __global__ void __launch_bounds__(ENGINE_THREADS, 1) sdrm_layer_engine_kernel(co
               }
             }
             xs_store16(xs, g, r, x);
+            if (T_tile == 0) {
+              // no reverse step in this tile (every row starts at t = 0): x_0 = x_T.  What the x_0 pass of the last posterior
+              // step would leave for the decoder: bf16 hi image in buffer 0 (the chain's last output when it ran no layer), lo
+              // image in buffer 2, and x0_out.  (T_tile is uniform over the CTA: the warp-collective stores stay converged.)
+              uint32_t ph[8], pl[8];
+#pragma unroll
+              for (int e = 0; e < 8; ++e) {
+                const float h0 = bf16_round(x[2 * e]), h1 = bf16_round(x[2 * e + 1]);
+                ph[e] = pack_bf16x2(h0, h1);
+                pl[e] = pack_bf16x2(x[2 * e] - h0, x[2 * e + 1] - h1);
+              }
+              store_act(in0_row, g * 16, ph);
+              store_act(sc + 2 * P.act_buf_bytes + row_off, g * 16, pl);
+              if (P.x0_out && valid) {
+#pragma unroll
+                for (int e = 0; e < 16; ++e)
+                  if (g * 16 + e < P.L) P.x0_out[static_cast<size_t>(row) * P.L + g * 16 + e] = x[e];
+              }
+              continue;
+            }
             // keep mask of the first step (the noise warps produce the masks of all later steps)
             uint32_t keep = 0;
             if (valid) {

@@ -58,7 +58,7 @@ class SDRM(nn.Module):
         args = timesteps[:, None].float() * freqs[None]
         emb = torch.cat([torch.cos(args), torch.sin(args)], dim=-1)
         if dim % 2:
-            emb = torch.cat([emb, torch.zeros_like(emb[:, :1])], dim=-1)
+            emb = torch.cat([emb, emb.new_zeros(emb.shape[0], 1)], dim=-1)   # (dim = 1: emb has no column to copy)
         return emb
 
     def forward(self, x, t, keep_mask=None, prescaled=False):

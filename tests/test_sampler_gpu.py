@@ -53,6 +53,10 @@ def test_golden_injected_noise(name, mode, engine):
     (1200, 8582, 40, 40, 16, 5, 1.0),     # cfg 3 adm
     (1208, 729, 550, 400, 43, 0, 0.2),    # cfg 4 alb, full T
     (300, 2000, 1000, 950, 6, 4, 1.0),    # cfg 5 layer shapes (I shortened)
+    (130, 500, 2048, 2048, 3, 1, 1.0),    # the widest latent, hidden and VAE hidden the library takes (8 x 256 columns)
+    (200, 1, 40, 65, 6, 1, 1.0),          # one column wider than the small-chain kernel takes; a single item
+    (300, 400, 100, 120, 1, 6, 0.0),      # K1: one step (no dropout mask or noise from the noise warps, no discard), nh = 6
+    (400, 150, 48, 40, 2, 6, 0.5),        # K6 (every width <= 64): two steps, nh = 6
 ])
 def test_vs_oracle_philox_noise(shape):
     """In-kernel Philox noise: the oracle is fed the numpy restatement of the same streams."""
@@ -130,6 +134,11 @@ def test_single_and_pair_mode_are_bit_identical():
     (2000, 729, 550, 400, 6, 0),     # cfg-4 widths: KB = 7 -> 2 stages left, no hidden layer
     (1000, 500, 300, 512, 5, 1),     # the widest denoiser the mode takes (2 x 256 columns, KB = 8)
     (700, 400, 200, 520, 4, 1),      # too wide (3 chunks): stays in streaming mode
+    (1000, 300, 200, 128, 5, 1),     # 128 columns: one tile per CTA streams; several tiles per CTA interleave (w = 128)
+    (1000, 300, 200, 129, 5, 1),     # one column more: KB = 3 (w = 192) -> resident with one tile per CTA
+    (1000, 300, 200, 256, 5, 1),     # one chunk of 256 columns (w = 256)
+    (1000, 300, 200, 257, 5, 1),     # two chunks of 144 columns, KB = 5 (w = 320: the widest that interleaves sub-tiles)
+    (700, 300, 200, 513, 4, 1),      # 3 chunks: streaming
 ])
 def test_resident_mode_is_bit_identical_to_streaming(shape):
     """Pair-mode launches of denoisers up to 512 wide keep the chain's activation tile in shared memory (resident mode), with
@@ -179,6 +188,8 @@ def test_resident_mode_is_bit_identical_to_streaming(shape):
     (6000, 300, 200, 600, 3, 1),     # 47 row tiles: only clusters of 2 fit (normal geometry, CTA j takes the chunks j and j + 2 of 3)
     (1500, 400, 128, 200, 7, 3),     # a single-chunk denoiser: 8 chunks of 32 columns
     (500, 300, 100, 72, 9, 1),       # 8 chunks of 16 columns (the narrowest UMMA)
+    (300, 700, 300, 2048, 3, 1),     # the widest denoiser: 8 chunks of 256 in either geometry (two per CTA on 4 CTAs)
+    (500, 10, 100, 65, 5, 1),        # one chunk of 80 -> 8 of 16; fewer items than one 16-column logits chunk
 ])
 def test_column_split_mode_is_bit_identical_to_streaming(shape):
     """Full-resolution launches of a few row tiles of a wide denoiser (>= 3 N chunks per chain layer) split every tile's chunks over

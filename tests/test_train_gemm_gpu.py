@@ -112,11 +112,18 @@ def test_denoiser_fwd_bwd_matches_autograd_linear_slopes(L, T, nh, B):
     assert not bad, (bad, mx)
 
 
-@pytest.mark.parametrize("L,T,nh,B", [(20, 6, 0, 5), (24, 7, 2, 12), (40, 9, 5, 30)])
-def test_denoiser_fwd_bwd_matches_autograd_small(L, T, nh, B):
+@pytest.mark.parametrize("L,T,nh,B,slopes", [
+    pytest.param(20, 6, 0, 5, (0.21, 0.33), id="20-6-0-5"),
+    pytest.param(24, 7, 2, 12, (0.21, 0.33), id="24-7-2-12"),
+    pytest.param(40, 9, 5, 30, (0.21, 0.33), id="40-9-5-30"),
+    pytest.param(20, 6, 0, 5, (-0.5, 1.5), id="20-6-0-5-slopes-0.5,1.5"),    # slopes outside [0, 1] (trained slopes can leave it)
+    pytest.param(24, 7, 2, 12, (-0.5, 1.5), id="24-7-2-12-slopes-0.5,1.5"),
+    pytest.param(40, 9, 5, 30, (-0.5, 1.5), id="40-9-5-30-slopes-0.5,1.5"),
+])
+def test_denoiser_fwd_bwd_matches_autograd_small(L, T, nh, B, slopes):
     """Real slopes at small shapes (a pre-activation within rounding distance of 0 -- where fp32-grade and float64 arithmetic
     legitimately pick different sides of the PReLU kink -- is improbable among a few thousand entries): 2e-4 of max|grad|."""
-    mx, _ = _fwd_bwd_report(L, T, nh, B, (0.21, 0.33))
+    mx, _ = _fwd_bwd_report(L, T, nh, B, slopes)
     bad = {k: v for k, v in mx.items() if v > 2e-4}
     assert not bad, (bad, mx)
 
