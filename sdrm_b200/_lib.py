@@ -22,6 +22,8 @@ SIGNATURES = {
     "sdrm_sample_workspace_bytes": (C.c_size_t, [_P, C.c_int64]),
     "sdrm_sample": (C.c_int, [_P, C.c_int64, C.c_int64, _P, _P, C.c_uint64, _P, _P, C.c_int64, _P, _P, _P, _P,
                               C.c_size_t, _P]),
+    "sdrm_sample_bf16": (C.c_int, [_P, C.c_int64, C.c_int64, _P, _P, C.c_uint64, _P, _P, C.c_int64, _P, _P, _P, _P,
+                                   C.c_size_t, _P]),
     "sdrm_last_launch_count": (C.c_int, [_P]),
     "sdrm_check_device_error": (C.c_int, [_P, _P]),
     "sdrm_probe_linear_workspace_bytes": (C.c_size_t, [C.c_int64, C.c_int, C.c_int]),
@@ -58,6 +60,11 @@ SIGNATURES = {
     "sdrm_select_histogram": (C.c_int, [_P, C.c_int64, C.c_int, C.c_int64, _P, C.c_int, _P, _P]),
     "sdrm_select_walk": (C.c_int, [_P, _P, C.c_int, C.c_double, C.c_int, _P]),
     "sdrm_select_threshold_pack": (C.c_int, [_P, C.c_int64, C.c_int, C.c_int64, _P, C.c_int, _P, C.c_int64, _P, _P]),
+    "sdrm_key_histogram_bf16": (C.c_int, [_P, C.c_int64, C.c_int, C.c_int64, C.c_uint32, C.c_int, C.c_int, C.c_int, _P, _P]),
+    "sdrm_threshold_pack_bf16": (C.c_int, [_P, C.c_int64, C.c_int, C.c_int64, C.c_double, C.c_int, _P, C.c_int64, _P, _P]),
+    "sdrm_select_histogram_bf16": (C.c_int, [_P, C.c_int64, C.c_int, C.c_int64, _P, C.c_int, _P, _P]),
+    "sdrm_select_walk_bf16": (C.c_int, [_P, _P, C.c_int, C.c_double, C.c_int, _P]),
+    "sdrm_select_threshold_pack_bf16": (C.c_int, [_P, C.c_int64, C.c_int, C.c_int64, _P, C.c_int, _P, C.c_int64, _P, _P]),
     "sdrm_loss_grad_seeds": (C.c_int, [_P, _P, _P, _P, C.c_int64, C.c_double, _P, _P, _P, _P, _P, _P]),
 }
 

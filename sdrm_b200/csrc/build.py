@@ -6,8 +6,8 @@ import sys
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB = os.path.join(HERE, "libsdrm_b200.so")
-SOURCES = ["errors.cu", "engine_host.cu", "metrics.cu", "train_kernels.cu", "train_gemm.cu", "sparsify.cu"]
-HEADERS = ["ptx_sm100.cuh", "philox.cuh", "layer_engine.cuh", "layer_engine_kernel.cuh", "gemm_x3_kernel.cuh", "small_chain_kernel.cuh", "host_util.h",
+SOURCES = ["errors.cu", "engine_host.cu", "engine_bf16.cu", "metrics.cu", "train_kernels.cu", "train_gemm.cu", "sparsify.cu"]
+HEADERS = ["ptx_sm100.cuh", "philox.cuh", "layer_engine.cuh", "layer_engine_kernel.cuh", "engine_launch.cuh", "gemm_x3_kernel.cuh", "small_chain_kernel.cuh", "host_util.h",
            "../../include/sdrm_b200.h"]
 FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",

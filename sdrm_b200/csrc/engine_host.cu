@@ -15,6 +15,7 @@
 #include "layer_engine_kernel.cuh"
 #include "ptx_sm100.cuh"
 #include "small_chain_kernel.cuh"
+#include "engine_launch.cuh"
 
 namespace sdrm {
 
@@ -382,38 +383,10 @@ static int fill_pair_maps(ChainParams& P, size_t workspace_bytes, int cluster) {
   return SDRM_OK;
 }
 
-static int launch_engine(const ChainParams& P, int grid, int cluster, cudaStream_t st, int split = 0) {
-  if (split > 1) {   // column-split mode: single-CTA tiles, a cluster of `split` CTAs per row tile
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(static_cast<unsigned>(grid));
-    cfg.blockDim = dim3(ENGINE_THREADS);
-    cfg.dynamicSmemBytes = ENGINE_SMEM_BYTES;
-    cfg.stream = st;
-    cudaLaunchAttribute attr;
-    attr.id = cudaLaunchAttributeClusterDimension;
-    attr.val.clusterDim.x = split; attr.val.clusterDim.y = 1; attr.val.clusterDim.z = 1;
-    cfg.attrs = &attr; cfg.numAttrs = 1;
-    SDRM_CUDA(cudaLaunchKernelEx(&cfg, (sdrm_layer_engine_kernel<1, false, true>), P));
-    return SDRM_OK;
-  }
-  if (cluster == 1) {
-    sdrm_layer_engine_kernel<1><<<grid, ENGINE_THREADS, ENGINE_SMEM_BYTES, st>>>(P);
-    SDRM_CUDA(cudaGetLastError());
-    return SDRM_OK;
-  }
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(static_cast<unsigned>(grid));
-  cfg.blockDim = dim3(ENGINE_THREADS);
-  cfg.dynamicSmemBytes = ENGINE_SMEM_BYTES;
-  cfg.stream = st;
-  cudaLaunchAttribute attr;
-  attr.id = cudaLaunchAttributeClusterDimension;
-  attr.val.clusterDim.x = cluster; attr.val.clusterDim.y = 1; attr.val.clusterDim.z = 1;
-  cfg.attrs = &attr; cfg.numAttrs = 1;
-  if (cluster == 2 && P.resident) SDRM_CUDA(cudaLaunchKernelEx(&cfg, (sdrm_layer_engine_kernel<2, true>), P));
-  else if (cluster == 2) SDRM_CUDA(cudaLaunchKernelEx(&cfg, sdrm_layer_engine_kernel<2>, P));
-  else return sdrm_fail(SDRM_ERR_BAD_ARG, "launch_engine: cluster size");
-  return SDRM_OK;
+// The bfloat16-logits instantiations (sdrm_sample_bf16) are compiled in engine_bf16.cu: in this translation unit they would
+// perturb how the compiler optimises the fp32 kernels, whose code stays as it is.
+static int launch_engine(const ChainParams& P, int grid, int cluster, cudaStream_t st, int split = 0, bool bf16 = false) {
+  return bf16 ? launch_engine_bf16(P, grid, cluster, st, split) : launch_engine_t<false>(P, grid, cluster, st, split);
 }
 
 static void launch_pack_weight(const float* W, int N, int K, long long ldw, int col_off, uint8_t* hi, uint8_t* lo,
@@ -641,10 +614,12 @@ size_t sdrm_sample_workspace_bytes(const sdrm_handle* h, int64_t n) {
   return static_cast<size_t>(grid) * stride;
 }
 
-int sdrm_sample(sdrm_handle* h, int64_t n, int64_t row_offset, const int32_t* d_t_start, const int32_t* d_row_ids,
-                uint64_t seed,
-                float* d_x0_out, float* d_logits, int64_t ld_logits, const float* d_inj_xT, const float* d_inj_z,
-                const uint8_t* d_inj_mask, void* d_workspace, size_t workspace_bytes, void* stream) {
+}  // extern "C"
+
+// sdrm_sample and sdrm_sample_bf16: d_logits holds fp32 or (bf16) bfloat16 logits, ld_logits counts elements either way
+static int sample_impl(sdrm_handle* h, int64_t n, int64_t row_offset, const int32_t* d_t_start, const int32_t* d_row_ids,
+                       uint64_t seed, float* d_x0_out, void* d_logits, int64_t ld_logits, bool bf16, const float* d_inj_xT,
+                       const float* d_inj_z, const uint8_t* d_inj_mask, void* d_workspace, size_t workspace_bytes, void* stream) {
   if (!h) return sdrm_fail(SDRM_ERR_BAD_ARG, "sdrm_sample: null handle");
   if (!h->have_den || !h->have_dec) return sdrm_fail(SDRM_ERR_STATE, "sdrm_sample: pack denoiser and decoder first");
   if (h->g1.K != h->L) return sdrm_fail(SDRM_ERR_STATE, "sdrm_sample: decoder latent dim != denoiser latent dim");
@@ -682,9 +657,13 @@ int sdrm_sample(sdrm_handle* h, int64_t n, int64_t row_offset, const int32_t* d_
       return SDRM_OK;
     };
     int rc_s;
-    if (nt <= 3) rc_s = launch(sdrm_small_chain_kernel<3>, SmallGeom<3>::SMEM_BYTES);
-    else if (nt <= 5) rc_s = launch(sdrm_small_chain_kernel<5>, SmallGeom<5>::SMEM_BYTES);
-    else rc_s = launch(sdrm_small_chain_kernel<8>, SmallGeom<8>::SMEM_BYTES);
+    if (bf16) {
+      rc_s = launch_small_chain_bf16(S, nt, static_cast<unsigned>(ctas), st);
+    } else {
+      if (nt <= 3) rc_s = launch(sdrm_small_chain_kernel<3>, SmallGeom<3>::SMEM_BYTES);
+      else if (nt <= 5) rc_s = launch(sdrm_small_chain_kernel<5>, SmallGeom<5>::SMEM_BYTES);
+      else rc_s = launch(sdrm_small_chain_kernel<8>, SmallGeom<8>::SMEM_BYTES);
+    }
     if (rc_s) return rc_s;
     h->last_launches = 1;
     h->last_cluster = 0;   // 0 = not the cluster engine
@@ -846,10 +825,27 @@ int sdrm_sample(sdrm_handle* h, int64_t n, int64_t row_offset, const int32_t* d_
   }
   if (static_cast<size_t>(split ? n_tiles : launch_grid) * P.n_sub * stride > workspace_bytes)
     return sdrm_fail(SDRM_ERR_WORKSPACE, "sdrm_sample: workspace too small for the sub-tile scratch slots");
-  rc = launch_engine(P, launch_grid, cluster, st, split);
+  rc = launch_engine(P, launch_grid, cluster, st, split, bf16);
   if (rc) return rc;
   h->last_launches = 1;
   return SDRM_OK;
+}
+
+extern "C" {
+
+int sdrm_sample(sdrm_handle* h, int64_t n, int64_t row_offset, const int32_t* d_t_start, const int32_t* d_row_ids,
+                uint64_t seed,
+                float* d_x0_out, float* d_logits, int64_t ld_logits, const float* d_inj_xT, const float* d_inj_z,
+                const uint8_t* d_inj_mask, void* d_workspace, size_t workspace_bytes, void* stream) {
+  return sample_impl(h, n, row_offset, d_t_start, d_row_ids, seed, d_x0_out, d_logits, ld_logits, false, d_inj_xT, d_inj_z,
+                     d_inj_mask, d_workspace, workspace_bytes, stream);
+}
+
+int sdrm_sample_bf16(sdrm_handle* h, int64_t n, int64_t row_offset, const int32_t* d_t_start, const int32_t* d_row_ids,
+                     uint64_t seed, float* d_x0_out, uint16_t* d_logits, int64_t ld_logits, const float* d_inj_xT,
+                     const float* d_inj_z, const uint8_t* d_inj_mask, void* d_workspace, size_t workspace_bytes, void* stream) {
+  return sample_impl(h, n, row_offset, d_t_start, d_row_ids, seed, d_x0_out, d_logits, ld_logits, true, d_inj_xT, d_inj_z,
+                     d_inj_mask, d_workspace, workspace_bytes, stream);
 }
 
 int sdrm_last_launch_count(const sdrm_handle* h) { return h ? h->last_launches : 0; }

@@ -83,7 +83,7 @@ struct ChainParams {
   const int32_t* t_start; // per-row start step or nullptr (indexed by physical row)
   const int32_t* row_ids; // physical -> logical row or nullptr
   float* x0_out;          // [n, L] or nullptr
-  float* logits;          // [n, ld_logits]
+  void* logits;           // [n, ld_logits] fp32, or bfloat16 bits in the BF16OUT instantiations (ld_logits in elements)
   long long ld_logits;
   const float* inj_xT;    // [n, L]
   const float* inj_z;     // [T+1, n, L]

@@ -130,7 +130,10 @@ __device__ __forceinline__ void xs_store16(float* xs, int g16, int r, const floa
 // RESK: the resident-mode instantiation (see below).  A template parameter, not a run-time flag: the streaming instantiation must not
 // carry the mode's branches in the single-thread UMMA issue loop and in the epilogue group loops (measured: +1.2 % per cfg-5 shard).
 // SPLITK: the column-split instantiation (see below): single-CTA tcgen05, a CLUSTER of 2 / 4 / 8 CTAs shares one row tile.
-template <int CS, bool RESK = false, bool SPLITK = false>
+// BF16OUT: the logits are stored as bfloat16 (round to nearest even of the fp32 value the fp32 instantiation writes; P.logits
+// points to uint16_t bits, ld_logits counts elements).  Only the decoder's last epilogue differs; the fp32 instantiations carry
+// none of it.
+template <int CS, bool RESK = false, bool SPLITK = false, bool BF16OUT = false>
 __global__ void __launch_bounds__(ENGINE_THREADS, 1) sdrm_layer_engine_kernel(const __grid_constant__ ChainParams P) {
   static_assert(!RESK || CS == 2, "resident mode runs on CTA pairs");
   static_assert(!SPLITK || CS == 1, "column-split clusters are built from single-CTA (cta_group::1) tiles");
@@ -1005,9 +1008,11 @@ __global__ void __launch_bounds__(ENGINE_THREADS, 1) sdrm_layer_engine_kernel(co
           mbar_wait_sleepy(bar_noise_ready(s), (noise_par >> s) & 1u, err, WD_EPI_NOISE, 128);
           noise_par ^= 1u << s;
         }
-        const bool vec_out = ((P.ld_logits & 3) == 0) && ((reinterpret_cast<uintptr_t>(P.logits) & 15) == 0);
+        using OutT = std::conditional_t<BF16OUT, uint16_t, float>;
+        constexpr long long VEC_ELEMS = 16 / sizeof(OutT);   // logits per 16-byte store
+        const bool vec_out = ((P.ld_logits & (VEC_ELEMS - 1)) == 0) && ((reinterpret_cast<uintptr_t>(P.logits) & 15) == 0);
         const bool lin_rows = P.row_ids == nullptr;   // the warp's 32 rows are consecutive rows of the logits matrix (row = physical row)
-        float* orow = (KIND == EPI_LINEAR_OUT) ? P.logits + static_cast<size_t>(row) * P.ld_logits : nullptr;
+        OutT* orow = (KIND == EPI_LINEAR_OUT) ? static_cast<OutT*>(P.logits) + static_cast<size_t>(row) * P.ld_logits : nullptr;
         const bool res_layer = RES && (KIND == EPI_PRELU || KIND == EPI_POSTERIOR);   // (chain layers; the decoder streams)
         const bool publishes = !last_of_tile && KIND != EPI_LINEAR_OUT && !last_step && !res_layer;
         const bool lazy = ns == 2;   // see publish_pending
@@ -1151,6 +1156,37 @@ __global__ void __launch_bounds__(ENGINE_THREADS, 1) sdrm_layer_engine_kernel(co
               }
               store_act(out_hi_row, f0, ph);
               store_act(out_lo_row, f0, pl);
+            } else if constexpr (BF16OUT) {  // EPI_LINEAR_OUT, bfloat16 logits: the same three store paths at half the bytes
+              uint32_t pk[8];
+#pragma unroll
+              for (int e = 0; e < 8; ++e) pk[e] = pack_bf16x2(h[2 * e], h[2 * e + 1]);
+              if (vec_out && (f0 + 16 <= n_valid)) {
+                if (valid) {
+                  __stcs(reinterpret_cast<uint4*>(orow + f0), make_uint4(pk[0], pk[1], pk[2], pk[3]));
+                  __stcs(reinterpret_cast<uint4*>(orow + f0) + 1, make_uint4(pk[4], pk[5], pk[6], pk[7]));
+                }
+              } else if (lin_rows) {
+                // Unaligned rows (an item count that is no multiple of 8): the group's 16 columns x 32 rows of bf16 fill the warp's
+                // slot in one pass and go out with lanes along the columns: one instruction = 2 rows x 32 contiguous bytes.
+                if (elect_one()) bulk_wait_group_read<0>();
+                __syncwarp();
+                asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(out_lane), "r"(pk[0]), "r"(pk[1]), "r"(pk[2]), "r"(pk[3]) : "memory");
+                asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(out_lane + 16u), "r"(pk[4]), "r"(pk[5]), "r"(pk[6]), "r"(pk[7]) : "memory");
+                __syncwarp();
+                const int col = f0 + (lane & 15);
+#pragma unroll
+                for (int i2 = 0; i2 < 16; ++i2) {
+                  const int rr = 2 * i2 + (lane >> 4);
+                  unsigned short val;
+                  asm volatile("ld.shared.u16 %0, [%1];" : "=h"(val) : "r"(out_slot + static_cast<uint32_t>(rr * 32 + (lane & 15) * 2)) : "memory");
+                  if (row - lane + rr < P.n_rows && col < n_valid) __stcs(orow + static_cast<long long>(rr - lane) * P.ld_logits + col, val);
+                }
+                __syncwarp();
+              } else if (valid) {
+#pragma unroll
+                for (int e = 0; e < 16; ++e)
+                  if (f0 + e < n_valid) orow[f0 + e] = static_cast<uint16_t>(pk[e >> 1] >> (16 * (e & 1)));
+              }
             } else {  // EPI_LINEAR_OUT
               if (vec_out && (f0 + 16 <= n_valid)) {
                 if (valid) {

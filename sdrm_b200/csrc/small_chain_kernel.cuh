@@ -20,6 +20,8 @@
 #include <cuda_bf16.h>
 #include <stdint.h>
 
+#include <type_traits>
+
 #include "philox.cuh"
 #include "ptx_sm100.cuh"
 
@@ -36,7 +38,8 @@ struct SmallParams {
   int T, L, H, I, nh;
   long long n_rows, row_offset, ld_logits;
   const int32_t *t_start, *row_ids;
-  float *x0_out, *logits;
+  float* x0_out;
+  void* logits;                             // fp32, or bfloat16 bits (BF16OUT); ld_logits in elements
   const float *inj_xT, *inj_z;
   const uint8_t* inj_mask;
   unsigned long long seed;
@@ -69,7 +72,8 @@ __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commi
 template <int N>
 __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
 
-template <int NT>
+// BF16OUT: the logits are stored as bfloat16, the round to nearest even of the fp32 value the fp32 instantiation writes
+template <int NT, bool BF16OUT = false>
 __global__ void __launch_bounds__(SMALL_THREADS) sdrm_small_chain_kernel(const SmallParams P) {
   using G = SmallGeom<NT>;
   constexpr int KS = G::KS, KP = G::KP;
@@ -340,8 +344,10 @@ __global__ void __launch_bounds__(SMALL_THREADS) sdrm_small_chain_kernel(const S
     cp_async_commit();
   };
   fetch(0, 0);
-  const bool pair_ok = ((P.ld_logits & 1) == 0) && ((reinterpret_cast<uintptr_t>(P.logits) & 7) == 0);
-  float* orow[2] = {P.logits + static_cast<size_t>(lrow[0]) * P.ld_logits, P.logits + static_cast<size_t>(lrow[1]) * P.ld_logits};
+  using OutT = std::conditional_t<BF16OUT, uint16_t, float>;
+  const bool pair_ok = ((P.ld_logits & 1) == 0) && ((reinterpret_cast<uintptr_t>(P.logits) & (2 * sizeof(OutT) - 1)) == 0);
+  OutT* orow[2] = {static_cast<OutT*>(P.logits) + static_cast<size_t>(lrow[0]) * P.ld_logits,
+                   static_cast<OutT*>(P.logits) + static_cast<size_t>(lrow[1]) * P.ld_logits};
   for (int st = 0; st < n_stage; ++st) {
     const int buf = st & 1;
     if (st + 1 < n_stage) { fetch(st + 1, buf ^ 1); cp_async_wait<1>(); }
@@ -371,7 +377,14 @@ __global__ void __launch_bounds__(SMALL_THREADS) sdrm_small_chain_kernel(const S
         for (int h = 0; h < 2; ++h) {
           if (!valid[h]) continue;
           const float o0 = (a_hh[2 * h] + (a_hl[2 * h] + a_lh[2 * h])) + bb.x, o1 = (a_hh[2 * h + 1] + (a_hl[2 * h + 1] + a_lh[2 * h + 1])) + bb.y;
-          if (pair_ok && c + 1 < P.I) __stcs(reinterpret_cast<float2*>(orow[h] + c), make_float2(o0, o1));
+          if constexpr (BF16OUT) {
+            const uint32_t pk = pack_bf16x2(o0, o1);
+            if (pair_ok && c + 1 < P.I) __stcs(reinterpret_cast<unsigned int*>(orow[h] + c), pk);
+            else {
+              orow[h][c] = static_cast<uint16_t>(pk);
+              if (c + 1 < P.I) orow[h][c + 1] = static_cast<uint16_t>(pk >> 16);
+            }
+          } else if (pair_ok && c + 1 < P.I) __stcs(reinterpret_cast<float2*>(orow[h] + c), make_float2(o0, o1));
           else {
             orow[h][c] = o0;
             if (c + 1 < P.I) orow[h][c + 1] = o1;

@@ -9,9 +9,15 @@
 // (HBM-bound: 4 bytes per score), with the 2048-bin histograms summed across GPUs between passes when the rows
 // are sharded.  A last pass compares against the threshold and emits 1 bit per score (32x less D2H / gather
 // traffic than the fp32 matrix) plus the number of ones.
+//
+// bfloat16 score matrices (sdrm_*_bf16) use the 32-bit key of the score widened to float32, whose low 16 bits are fixed by its
+// sign (0 for a positive score, 0xFFFF for a negative one): an 11-bit and a 5-bit digit (bits 31..21, 20..16) pin the score
+// exactly, so the select reads the matrix twice at 2 bytes per score, and the pack pass once more.
 #include <cuda_runtime.h>
 #include <math.h>
 #include <stdint.h>
+
+#include <type_traits>
 
 #include "../../include/sdrm_b200.h"
 #include "host_util.h"
@@ -43,11 +49,17 @@ struct SelectState {
 };
 static_assert(sizeof(SelectState) == 56, "SelectState layout (mirrored by sdrm_b200/sparsify.py)");
 
-struct MatView {
-  const float* x;
+// T = float, or uint16_t for bfloat16 bits
+template <typename T>
+struct MatViewT {
+  const T* x;
   long long rows, ld;
   int n_cols;
 };
+using MatView = MatViewT<float>;
+using MatViewBf16 = MatViewT<uint16_t>;
+
+__device__ __forceinline__ float bf16_bits_float(uint32_t b) { return __uint_as_float(b << 16); }
 
 // Calls f(value) for every score of the view; float4 loads when the layout allows, grid-stride over the matrix.
 template <typename F>
@@ -88,9 +100,51 @@ __device__ __forceinline__ void for_each_score(const MatView& m, F&& f) {
   }
 }
 
+// bfloat16 scores: f(value widened to float32); 16-byte loads of 8 scores when the layout allows
+template <typename F>
+__device__ __forceinline__ void for_each_score(const MatViewBf16& m, F&& f) {
+  const long long tid = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x;
+  const long long nth = static_cast<long long>(gridDim.x) * blockDim.x;
+  const bool vec = ((m.n_cols & 7) == 0) && ((m.ld & 7) == 0) && ((reinterpret_cast<uintptr_t>(m.x) & 15) == 0);
+  auto f8 = [&](const uint4& v) {
+    f(bf16_bits_float(v.x & 0xFFFFu)); f(bf16_bits_float(v.x >> 16));
+    f(bf16_bits_float(v.y & 0xFFFFu)); f(bf16_bits_float(v.y >> 16));
+    f(bf16_bits_float(v.z & 0xFFFFu)); f(bf16_bits_float(v.z >> 16));
+    f(bf16_bits_float(v.w & 0xFFFFu)); f(bf16_bits_float(v.w >> 16));
+  };
+  if (vec) {
+    const long long c8 = m.n_cols >> 3;
+    const long long total = m.rows * c8;
+    if (m.ld == m.n_cols) {   // contiguous: plain 1-D sweep, four independent 16-byte loads in flight per thread
+      const uint4* p = reinterpret_cast<const uint4*>(m.x);
+      long long i = tid;
+      for (; i + 3 * nth < total; i += 4 * nth) {
+        uint4 v[4];
+#pragma unroll
+        for (int u = 0; u < 4; ++u) v[u] = __ldcs(p + i + u * nth);
+#pragma unroll
+        for (int u = 0; u < 4; ++u) f8(v[u]);
+      }
+      for (; i < total; i += nth) f8(__ldcs(p + i));
+    } else {
+      for (long long i = tid; i < total; i += nth) {
+        const long long r = i / c8, c = i - r * c8;
+        f8(__ldcs(reinterpret_cast<const uint4*>(m.x + r * m.ld) + c));
+      }
+    }
+  } else {
+    const long long total = m.rows * m.n_cols;
+    for (long long i = tid; i < total; i += nth) {
+      const long long r = i / m.n_cols, c = i - r * m.n_cols;
+      f(bf16_bits_float(__ldcs(m.x + r * m.ld + c)));
+    }
+  }
+}
+
 // One radix-select pass: histogram of the `bits`-wide digit at `shift` over the keys whose top `prefix_bits` bits equal
 // `prefix`; each warp keeps a private shared-memory histogram (no inter-warp conflicts), merged into global memory once.
-__global__ void __launch_bounds__(HIST_THREADS) key_hist_kernel(MatView m, uint32_t prefix, int prefix_bits, int shift, int bits,
+template <typename T>
+__global__ void __launch_bounds__(HIST_THREADS) key_hist_kernel(MatViewT<T> m, uint32_t prefix, int prefix_bits, int shift, int bits,
                                                                unsigned long long* __restrict__ hist, SelectState* __restrict__ st) {
   extern __shared__ uint32_t sh[];   // [HIST_WARPS][HIST_BINS]
   for (int i = threadIdx.x; i < HIST_WARPS * HIST_BINS; i += HIST_THREADS) sh[i] = 0;
@@ -137,8 +191,9 @@ __device__ __forceinline__ float key_float(uint32_t key) {
 // One block walks one (all-reduced) histogram: finds the digit of the lower order statistic, checks that the upper one (rank
 // + 1) shares it, narrows the prefix; behind the LAST digit it rebuilds the two floats and interpolates with NumPy's rule
 // (numpy/lib/_function_base_impl.py _lerp; since NumPy 2.0 gamma is float32 for float32 data, before it was float64).
+// low_bits: key bits below the last digit (16 for bfloat16 scores: their value follows from the sign bit, see the top).
 __global__ void __launch_bounds__(1024) select_walk_kernel(const unsigned long long* __restrict__ hist, SelectState* st, int bits, int last,
-                                                           double gamma, int gamma_f32) {
+                                                           double gamma, int gamma_f32, int low_bits) {
   __shared__ unsigned long long cum[HIST_BINS];
   __shared__ unsigned long long part[32];
   const int n = 1 << bits;
@@ -188,7 +243,12 @@ __global__ void __launch_bounds__(1024) select_walk_kernel(const unsigned long l
       st->rem[0] = r0 - before;
     } else {
       const uint32_t p1 = (st->prefix << bits) | static_cast<uint32_t>(b1 < n ? b1 : b0);
-      const float x0 = key_float(p0), x1 = st->two ? key_float(p1) : x0;
+      auto full_key = [&](uint32_t p) {
+        if (low_bits == 0) return p;
+        const uint32_t positive = (p >> (31 - low_bits)) & 1u;
+        return (p << low_bits) | (positive ? 0u : (1u << low_bits) - 1u);
+      };
+      const float x0 = key_float(full_key(p0)), x1 = st->two ? key_float(full_key(p1)) : x0;
       st->v0 = x0; st->v1 = x1;
       double thr;
       if (gamma_f32) {   // float32 arithmetic without contraction, exactly _lerp on np.float32 scalars
@@ -213,16 +273,22 @@ __global__ void __launch_bounds__(1024) select_walk_kernel(const unsigned long l
 // loads 4 consecutive scores (a 512-byte coalesced warp load, two in flight), forms its 4-bit nibble and three xor-shuffles
 // assemble the four 32-bit words of the 128 columns.
 template <int MODE>
-__global__ void __launch_bounds__(256) threshold_pack_kernel(MatView m, float thr, uint32_t* __restrict__ bits,
-                                                             long long words_per_row, unsigned long long* __restrict__ count,
-                                                             const SelectState* __restrict__ st) {
-  const int lane = threadIdx.x & 31;
+__device__ __forceinline__ float device_threshold(float thr, const SelectState* __restrict__ st) {
   if (st) {   // threshold selected on the device: same double -> float32 predicate conversion as the host entry
     const double td = st->threshold;
     thr = static_cast<float>(td);
     if (MODE == 0 && static_cast<double>(thr) < td) thr = nextafterf(thr, INFINITY);
     if (MODE == 1 && static_cast<double>(thr) > td) thr = nextafterf(thr, -INFINITY);
   }
+  return thr;
+}
+
+template <int MODE>
+__global__ void __launch_bounds__(256) threshold_pack_kernel(MatView m, float thr, uint32_t* __restrict__ bits,
+                                                             long long words_per_row, unsigned long long* __restrict__ count,
+                                                             const SelectState* __restrict__ st) {
+  const int lane = threadIdx.x & 31;
+  thr = device_threshold<MODE>(thr, st);
   const long long warp = (blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x) >> 5;
   const long long n_warps = (static_cast<long long>(gridDim.x) * blockDim.x) >> 5;
   const bool vec = ((m.ld & 3) == 0) && ((reinterpret_cast<uintptr_t>(m.x) & 15) == 0);
@@ -289,6 +355,70 @@ __global__ void __launch_bounds__(256) threshold_pack_kernel(MatView m, float th
   if (count && lane == 0 && ones) atomicAdd(count, ones);
 }
 
+// The same on bfloat16 scores (compared widened to float32: exact).  A lane loads 8 consecutive scores (one 16-byte load, a
+// 512-byte warp load of 256 columns) and forms their byte; two xor-shuffles assemble the eight 32-bit words.
+template <int MODE>
+__global__ void __launch_bounds__(256) threshold_pack_bf16_kernel(MatViewBf16 m, float thr, uint32_t* __restrict__ bits,
+                                                                  long long words_per_row, unsigned long long* __restrict__ count,
+                                                                  const SelectState* __restrict__ st) {
+  const int lane = threadIdx.x & 31;
+  thr = device_threshold<MODE>(thr, st);
+  const long long warp = (blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x) >> 5;
+  const long long n_warps = (static_cast<long long>(gridDim.x) * blockDim.x) >> 5;
+  const bool vec = ((m.ld & 7) == 0) && ((reinterpret_cast<uintptr_t>(m.x) & 15) == 0);
+  const int n_cols = m.n_cols;
+  unsigned long long ones = 0;
+  auto hit = [&](uint32_t b) { const float v = bf16_bits_float(b); return MODE == 0 ? (v >= thr) : (v <= thr); };
+  auto byte_of = [&](const uint4& v) {
+    const uint32_t w[4] = {v.x, v.y, v.z, v.w};
+    uint32_t r = 0;
+#pragma unroll
+    for (int k = 0; k < 4; ++k) r |= (hit(w[k] & 0xFFFFu) ? 1u : 0u) << (2 * k) | (hit(w[k] >> 16) ? 1u : 0u) << (2 * k + 1);
+    return r;
+  };
+  // lane l holds columns 8l..8l+7 of a 256-column block: word l/4, bits 8 (l%4) ..
+  auto emit = [&](uint32_t byte, uint32_t* out, int c_block) {
+    uint32_t w = byte << (8 * (lane & 3));
+    w |= __shfl_xor_sync(0xffffffffu, w, 1);
+    w |= __shfl_xor_sync(0xffffffffu, w, 2);
+    const int word = c_block / 32 + (lane >> 2);
+    if ((lane & 3) == 0 && word * 32 < n_cols) {
+      out[word] = w;
+      ones += __popc(w);
+    }
+  };
+  for (long long r = warp; r < m.rows; r += n_warps) {
+    const uint16_t* x = m.x + r * m.ld;
+    uint32_t* out = bits + r * words_per_row;
+    int c0 = 0;
+    // interior: whole 1024-column spans of 16-byte aligned rows, four loads in flight per lane, no per-element range checks
+    if (vec) {
+      for (; c0 + 1024 <= n_cols; c0 += 1024) {
+        uint4 v[4];
+#pragma unroll
+        for (int u = 0; u < 4; ++u) v[u] = __ldcs(reinterpret_cast<const uint4*>(x + c0 + u * 256 + lane * 8));
+#pragma unroll
+        for (int u = 0; u < 4; ++u) emit(byte_of(v[u]), out, c0 + u * 256);
+      }
+    }
+    for (; c0 < n_cols; c0 += 256) {
+      const int c = c0 + lane * 8;
+      uint32_t byte = 0;
+      if (vec && c + 8 <= n_cols) {
+        byte = byte_of(__ldcs(reinterpret_cast<const uint4*>(x + c)));
+      } else {
+#pragma unroll
+        for (int k = 0; k < 8; ++k)
+          if (c + k < n_cols && hit(__ldcs(x + c + k))) byte |= 1u << k;
+      }
+      emit(byte, out, c0);
+    }
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) ones += __shfl_xor_sync(0xffffffffu, ones, o);
+  if (count && lane == 0 && ones) atomicAdd(count, ones);
+}
+
 static int grid_for(long long work_items, int threads, int per_thread, int blocks_per_sm) {
   int dev = 0, sms = 148;
   cudaGetDevice(&dev);
@@ -304,29 +434,104 @@ static int grid_for(long long work_items, int threads, int per_thread, int block
 
 using namespace sdrm;
 
-extern "C" {
-
-int sdrm_key_histogram(const float* d_scores, int64_t rows, int n_cols, int64_t ld, uint32_t prefix, int prefix_bits,
-                       int shift, int bits, unsigned long long* d_hist, void* stream) {
-  if (!d_scores || !d_hist) return sdrm_fail(SDRM_ERR_BAD_ARG, "sdrm_key_histogram: null pointer");
-  if (rows < 0 || n_cols <= 0 || ld < n_cols) return sdrm_fail(SDRM_ERR_BAD_ARG, "sdrm_key_histogram: bad shape");
-  if (bits < 1 || bits > 11 || shift < 0 || shift + bits > 32 || prefix_bits < 0 || prefix_bits > 31 || prefix_bits + bits + shift != 32)
-    return sdrm_fail(SDRM_ERR_BAD_ARG, "sdrm_key_histogram: digit layout (prefix_bits + bits + shift must be 32, bits <= 11)");
-  if (rows == 0) return SDRM_OK;
+// ---- host side, shared by the float32 and the bfloat16 entries (T = float / uint16_t) -----------------------------------------
+template <typename T>
+static int launch_key_hist(const T* d_scores, int64_t rows, int n_cols, int64_t ld, uint32_t prefix, int prefix_bits,
+                           int shift, int bits, unsigned long long* d_hist, SelectState* st, void* stream) {
   static bool attr_done = false;
   const int smem = HIST_WARPS * HIST_BINS * static_cast<int>(sizeof(uint32_t));   // 64 KB
   if (!attr_done) {
-    SDRM_CUDA(cudaFuncSetAttribute(key_hist_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    SDRM_CUDA(cudaFuncSetAttribute(key_hist_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
     attr_done = true;
   }
-  MatView m{d_scores, rows, ld, n_cols};
+  MatViewT<T> m{d_scores, rows, ld, n_cols};
   const int grid = grid_for(rows * static_cast<long long>(n_cols), HIST_THREADS, 64, 3);
-  key_hist_kernel<<<grid, HIST_THREADS, smem, static_cast<cudaStream_t>(stream)>>>(m, prefix, prefix_bits, shift, bits, d_hist, nullptr);
+  key_hist_kernel<T><<<grid, HIST_THREADS, smem, static_cast<cudaStream_t>(stream)>>>(m, prefix, prefix_bits, shift, bits, d_hist, st);
   SDRM_CUDA(cudaGetLastError());
   return SDRM_OK;
 }
 
+template <typename T>
+static int key_histogram(const char* what, const T* d_scores, int64_t rows, int n_cols, int64_t ld, uint32_t prefix, int prefix_bits,
+                         int shift, int bits, unsigned long long* d_hist, void* stream) {
+  char msg[160];
+  if (!d_scores || !d_hist) { snprintf(msg, sizeof msg, "%s: null pointer", what); return sdrm_fail(SDRM_ERR_BAD_ARG, msg); }
+  if (rows < 0 || n_cols <= 0 || ld < n_cols) { snprintf(msg, sizeof msg, "%s: bad shape", what); return sdrm_fail(SDRM_ERR_BAD_ARG, msg); }
+  if (bits < 1 || bits > 11 || shift < 0 || shift + bits > 32 || prefix_bits < 0 || prefix_bits > 31 || prefix_bits + bits + shift != 32) {
+    snprintf(msg, sizeof msg, "%s: digit layout (prefix_bits + bits + shift must be 32, bits <= 11)", what);
+    return sdrm_fail(SDRM_ERR_BAD_ARG, msg);
+  }
+  if (rows == 0) return SDRM_OK;
+  return launch_key_hist<T>(d_scores, rows, n_cols, ld, prefix, prefix_bits, shift, bits, d_hist, nullptr, stream);
+}
+
+// Digits of the device-side select: float32 keys 11 + 11 + 10 bits, bfloat16 keys 11 + 5 (the low 16 key bits follow from the sign)
 static const int kDigitBits[3] = {11, 11, 10}, kDigitShift[3] = {21, 10, 0};
+static const int kDigitBitsBf16[2] = {11, 5}, kDigitShiftBf16[2] = {21, 16};
+
+template <typename T>
+static int select_histogram(const char* what, const T* d_scores, int64_t rows, int n_cols, int64_t ld, void* d_state, int digit,
+                            unsigned long long* d_hist, void* stream) {
+  constexpr bool BF16 = std::is_same<T, uint16_t>::value;
+  const int n_digits = BF16 ? 2 : 3;
+  char msg[160];
+  if (!d_scores || !d_hist || !d_state) { snprintf(msg, sizeof msg, "%s: null pointer", what); return sdrm_fail(SDRM_ERR_BAD_ARG, msg); }
+  if (rows < 0 || n_cols <= 0 || ld < n_cols || digit < 0 || digit >= n_digits) {
+    snprintf(msg, sizeof msg, "%s: bad shape / digit", what);
+    return sdrm_fail(SDRM_ERR_BAD_ARG, msg);
+  }
+  if (rows == 0) return SDRM_OK;
+  const int bits = BF16 ? kDigitBitsBf16[digit] : kDigitBits[digit], shift = BF16 ? kDigitShiftBf16[digit] : kDigitShift[digit];
+  return launch_key_hist<T>(d_scores, rows, n_cols, ld, 0u, 32 - bits - shift, shift, bits, d_hist, static_cast<SelectState*>(d_state),
+                            stream);
+}
+
+template <typename T>
+static int threshold_pack(const char* what, const T* d_scores, int64_t rows, int n_cols, int64_t ld, float tf, const void* d_state, int mode,
+                          uint32_t* d_bits, int64_t words_per_row, unsigned long long* d_count, void* stream) {
+  char msg[160];
+  if (!d_scores || !d_bits) { snprintf(msg, sizeof msg, "%s: null pointer", what); return sdrm_fail(SDRM_ERR_BAD_ARG, msg); }
+  if (rows < 0 || n_cols <= 0 || ld < n_cols || words_per_row < (n_cols + 31) / 32 || (mode != 0 && mode != 1)) {
+    snprintf(msg, sizeof msg, "%s: bad shape / mode", what);
+    return sdrm_fail(SDRM_ERR_BAD_ARG, msg);
+  }
+  if (rows == 0) return SDRM_OK;
+  MatViewT<T> m{d_scores, rows, ld, n_cols};
+  const int grid = grid_for(rows * 32, 256, 1, 8);   // one warp per row until the wave is full
+  const SelectState* st = static_cast<const SelectState*>(d_state);
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  if constexpr (std::is_same<T, uint16_t>::value) {
+    if (mode == 0) threshold_pack_bf16_kernel<0><<<grid, 256, 0, s>>>(m, tf, d_bits, words_per_row, d_count, st);
+    else threshold_pack_bf16_kernel<1><<<grid, 256, 0, s>>>(m, tf, d_bits, words_per_row, d_count, st);
+  } else {
+    if (mode == 0) threshold_pack_kernel<0><<<grid, 256, 0, s>>>(m, tf, d_bits, words_per_row, d_count, st);
+    else threshold_pack_kernel<1><<<grid, 256, 0, s>>>(m, tf, d_bits, words_per_row, d_count, st);
+  }
+  SDRM_CUDA(cudaGetLastError());
+  return SDRM_OK;
+}
+
+// The scores are float32 (or bfloat16, exact in float32): x >= t (double) is the same predicate as x >= the smallest float32 not
+// below t (and x <= t the same as x <= the largest float32 not above t), so the device compares in fp32 (B200 runs FP64 at a
+// fraction of the rate).
+static float predicate_threshold(double threshold, int mode) {
+  float tf = static_cast<float>(threshold);
+  if (mode == 0 && static_cast<double>(tf) < threshold) tf = nextafterf(tf, INFINITY);
+  if (mode == 1 && static_cast<double>(tf) > threshold) tf = nextafterf(tf, -INFINITY);
+  return tf;
+}
+
+extern "C" {
+
+int sdrm_key_histogram(const float* d_scores, int64_t rows, int n_cols, int64_t ld, uint32_t prefix, int prefix_bits,
+                       int shift, int bits, unsigned long long* d_hist, void* stream) {
+  return key_histogram("sdrm_key_histogram", d_scores, rows, n_cols, ld, prefix, prefix_bits, shift, bits, d_hist, stream);
+}
+
+int sdrm_key_histogram_bf16(const uint16_t* d_scores, int64_t rows, int n_cols, int64_t ld, uint32_t prefix, int prefix_bits,
+                            int shift, int bits, unsigned long long* d_hist, void* stream) {
+  return key_histogram("sdrm_key_histogram_bf16", d_scores, rows, n_cols, ld, prefix, prefix_bits, shift, bits, d_hist, stream);
+}
 
 size_t sdrm_select_state_bytes(void) { return sizeof(SelectState); }
 
@@ -339,63 +544,53 @@ int sdrm_select_begin(void* d_state, uint64_t rank_lo, uint64_t rank_hi, void* s
 
 int sdrm_select_histogram(const float* d_scores, int64_t rows, int n_cols, int64_t ld, void* d_state, int digit,
                           unsigned long long* d_hist, void* stream) {
-  if (!d_scores || !d_hist || !d_state) return sdrm_fail(SDRM_ERR_BAD_ARG, "sdrm_select_histogram: null pointer");
-  if (rows < 0 || n_cols <= 0 || ld < n_cols || digit < 0 || digit > 2) return sdrm_fail(SDRM_ERR_BAD_ARG, "sdrm_select_histogram: bad shape / digit");
-  if (rows == 0) return SDRM_OK;
-  static bool attr_done = false;
-  const int smem = HIST_WARPS * HIST_BINS * static_cast<int>(sizeof(uint32_t));
-  if (!attr_done) {
-    SDRM_CUDA(cudaFuncSetAttribute(key_hist_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-    attr_done = true;
-  }
-  MatView m{d_scores, rows, ld, n_cols};
-  const int grid = grid_for(rows * static_cast<long long>(n_cols), HIST_THREADS, 64, 3);
-  key_hist_kernel<<<grid, HIST_THREADS, smem, static_cast<cudaStream_t>(stream)>>>(m, 0u, 32 - kDigitBits[digit] - kDigitShift[digit], kDigitShift[digit],
-                                                                                   kDigitBits[digit], d_hist, static_cast<SelectState*>(d_state));
-  SDRM_CUDA(cudaGetLastError());
-  return SDRM_OK;
+  return select_histogram("sdrm_select_histogram", d_scores, rows, n_cols, ld, d_state, digit, d_hist, stream);
+}
+
+int sdrm_select_histogram_bf16(const uint16_t* d_scores, int64_t rows, int n_cols, int64_t ld, void* d_state, int digit,
+                               unsigned long long* d_hist, void* stream) {
+  return select_histogram("sdrm_select_histogram_bf16", d_scores, rows, n_cols, ld, d_state, digit, d_hist, stream);
 }
 
 int sdrm_select_walk(const unsigned long long* d_hist, void* d_state, int digit, double gamma, int gamma_is_f32, void* stream) {
   if (!d_hist || !d_state || digit < 0 || digit > 2) return sdrm_fail(SDRM_ERR_BAD_ARG, "sdrm_select_walk: bad argument");
   select_walk_kernel<<<1, 1024, 0, static_cast<cudaStream_t>(stream)>>>(d_hist, static_cast<SelectState*>(d_state), kDigitBits[digit], digit == 2, gamma,
-                                                                        gamma_is_f32);
+                                                                        gamma_is_f32, 0);
+  SDRM_CUDA(cudaGetLastError());
+  return SDRM_OK;
+}
+
+int sdrm_select_walk_bf16(const unsigned long long* d_hist, void* d_state, int digit, double gamma, int gamma_is_f32, void* stream) {
+  if (!d_hist || !d_state || digit < 0 || digit > 1) return sdrm_fail(SDRM_ERR_BAD_ARG, "sdrm_select_walk_bf16: bad argument");
+  select_walk_kernel<<<1, 1024, 0, static_cast<cudaStream_t>(stream)>>>(d_hist, static_cast<SelectState*>(d_state), kDigitBitsBf16[digit], digit == 1,
+                                                                        gamma, gamma_is_f32, 16);
   SDRM_CUDA(cudaGetLastError());
   return SDRM_OK;
 }
 
 int sdrm_select_threshold_pack(const float* d_scores, int64_t rows, int n_cols, int64_t ld, const void* d_state, int mode,
                                uint32_t* d_bits, int64_t words_per_row, unsigned long long* d_count, void* stream) {
-  if (!d_scores || !d_bits || !d_state) return sdrm_fail(SDRM_ERR_BAD_ARG, "sdrm_select_threshold_pack: null pointer");
-  if (rows < 0 || n_cols <= 0 || ld < n_cols || words_per_row < (n_cols + 31) / 32 || (mode != 0 && mode != 1))
-    return sdrm_fail(SDRM_ERR_BAD_ARG, "sdrm_select_threshold_pack: bad shape / mode");
-  if (rows == 0) return SDRM_OK;
-  MatView m{d_scores, rows, ld, n_cols};
-  const int grid = grid_for(rows * 32, 256, 1, 8);
-  const SelectState* st = static_cast<const SelectState*>(d_state);
-  if (mode == 0) threshold_pack_kernel<0><<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(m, 0.0f, d_bits, words_per_row, d_count, st);
-  else threshold_pack_kernel<1><<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(m, 0.0f, d_bits, words_per_row, d_count, st);
-  SDRM_CUDA(cudaGetLastError());
-  return SDRM_OK;
+  if (!d_state) return sdrm_fail(SDRM_ERR_BAD_ARG, "sdrm_select_threshold_pack: null pointer");
+  return threshold_pack("sdrm_select_threshold_pack", d_scores, rows, n_cols, ld, 0.0f, d_state, mode, d_bits, words_per_row, d_count, stream);
+}
+
+int sdrm_select_threshold_pack_bf16(const uint16_t* d_scores, int64_t rows, int n_cols, int64_t ld, const void* d_state, int mode,
+                                    uint32_t* d_bits, int64_t words_per_row, unsigned long long* d_count, void* stream) {
+  if (!d_state) return sdrm_fail(SDRM_ERR_BAD_ARG, "sdrm_select_threshold_pack_bf16: null pointer");
+  return threshold_pack("sdrm_select_threshold_pack_bf16", d_scores, rows, n_cols, ld, 0.0f, d_state, mode, d_bits, words_per_row, d_count,
+                        stream);
 }
 
 int sdrm_threshold_pack(const float* d_scores, int64_t rows, int n_cols, int64_t ld, double threshold, int mode,
                         uint32_t* d_bits, int64_t words_per_row, unsigned long long* d_count, void* stream) {
-  if (!d_scores || !d_bits) return sdrm_fail(SDRM_ERR_BAD_ARG, "sdrm_threshold_pack: null pointer");
-  if (rows < 0 || n_cols <= 0 || ld < n_cols || words_per_row < (n_cols + 31) / 32 || (mode != 0 && mode != 1))
-    return sdrm_fail(SDRM_ERR_BAD_ARG, "sdrm_threshold_pack: bad shape / mode");
-  if (rows == 0) return SDRM_OK;
-  MatView m{d_scores, rows, ld, n_cols};
-  // The scores are float32: x >= t (double) is the same predicate as x >= the smallest float32 not below t (and x <= t the
-  // same as x <= the largest float32 not above t), so the device compares in fp32 (B200 runs FP64 at a fraction of the rate).
-  float tf = static_cast<float>(threshold);
-  if (mode == 0 && static_cast<double>(tf) < threshold) tf = nextafterf(tf, INFINITY);
-  if (mode == 1 && static_cast<double>(tf) > threshold) tf = nextafterf(tf, -INFINITY);
-  const int grid = grid_for(rows * 32, 256, 1, 8);   // one warp per row until the wave is full
-  if (mode == 0) threshold_pack_kernel<0><<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(m, tf, d_bits, words_per_row, d_count, nullptr);
-  else threshold_pack_kernel<1><<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(m, tf, d_bits, words_per_row, d_count, nullptr);
-  SDRM_CUDA(cudaGetLastError());
-  return SDRM_OK;
+  return threshold_pack("sdrm_threshold_pack", d_scores, rows, n_cols, ld, predicate_threshold(threshold, mode), nullptr, mode, d_bits,
+                        words_per_row, d_count, stream);
+}
+
+int sdrm_threshold_pack_bf16(const uint16_t* d_scores, int64_t rows, int n_cols, int64_t ld, double threshold, int mode,
+                             uint32_t* d_bits, int64_t words_per_row, unsigned long long* d_count, void* stream) {
+  return threshold_pack("sdrm_threshold_pack_bf16", d_scores, rows, n_cols, ld, predicate_threshold(threshold, mode), nullptr, mode, d_bits,
+                        words_per_row, d_count, stream);
 }
 
 }  // extern "C"

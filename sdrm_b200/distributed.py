@@ -26,7 +26,7 @@ def shard_bounds(n, rank, world):
 
 
 def sample_ddpm_sharded(n_sample, diff_net, vae_net, diff_latent_dim, noise_divider=1.0, timesteps=None,
-                        n_timesteps=None, *, seed, group=None, gather=False, sparsity=None, sampler=None):
+                        n_timesteps=None, *, seed, group=None, gather=False, sparsity=None, sampler=None, out_dtype=None):
     """Each rank samples its contiguous block of the n_sample rows (same `seed` on every rank; the Philox streams are keyed
     by the global row id, so in full-resolution mode the union of the blocks is bit-identical to a single-GPU run).
 
@@ -40,6 +40,9 @@ def sample_ddpm_sharded(n_sample, diff_net, vae_net, diff_latent_dim, noise_divi
     gather="bits"     -> equal-sparsity binarisation with the GLOBAL np.quantile threshold (sparsity = the reference's SPARSITY,
                          main.py:177-178) and an all_gather of the BIT-PACKED rows (32x less NVLink traffic: 312 MB per GPU at the
                          scale-up shape); returns (PackedMatrix of all n_sample rows, (0, n_sample))
+    out_dtype=torch.bfloat16 samples bfloat16 rows (the rounded float32 rows, sample_ddpm's out_dtype): gather=False / True then
+    return / gather bfloat16 blocks (half the NVLink bytes), and gather="bits" binarises the bfloat16 rows (sparsify.py: ties
+    at the threshold can keep a few more ones than the float32 rows would).
     An empty block (more ranks than rows) is legal: the rank still takes part in the collectives."""
     import numpy as np
     if sampler is None:
@@ -51,6 +54,8 @@ def sample_ddpm_sharded(n_sample, diff_net, vae_net, diff_latent_dim, noise_divi
     if isinstance(timesteps, str) and timesteps == "random" and n_timesteps is not None:
         t_all = np.random.RandomState(int(seed) & 0x7FFFFFFF).randint(1, int(n_timesteps), size=int(n_sample)).astype(np.int32)
         kw["t_rows"] = t_all[lo:hi]
+    if out_dtype is not None:
+        kw["out_dtype"] = out_dtype
     rows = sampler(hi - lo, diff_net, vae_net, diff_latent_dim, noise_divider, timesteps=timesteps,
                    n_timesteps=n_timesteps, seed=seed, row_offset=lo, **kw)
     if not gather or world == 1:

@@ -104,13 +104,17 @@ class SamplerEngine:
 
     def sample(self, n, row_offset=0, t_start=None, row_ids=None, seed=0, out=None, latent_out=None, inj_xT=None, inj_z=None,
                inj_keep=None, check=False):
-        """Run the chain + decode for n rows; returns logits [n, I] fp32 on the device."""
+        """Run the chain + decode for n rows; returns logits [n, I] on the device, fp32 unless `out` is a bfloat16 tensor: then
+        every logit is the round-to-nearest-even bfloat16 of the fp32 value (sdrm_sample_bf16), at half the bytes."""
         if self._den_key is None or self._dec_key is None:
             raise _lib.SdrmError("pack_denoiser / pack_decoder must be called before sample")
         if out is None:
             out = torch.empty((n, self.I), dtype=torch.float32, device=self.device)
-        if out.dtype != torch.float32 or out.stride(1) != 1 or out.shape[0] < n or out.shape[1] < self.I:
-            raise ValueError("out must be float32 [>=n, >=I] with unit column stride")
+        if out.device.type != "cuda":
+            raise _lib.SdrmError("out must be a CUDA tensor (no CPU fallback)")
+        if (out.dtype not in (torch.float32, torch.bfloat16) or out.dim() != 2 or out.stride(1) != 1 or out.shape[0] < n
+                or out.shape[1] < self.I):
+            raise ValueError("out must be float32 or bfloat16 [>=n, >=I] with unit column stride")
         if n == 0:
             return out
         ws, need = self.workspace(n)
@@ -128,10 +132,11 @@ class SamplerEngine:
                             ("inj_keep", inj_keep, torch.uint8)):
             if t is not None and (t.dtype != dt or not t.is_contiguous() or t.device != self.device):
                 raise ValueError(f"{name} must be a contiguous {dt} tensor on {self.device}")
-        rc = self.lib.sdrm_sample(self.handle, n, row_offset, _lib.ptr(t_start), _lib.ptr(row_ids), seed & (2 ** 64 - 1),
-                                  _lib.ptr(latent_out), _lib.ptr(out), out.stride(0), _lib.ptr(inj_xT),
-                                  _lib.ptr(inj_z), _lib.ptr(inj_keep), _lib.ptr(ws), need, _lib.stream_ptr())
-        _lib.check(rc, "sdrm_sample")
+        entry = self.lib.sdrm_sample_bf16 if out.dtype == torch.bfloat16 else self.lib.sdrm_sample
+        rc = entry(self.handle, n, row_offset, _lib.ptr(t_start), _lib.ptr(row_ids), seed & (2 ** 64 - 1),
+                   _lib.ptr(latent_out), _lib.ptr(out), out.stride(0), _lib.ptr(inj_xT),
+                   _lib.ptr(inj_z), _lib.ptr(inj_keep), _lib.ptr(ws), need, _lib.stream_ptr())
+        _lib.check(rc, "sdrm_sample_bf16" if out.dtype == torch.bfloat16 else "sdrm_sample")
         if check:
             _lib.check(self.lib.sdrm_check_device_error(self.handle, _lib.stream_ptr()), "sdrm_sample (device)")
         return out

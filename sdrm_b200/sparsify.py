@@ -13,6 +13,11 @@ threshold is bit-identical to `np.quantile`, and `sdrm_threshold_pack` emits one
 sharded over several GPUs the 2048-bin histograms are summed with one all-reduce per pass (the only exchange step), so
 every rank derives the SAME global threshold the single-process reference would.
 
+bfloat16 score matrices (sample_ddpm(..., out_dtype=torch.bfloat16)) take the same path at 2 bytes per score.  Their scores
+are ranked and compared as float32 values, so the threshold is np.quantile(S.astype(np.float32).flatten(), q) bit for bit and
+the bits are S >= thr.  The float32 key of a bfloat16 score has its low 16 bits fixed by the sign, so two histogram passes
+(11 + 5 bits) pin it instead of three.
+
 No CPU fallback: a CPU tensor raises.
 """
 import ctypes as C
@@ -23,6 +28,7 @@ import torch
 from . import _lib
 
 _DIGITS = ((11, 21), (11, 10), (10, 0))   # (bits, shift): 11 + 11 + 10 = 32
+_DIGITS_BF16 = ((11, 21), (5, 16))         # bfloat16 scores: the low 16 key bits follow from the sign bit
 
 
 # --------------------------------------------------------------------------------------------------
@@ -78,14 +84,15 @@ def float_to_key(x):
     return (~u & 0xFFFFFFFF) if (u & 0x80000000) else (u | 0x80000000)
 
 
-def select_ranks(hist_fn, ranks):
+def select_ranks(hist_fn, ranks, digits=_DIGITS):
     """Exact radix select.  hist_fn(prefix, prefix_bits, shift, bits) -> int64 array of global digit counts.
-    Returns the float32 order statistic for every 0-based rank in `ranks` (histograms shared between ranks)."""
+    Returns the float32 order statistic for every 0-based rank in `ranks` (histograms shared between ranks).
+    digits=_DIGITS_BF16 for bfloat16 scores: the key bits below the last digit are 0 for a positive score, all ones else."""
     cache = {}
     out = []
     for r in ranks:
         prefix, pbits, rem = 0, 0, int(r)
-        for bits, shift in _DIGITS:
+        for bits, shift in digits:
             k = (prefix, pbits)
             if k not in cache:
                 cache[k] = np.cumsum(np.asarray(hist_fn(prefix, pbits, shift, bits), dtype=np.int64)[: 1 << bits])
@@ -96,6 +103,9 @@ def select_ranks(hist_fn, ranks):
             if b:
                 rem -= int(cum[b - 1])
             prefix, pbits = (prefix << bits) | b, pbits + bits
+        low = 32 - pbits
+        if low:
+            prefix = (prefix << low) | (0 if (prefix >> (pbits - 1)) & 1 else (1 << low) - 1)
         out.append(key_to_float(prefix))
     return out
 
@@ -106,8 +116,12 @@ def select_ranks(hist_fn, ranks):
 def _check(scores):
     if not isinstance(scores, torch.Tensor) or scores.device.type != "cuda":
         raise _lib.SdrmError("sparsify: scores must be a CUDA tensor (no CPU fallback)")
-    if scores.dtype != torch.float32 or scores.dim() != 2 or scores.stride(1) != 1:
-        raise ValueError("scores must be float32 [rows, items] with unit column stride")
+    if scores.dtype not in (torch.float32, torch.bfloat16) or scores.dim() != 2 or scores.stride(1) != 1:
+        raise ValueError("scores must be float32 or bfloat16 [rows, items] with unit column stride")
+
+
+def _bf16(scores):
+    return scores.dtype == torch.bfloat16
 
 
 def _world(group):
@@ -126,8 +140,9 @@ def device_histogram_fn(scores, group=None):
 
     def hist_fn(prefix, prefix_bits, shift, bits):
         h = torch.zeros(2048, dtype=torch.int64, device=scores.device)
-        _lib.check(lib.sdrm_key_histogram(_lib.ptr(scores), rows, n_cols, scores.stride(0) if rows else n_cols, prefix, prefix_bits,
-                                          shift, bits, _lib.ptr(h), _lib.stream_ptr()), "sdrm_key_histogram")
+        entry = lib.sdrm_key_histogram_bf16 if _bf16(scores) else lib.sdrm_key_histogram
+        _lib.check(entry(_lib.ptr(scores), rows, n_cols, scores.stride(0) if rows else n_cols, prefix, prefix_bits,
+                         shift, bits, _lib.ptr(h), _lib.stream_ptr()), "sdrm_key_histogram")
         if dist is not None:
             dist.all_reduce(h, group=group)
         return h.cpu().numpy()
@@ -151,13 +166,13 @@ def quantile_host_walk(scores, q, group=None):
     n_total = global_count(scores, group)
     prev_i, nxt_i, gamma = quantile_plan(n_total, q, np.float32)
     ranks = [prev_i] if nxt_i == prev_i else [prev_i, nxt_i]
-    vals = select_ranks(device_histogram_fn(scores, group), ranks)
+    vals = select_ranks(device_histogram_fn(scores, group), ranks, _DIGITS_BF16 if _bf16(scores) else _DIGITS)
     return lerp(vals[0], vals[-1], gamma)
 
 
 def quantile_device(scores, q, group=None):
     """np.quantile(S.flatten(), q) for a float32 CUDA matrix (row-sharded over `group` if given), bit-identical to NumPy
-    (NaN as soon as one score is NaN)."""
+    (NaN as soon as one score is NaN).  For a bfloat16 matrix: np.quantile(S.astype(np.float32).flatten(), q)."""
     _check(scores)
     state, g32 = _select_enqueue(scores, q, group)
     thr, fallback, nans = _read_state(state, g32)
@@ -184,22 +199,25 @@ class PackedMatrix:
 
 
 def threshold_pack(scores, threshold, lower=False):
-    """(S >= threshold) — or (S <= threshold) with lower=True — as a PackedMatrix."""
+    """(S >= threshold) — or (S <= threshold) with lower=True — as a PackedMatrix (float32 or bfloat16 scores, compared as
+    float32 values)."""
     _check(scores)
     lib = _lib.load()
     rows, n_cols = scores.shape
     wpr = (n_cols + 31) // 32
     bits = torch.empty((rows, wpr), dtype=torch.int32, device=scores.device)
     count = torch.zeros(1, dtype=torch.int64, device=scores.device)
-    _lib.check(lib.sdrm_threshold_pack(_lib.ptr(scores), rows, n_cols, scores.stride(0) if rows else n_cols, float(threshold),
+    entry = lib.sdrm_threshold_pack_bf16 if _bf16(scores) else lib.sdrm_threshold_pack
+    _lib.check(entry(_lib.ptr(scores), rows, n_cols, scores.stride(0) if rows else n_cols, float(threshold),
                                        1 if lower else 0, _lib.ptr(bits), wpr, _lib.ptr(count), _lib.stream_ptr()),
                "sdrm_threshold_pack")
     return PackedMatrix(bits, n_cols, threshold, count)
 
 
 def _select_enqueue(scores, q, group):
-    """Enqueue the device-side quantile selection (C ABI sdrm_select_*): three histogram passes with a one-block walk kernel
-    between them (and one all-reduce of 2048 bins per pass when the rows are sharded); nothing is read back here."""
+    """Enqueue the device-side quantile selection (C ABI sdrm_select_*): three histogram passes (two for bfloat16 scores) with a
+    one-block walk kernel between them (and one all-reduce of 2048 bins per pass when the rows are sharded); nothing is read
+    back here."""
     lib = _lib.load()
     dist = _world(group)
     rows, n_cols = scores.shape
@@ -207,19 +225,23 @@ def _select_enqueue(scores, q, group):
     prev_i, nxt_i, gamma = quantile_plan(n_total, q, np.float32)
     dev = scores.device
     state = torch.zeros(lib.sdrm_select_state_bytes(), dtype=torch.uint8, device=dev)
-    hists = torch.zeros((3, 2048), dtype=torch.int64, device=dev)
+    bf16 = _bf16(scores)
+    n_digits = len(_DIGITS_BF16 if bf16 else _DIGITS)
+    hist_entry, walk_entry = ((lib.sdrm_select_histogram_bf16, lib.sdrm_select_walk_bf16) if bf16
+                              else (lib.sdrm_select_histogram, lib.sdrm_select_walk))
+    hists = torch.zeros((n_digits, 2048), dtype=torch.int64, device=dev)
     st = _lib.stream_ptr()
     ld = scores.stride(0) if rows else n_cols
     _lib.check(lib.sdrm_select_begin(_lib.ptr(state), prev_i, nxt_i, st), "sdrm_select_begin")
     g32 = 1 if np.asarray(gamma).dtype == np.float32 else 0
-    for d in range(3):
-        _lib.check(lib.sdrm_select_histogram(_lib.ptr(scores), rows, n_cols, ld, _lib.ptr(state), d, _lib.ptr(hists[d]), st),
+    for d in range(n_digits):
+        _lib.check(hist_entry(_lib.ptr(scores), rows, n_cols, ld, _lib.ptr(state), d, _lib.ptr(hists[d]), st),
                    "sdrm_select_histogram")
         if dist is not None:
             dist.all_reduce(hists[d], group=group)
             if d == 0:      # the NaN count of the other ranks (bytes 16..24 of the state)
                 dist.all_reduce(state[16:24].view(torch.int64), group=group)
-        _lib.check(lib.sdrm_select_walk(_lib.ptr(hists[d]), _lib.ptr(state), d, float(gamma), g32, st), "sdrm_select_walk")
+        _lib.check(walk_entry(_lib.ptr(hists[d]), _lib.ptr(state), d, float(gamma), g32, st), "sdrm_select_walk")
     return state, g32
 
 
@@ -239,7 +261,8 @@ def _select_pack_device(scores, q, group, lower):
     wpr = (n_cols + 31) // 32
     bits = torch.empty((rows, wpr), dtype=torch.int32, device=scores.device)
     count = torch.zeros(1, dtype=torch.int64, device=scores.device)
-    _lib.check(lib.sdrm_select_threshold_pack(_lib.ptr(scores), rows, n_cols, scores.stride(0) if rows else n_cols, _lib.ptr(state),
+    entry = lib.sdrm_select_threshold_pack_bf16 if _bf16(scores) else lib.sdrm_select_threshold_pack
+    _lib.check(entry(_lib.ptr(scores), rows, n_cols, scores.stride(0) if rows else n_cols, _lib.ptr(state),
                                               1 if lower else 0, _lib.ptr(bits), wpr, _lib.ptr(count), _lib.stream_ptr()),
                "sdrm_select_threshold_pack")
     thr, fallback, nans = _read_state(state, g32)
@@ -255,6 +278,11 @@ def equal_sparsity_device(scores, sparsity, group=None, lower=False, host_walk=F
     (main.py:259-262).  With `group`, `scores` is this rank's row shard and the threshold is the GLOBAL quantile.
     A NaN score makes the threshold NaN (and every bit 0), like np.quantile.  host_walk=True forces the first implementation
     (histograms copied to the host between the passes), which is also the fallback of the device walk.
+
+    bfloat16 scores (sample_ddpm(..., out_dtype=torch.bfloat16)): the reference's rule applied to the ROUNDED scores, i.e.
+    thr = np.quantile(S.astype(np.float32).flatten(), q) and S >= thr.  Rounding to bfloat16 merges nearby scores, so the
+    threshold often lands on a value many scores share, and every one of them is kept: the matrix can hold more ones than the
+    binarisation of the float32 rows of the same seed (DESIGN.md section 3 gives the measured size of the effect).
     """
     _check(scores)
     q = (1 - sparsity) if lower else sparsity

@@ -115,9 +115,18 @@ def engine_for(diff_net, device=None):
     return eng
 
 
+def _check_out_dtype(out_dtype, out):
+    if out_dtype not in (torch.float32, torch.bfloat16):
+        raise ValueError(f"out_dtype must be torch.float32 or torch.bfloat16, got {out_dtype}")
+    if out is not None and out.dtype != out_dtype:
+        raise ValueError(f"out has dtype {out.dtype} but out_dtype is {out_dtype}")
+    return out_dtype
+
+
 @torch.no_grad()
 def sample_ddpm(n_sample, diff_net, vae_net, diff_latent_dim, noise_divider=1.0, timesteps=None, n_timesteps=None,
-                verbose=False, *, seed=None, row_offset=0, out=None, return_latent=False, reuse_packed=False, t_rows=None):
+                verbose=False, *, seed=None, row_offset=0, out=None, return_latent=False, reuse_packed=False, t_rows=None,
+                out_dtype=torch.float32):
     """Reverse diffusion in the VAE latent space + decode -> float32 logits [n_sample, N_ITEMS] on the GPU.
 
     timesteps='random' is the multi-resolution mode: row j runs only t_j ~ U{1..T-1} steps, t_j drawn from
@@ -127,8 +136,12 @@ def sample_ddpm(n_sample, diff_net, vae_net, diff_latent_dim, noise_divider=1.0,
     skips re-packing the weights when the parameter tensors are unchanged since the last call (the default re-packs: ~0.1 ms,
     and safe against in-place edits through `.data` that no version counter records), `t_rows` gives the multi-resolution
     chain lengths explicitly (row-sharded callers slice one global draw, sdrm_b200.distributed.sample_ddpm_sharded).
+    `out_dtype=torch.bfloat16` returns bfloat16 logits: each one the round-to-nearest-even bfloat16 of the float32 logit the
+    default would return for the same seed (half the bytes to keep, copy or gather; the latent stays float32).  An `out` tensor
+    must have dtype `out_dtype`.
     """
     start_time = time.time()
+    out_dtype = _check_out_dtype(out_dtype, out)
     diff_net.eval()
     vae_net.eval()
     dev = next(diff_net.parameters()).device
@@ -156,8 +169,10 @@ def sample_ddpm(n_sample, diff_net, vae_net, diff_latent_dim, noise_divider=1.0,
         row_ids = torch.from_numpy(order)
     latent = torch.empty((n_sample, L), dtype=torch.float32, device=dev) if return_latent else None
     if int(n_sample) == 0:
-        empty = torch.empty((0, eng.I), dtype=torch.float32, device=dev)
+        empty = torch.empty((0, eng.I), dtype=out_dtype, device=dev)
         return (empty, latent) if return_latent else empty
+    if out is None and out_dtype != torch.float32:
+        out = torch.empty((int(n_sample), eng.I), dtype=out_dtype, device=dev)
     samples = eng.sample(int(n_sample), row_offset=int(row_offset), t_start=t_start, row_ids=row_ids, seed=seed,
                          out=out, latent_out=latent)
     if verbose:
@@ -168,11 +183,16 @@ def sample_ddpm(n_sample, diff_net, vae_net, diff_latent_dim, noise_divider=1.0,
 
 @torch.no_grad()
 def sample_ddpm_host(n_sample, diff_net, vae_net, diff_latent_dim, noise_divider=1.0, timesteps=None, n_timesteps=None,
-                     verbose=False, *, seed=None, row_offset=0, host_out=None, chunk_rows=None):
+                     verbose=False, *, seed=None, row_offset=0, host_out=None, chunk_rows=None, out_dtype=None):
     """Full-resolution sample_ddpm whose result is delivered in (pinned) HOST memory — what main.py's
     `.detach().cpu().numpy()` consumes (main.py:171,175).  Rows are generated in chunks of whole CTA waves; the
     device->host copy of chunk c runs on a side stream while chunk c+1 is being computed, so the 4*I bytes per
-    user never wait for the chain.  Row content is identical to sample_ddpm(seed=..., row_offset=...)."""
+    user never wait for the chain.  Row content is identical to sample_ddpm(seed=..., row_offset=...).
+    A bfloat16 `host_out` or `out_dtype=torch.bfloat16` delivers bfloat16 rows (2*I bytes per user), identical to
+    sample_ddpm(..., out_dtype=torch.bfloat16); out_dtype defaults to host_out's dtype, else float32."""
+    if out_dtype is None:
+        out_dtype = host_out.dtype if host_out is not None else torch.float32
+    out_dtype = _check_out_dtype(out_dtype, host_out)
     diff_net.eval()
     vae_net.eval()
     dev = next(diff_net.parameters()).device
@@ -191,15 +211,15 @@ def sample_ddpm_host(n_sample, diff_net, vae_net, diff_latent_dim, noise_divider
         seed = int(torch.randint(0, 2 ** 62, (1,)).item())
     n_sample = int(n_sample)
     if host_out is None:
-        host_out = torch.empty((n_sample, eng.I), dtype=torch.float32, pin_memory=True)
+        host_out = torch.empty((n_sample, eng.I), dtype=out_dtype, pin_memory=True)
     if chunk_rows is None:
         sms = torch.cuda.get_device_properties(dev).multi_processor_count
         # one CTA wave per chunk: the device->host copy of a wave (57 GB/s) is shorter than its compute, so only the LAST
         # chunk's copy is exposed, and a one-wave chunk makes that tail as short as it gets
         chunk_rows = int(os.environ.get("SDRM_HOST_CHUNK_WAVES", "1")) * sms * 128
     bufs = getattr(eng, "_host_bufs", None)
-    if bufs is None or bufs[0].shape != (chunk_rows, eng.I):
-        bufs = [torch.empty((chunk_rows, eng.I), dtype=torch.float32, device=dev) for _ in range(2)]
+    if bufs is None or bufs[0].shape != (chunk_rows, eng.I) or bufs[0].dtype != out_dtype:
+        bufs = [torch.empty((chunk_rows, eng.I), dtype=out_dtype, device=dev) for _ in range(2)]
         eng._host_bufs = bufs
         eng._copy_stream = torch.cuda.Stream(dev)
     copy_stream = eng._copy_stream
