@@ -27,6 +27,10 @@ def build_parser():
     p.add_argument("--SDRM-timesteps", type=int, default=50, help="Number of timesteps to use for training SDRM")
     p.add_argument("--SDRM-noise-variance-diminisher", type=float, default=0.5,
                    help="Noise variance diminisher to use for training SDRM")
+    p.add_argument("--SDRM-sampling-steps", type=int, default=None,
+                   help="reverse steps of the sampling chain (strided over the training timesteps); default: all of them")
+    p.add_argument("--SDRM-eta", type=float, default=None,
+                   help="sample with DDIM at this noise scale in [0, 1] instead of DDPM; default: DDPM")
     p.add_argument("--MLP-hidden-layers", type=int, default=2, help="Number of hidden layers to use for training MLP")
     p.add_argument("--VAE-batch-size", type=int, default=500, help="Batch size to use for training VAE")
     p.add_argument("--VAE-hidden-layer-neurons", type=int, default=100,
@@ -93,10 +97,12 @@ def main(argv=None):
 
         print("Sampling Multi-resolution Data")
         M_SDRM = sample_ddpm(N_USERS, SDRM, VAE, args.MLP_latent_neurons, args.SDRM_noise_variance_diminisher,
-                             timesteps="random", n_timesteps=args.SDRM_timesteps, verbose=True)
+                             timesteps="random", n_timesteps=args.SDRM_timesteps, verbose=True,
+                             sampling_steps=args.SDRM_sampling_steps, eta=args.SDRM_eta)
         print("Sampling Full-resolution Data")
         F_SDRM = sample_ddpm(N_USERS, SDRM, VAE, args.MLP_latent_neurons, args.SDRM_noise_variance_diminisher,
-                             n_timesteps=args.SDRM_timesteps, verbose=True)
+                             n_timesteps=args.SDRM_timesteps, verbose=True,
+                             sampling_steps=args.SDRM_sampling_steps, eta=args.SDRM_eta)
         synth = {
             "M-SDRM": pd.DataFrame(equal_sparsity(M_SDRM, SPARSITY)),
             "F-SDRM": pd.DataFrame(equal_sparsity(F_SDRM, SPARSITY)),

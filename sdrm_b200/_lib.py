@@ -24,6 +24,8 @@ SIGNATURES = {
                               C.c_size_t, _P]),
     "sdrm_sample_bf16": (C.c_int, [_P, C.c_int64, C.c_int64, _P, _P, C.c_uint64, _P, _P, C.c_int64, _P, _P, _P, _P,
                                    C.c_size_t, _P]),
+    "sdrm_set_step_grid": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_float, _P]),
+    "sdrm_step_grid_size": (C.c_int, [_P]),
     "sdrm_last_launch_count": (C.c_int, [_P]),
     "sdrm_check_device_error": (C.c_int, [_P, _P]),
     "sdrm_probe_linear_workspace_bytes": (C.c_size_t, [C.c_int64, C.c_int, C.c_int]),

@@ -8,6 +8,7 @@
 
 #include <algorithm>
 #include <string>
+#include <vector>
 
 #include "../../include/sdrm_b200.h"
 #include "host_util.h"
@@ -201,6 +202,52 @@ __global__ void coef_kernel(const float* __restrict__ sched, int T, float nd, fl
   reinterpret_cast<float4*>(coef)[i] = c;
 }
 
+// Coefficient rows of a step grid (sdrm_set_step_grid) in coef_kernel's layout: row j (1 <= j <= S) is the jump
+// tau_j -> tau_{j-1} of the S-step chain, row 0 is zero.  tau [S+1] with tau_0 = 0; sched = b | a | ab as packed.
+//   mode 0 (strided DDPM): a span of one step is coef_kernel's row tau_j (same float32 expressions, so the full grid
+//     reproduces the packed table bit for bit); a longer span takes a' = prod a_t over (tau_{j-1}, tau_j] in float64 and
+//     c0 = (1 - a') / sqrt(1 - ab_{tau_j}), c1 = 1 / sqrt(a'), c2 = sqrt(1 - a') nd, rounded once.
+//   mode 1 (DDIM, eta): c1 = sqrt(ab_p / ab_c), c0 = sqrt(1 - ab_c) - sqrt(max(0, 1 - ab_p - sigma^2)) / c1, c2 = sigma nd with
+//     sigma = eta sqrt((1 - ab_p) / (1 - ab_c)) sqrt(1 - ab_c / ab_p), ab_p = 1 at tau_0; float64, rounded once.
+// The last step (j = 1) draws no noise in either mode.
+__global__ void grid_coef_kernel(const float* __restrict__ sched, int T, const int32_t* __restrict__ tau, int S, int mode,
+                                 float eta, float nd, float* __restrict__ coef) {
+  const int j = blockIdx.x * blockDim.x + threadIdx.x;
+  if (j > S) return;
+  const float *b_t = sched, *a_t = sched + (T + 1), *ab_t = sched + 2 * (T + 1);
+  float4 c = make_float4(0.f, 0.f, 0.f, 0.f);
+  if (j >= 1) {
+    const int tc = tau[j], tp = tau[j - 1];
+    if (mode == 0 && tc - tp == 1) {
+      const float b = b_t[tc], a = a_t[tc], ab = ab_t[tc];
+      c.x = (1.0f - a) / sqrtf(1.0f - ab);
+      c.y = 1.0f / sqrtf(a);
+      c.z = j > 1 ? sqrtf(b) * nd : 0.0f;
+    } else if (mode == 0) {
+      double ap = 1.0;
+      for (int t = tp + 1; t <= tc; ++t) ap *= static_cast<double>(a_t[t]);
+      c.x = static_cast<float>((1.0 - ap) / sqrt(1.0 - static_cast<double>(ab_t[tc])));
+      c.y = static_cast<float>(1.0 / sqrt(ap));
+      c.z = j > 1 ? static_cast<float>(sqrt(1.0 - ap) * static_cast<double>(nd)) : 0.0f;
+    } else {
+      const double abc = ab_t[tc], abp = tp == 0 ? 1.0 : static_cast<double>(ab_t[tp]);
+      const double sigma = static_cast<double>(eta) * sqrt((1.0 - abp) / (1.0 - abc)) * sqrt(fmax(0.0, 1.0 - abc / abp));
+      const double c1 = sqrt(abp / abc);
+      c.x = static_cast<float>(sqrt(1.0 - abc) - sqrt(fmax(0.0, 1.0 - abp - sigma * sigma)) / c1);
+      c.y = static_cast<float>(c1);
+      c.z = static_cast<float>(sigma * static_cast<double>(nd));
+    }
+  }
+  reinterpret_cast<float4*>(coef)[j] = c;
+}
+
+// rows tau_0 .. tau_S of a per-step bias table [T+1][ld] -> rows 0 .. S of the grid's table (same pitch): one block per row
+__global__ void grid_bias_kernel(const float* __restrict__ src, int ld, const int32_t* __restrict__ tau, float* __restrict__ dst) {
+  const float* s = src + static_cast<size_t>(tau[blockIdx.x]) * ld;
+  float* d = dst + static_cast<size_t>(blockIdx.x) * ld;
+  for (int c = threadIdx.x; c < ld; c += blockDim.x) d[c] = s[c];
+}
+
 }  // namespace sdrm
 
 // ------------------------------------------------------------------------------------------------
@@ -248,6 +295,13 @@ struct sdrm_handle {
   float *s_bias = nullptr;          // bias0 [T+1][64] | bh [64] | bo [64]
   float *s_b1 = nullptr;            // b1 [64] | b2 [I rounded up to 64]
   int engine_choice = 0;            // SDRM_OPT_ENGINE: 0 automatic, 1 tcgen05 layer engine, 2 small-chain kernel
+  // step grid (sdrm_set_step_grid): grid_S = 0 runs the packed full chain; else the chain has grid_S steps and reads the grid
+  // tables below (rows 0 .. grid_S; sized for T + 1 rows)
+  int grid_S = 0;
+  float* sched = nullptr;           // the packed schedule b | a | ab [3 (T+1)]
+  int32_t* grid_tau = nullptr;      // tau_0 = 0, tau_1 .. tau_S
+  float *grid_bias0 = nullptr, *grid_coef = nullptr;   // bias0 rows tau_j [T+1][np0]; coefficients [T+1][4]
+  float* grid_s_bias = nullptr;     // K6: bias0 rows tau_j [T+1][64]
   // decoder
   bool have_dec = false;
   int H = 0, I = 0;
@@ -263,6 +317,8 @@ static void free_den(sdrm_handle* h) {
   cudaFree(h->bias0); cudaFree(h->bh); cudaFree(h->bo); cudaFree(h->slopes); cudaFree(h->coef);
   cudaFree(h->s_den); cudaFree(h->s_bias);
   h->s_den = nullptr; h->s_bias = nullptr; h->small_den = false;
+  cudaFree(h->sched); cudaFree(h->grid_tau); cudaFree(h->grid_bias0); cudaFree(h->grid_coef); cudaFree(h->grid_s_bias);
+  h->sched = h->grid_bias0 = h->grid_coef = h->grid_s_bias = nullptr; h->grid_tau = nullptr; h->grid_S = 0;
   h->w0 = h->wh = h->wo = nullptr;
   h->bias0 = h->bh = h->bo = h->slopes = h->coef = nullptr;
   h->have_den = false;
@@ -483,8 +539,14 @@ int sdrm_denoiser_pack(sdrm_handle* h, const float* d_We, const float* d_be, con
     SDRM_CUDA(cudaMalloc(&h->bo, sizeof(float) * h->npo));
     SDRM_CUDA(cudaMalloc(&h->slopes, sizeof(float) * 2));
     SDRM_CUDA(cudaMalloc(&h->coef, sizeof(float) * 4 * (T + 1)));
+    SDRM_CUDA(cudaMalloc(&h->sched, sizeof(float) * 3 * (T + 1)));
+    SDRM_CUDA(cudaMalloc(&h->grid_tau, sizeof(int32_t) * (T + 1)));
+    SDRM_CUDA(cudaMalloc(&h->grid_bias0, sizeof(float) * (T + 1) * h->np0));
+    SDRM_CUDA(cudaMalloc(&h->grid_coef, sizeof(float) * 4 * (T + 1)));
   }
+  h->grid_S = 0;   // new weights or schedule: the full chain until a grid is set again
   h->nd = noise_divider;
+  SDRM_CUDA(cudaMemcpyAsync(h->sched, d_sched, sizeof(float) * 3 * (T + 1), cudaMemcpyDeviceToDevice, st));
   launch_pack_weight(d_W0, D, L, L + T, 0, h->w0, nullptr, h->g0, st);
   if (nh > 0) launch_pack_weight(d_Wh, D, D, D, 0, h->wh, nullptr, h->gh, st);
   launch_pack_weight(d_Wo, L, D, D, 0, h->wo, nullptr, h->go, st);
@@ -505,6 +567,7 @@ int sdrm_denoiser_pack(sdrm_handle* h, const float* d_We, const float* d_be, con
     if (!h->s_den) {
       SDRM_CUDA(cudaMalloc(&h->s_den, 3 * img * sizeof(__nv_bfloat16)));
       SDRM_CUDA(cudaMalloc(&h->s_bias, sizeof(float) * 64 * (T + 3)));
+      SDRM_CUDA(cudaMalloc(&h->grid_s_bias, sizeof(float) * 64 * (T + 1)));
     }
     pack_small_weight_kernel<<<18, 256, 0, st>>>(d_W0, D, L, L + T, 0, 64, h->s_den, nullptr);
     pack_small_weight_kernel<<<18, 256, 0, st>>>(nh > 0 ? d_Wh : d_Wo, nh > 0 ? D : 0, nh > 0 ? D : 0, D, 0, 64, h->s_den + img, nullptr);
@@ -628,6 +691,8 @@ static int sample_impl(sdrm_handle* h, int64_t n, int64_t row_offset, const int3
   if (!d_workspace) return sdrm_fail(SDRM_ERR_BAD_ARG, "sdrm_sample: null workspace");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   SDRM_CUDA(cudaSetDevice(h->device));
+  const bool on_grid = h->grid_S > 0;
+  const int steps = on_grid ? h->grid_S : h->T;   // reverse steps of this launch (t_start entries are clamped to [0, steps])
   // ---- small denoisers (every width <= 64): the register / shared-memory resident chain (K6) instead of the tcgen05 engine
   const bool small_ok = h->small_den && h->small_dec && h->D <= SMALL_MAX && h->H <= SMALL_MAX;
   if (h->engine_choice == 2 && !small_ok) return sdrm_fail(SDRM_ERR_UNSUPPORTED, "sdrm_sample: the small-chain kernel needs every width <= 64");
@@ -639,10 +704,10 @@ static int sample_impl(sdrm_handle* h, int64_t n, int64_t row_offset, const int3
     S.w0 = h->s_den; S.wh = h->s_den + img; S.wo = h->s_den + 2 * img;
     S.w1_hi = h->s_dec1; S.w1_lo = h->s_dec1 + img;
     S.w2_hi = h->s_dec2; S.w2_lo = h->s_dec2 + img2;
-    S.bias0 = h->s_bias; S.bias0_ld = 64;
+    S.bias0 = on_grid ? h->grid_s_bias : h->s_bias; S.bias0_ld = 64;
     S.bh = h->s_bias + 64 * (h->T + 1); S.bo = h->s_bias + 64 * (h->T + 2); S.b1 = h->s_b1; S.b2 = h->s_b1 + 64;
-    S.slopes = h->slopes; S.coef = h->coef;
-    S.T = h->T; S.L = h->L; S.H = h->H; S.I = h->I; S.nh = h->nh;
+    S.slopes = h->slopes; S.coef = on_grid ? h->grid_coef : h->coef;
+    S.T = steps; S.L = h->L; S.H = h->H; S.I = h->I; S.nh = h->nh;
     S.n_rows = n; S.row_offset = row_offset; S.ld_logits = ld_logits;
     S.t_start = d_t_start; S.row_ids = d_row_ids; S.x0_out = d_x0_out; S.logits = d_logits;
     S.inj_xT = d_inj_xT; S.inj_z = d_inj_z; S.inj_mask = d_inj_mask; S.seed = seed;
@@ -720,17 +785,17 @@ static int sample_impl(sdrm_handle* h, int64_t n, int64_t row_offset, const int3
   const Geom& G1 = split_geom ? h->s1 : h->g1;
   const Geom& G2 = split_geom ? h->s2 : h->g2;
   int l = 0;
-  fill(P.step[l++], split_geom ? h->w0s : h->w0, h->bias0, h->slopes, h->np0, G0, 1, EPI_PRELU, 0, 0, 0, 0);
+  fill(P.step[l++], split_geom ? h->w0s : h->w0, on_grid ? h->grid_bias0 : h->bias0, h->slopes, h->np0, G0, 1, EPI_PRELU, 0, 0, 0, 0);
   for (int j = 0; j < h->nh; ++j) fill(P.step[l++], split_geom ? h->whs : h->wh, h->bh, h->slopes + 1, 0, GH, 1, EPI_PRELU, 0, 0, 0, 0);
   fill(P.step[l++], split_geom ? h->wos : h->wo, h->bo, nullptr, 0, GO, 1, EPI_POSTERIOR, 0, 0, 0, 0);
   P.n_step = l;
   fill(P.dec[0], (split_geom && h->w1s) ? h->w1s : h->w1, h->b1, nullptr, 0, G1, 3, EPI_TANH_SPLIT, 0, 2, 1, 3);
   fill(P.dec[1], (split_geom && h->w2s) ? h->w2s : h->w2, h->b2, nullptr, 0, G2, 3, EPI_LINEAR_OUT, 1, 3, 0, 0);
   P.n_dec = 2;
-  P.T = h->T; P.L = h->L; P.Lg16 = (h->L + 15) / 16;
+  P.T = steps; P.L = h->L; P.Lg16 = (h->L + 15) / 16;
   P.preloaded_input = 0;
   P.n_rows = n; P.row_offset = row_offset;
-  P.coef = h->coef;
+  P.coef = on_grid ? h->grid_coef : h->coef;
   P.t_start = d_t_start;
   P.row_ids = d_row_ids;
   P.x0_out = d_x0_out;
@@ -790,7 +855,7 @@ static int sample_impl(sdrm_handle* h, int64_t n, int64_t row_offset, const int3
   // chain layer's epilogue rewrites completely (64-column blocks below the narrowest written width), so a partly written
   // last k-block keeps the zero padding it got at kernel start.
   P.discard_kb = 0;
-  if (cluster >= 2 && !h->no_discard && h->T >= 2 && d_t_start == nullptr) {   // (the discard warp counts P.T steps per tile)
+  if (cluster >= 2 && !h->no_discard && steps >= 2 && d_t_start == nullptr) {   // (the discard warp counts P.T steps per tile)
     const int written = std::min(std::min(h->g0.Np, h->nh > 0 ? h->gh.Np : h->g0.Np), std::min(h->go.Np, P.Lg16 * 16));
     const int kb_read = std::min(std::min(h->g0.KB, h->nh > 0 ? h->gh.KB : h->g0.KB), h->go.KB);
     P.discard_kb = std::max(0, std::min(written / KBLK, kb_read));
@@ -847,6 +912,34 @@ int sdrm_sample_bf16(sdrm_handle* h, int64_t n, int64_t row_offset, const int32_
   return sample_impl(h, n, row_offset, d_t_start, d_row_ids, seed, d_x0_out, d_logits, ld_logits, true, d_inj_xT, d_inj_z,
                      d_inj_mask, d_workspace, workspace_bytes, stream);
 }
+
+int sdrm_set_step_grid(sdrm_handle* h, const int32_t* timesteps, int S, int mode, float eta, void* stream) {
+  if (!h) return sdrm_fail(SDRM_ERR_BAD_ARG, "sdrm_set_step_grid: null handle");
+  if (!h->have_den) return sdrm_fail(SDRM_ERR_STATE, "sdrm_set_step_grid: pack the denoiser first");
+  if (S < 0 || S > h->T) return sdrm_fail(SDRM_ERR_BAD_ARG, "sdrm_set_step_grid: S must lie in [0, T]");
+  if (mode != 0 && mode != 1) return sdrm_fail(SDRM_ERR_BAD_ARG, "sdrm_set_step_grid: mode must be 0 (strided DDPM) or 1 (DDIM)");
+  if (!(eta >= 0.0f && eta <= 1.0f)) return sdrm_fail(SDRM_ERR_BAD_ARG, "sdrm_set_step_grid: eta must lie in [0, 1]");
+  if (S == 0) { h->grid_S = 0; return SDRM_OK; }
+  if (!timesteps) return sdrm_fail(SDRM_ERR_BAD_ARG, "sdrm_set_step_grid: null timesteps");
+  std::vector<int32_t> tau(static_cast<size_t>(S) + 1, 0);
+  for (int j = 0; j < S; ++j) {
+    if (timesteps[j] < 1 || timesteps[j] > h->T || timesteps[j] <= tau[j])
+      return sdrm_fail(SDRM_ERR_BAD_ARG, "sdrm_set_step_grid: timesteps must increase strictly within [1, T]");
+    tau[j + 1] = timesteps[j];
+  }
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  SDRM_CUDA(cudaSetDevice(h->device));
+  // (pageable source: the copy is staged before this call returns)
+  SDRM_CUDA(cudaMemcpyAsync(h->grid_tau, tau.data(), sizeof(int32_t) * (S + 1), cudaMemcpyHostToDevice, st));
+  grid_coef_kernel<<<(S + 1 + 127) / 128, 128, 0, st>>>(h->sched, h->T, h->grid_tau, S, mode, eta, h->nd, h->grid_coef);
+  grid_bias_kernel<<<S + 1, 256, 0, st>>>(h->bias0, h->np0, h->grid_tau, h->grid_bias0);
+  if (h->small_den) grid_bias_kernel<<<S + 1, 64, 0, st>>>(h->s_bias, 64, h->grid_tau, h->grid_s_bias);
+  SDRM_CUDA(cudaGetLastError());
+  h->grid_S = S;
+  return SDRM_OK;
+}
+
+int sdrm_step_grid_size(const sdrm_handle* h) { return h ? h->grid_S : 0; }
 
 int sdrm_last_launch_count(const sdrm_handle* h) { return h ? h->last_launches : 0; }
 int sdrm_last_resident_mode(const sdrm_handle* h) { return h ? h->last_resident : 0; }

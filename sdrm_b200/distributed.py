@@ -26,7 +26,8 @@ def shard_bounds(n, rank, world):
 
 
 def sample_ddpm_sharded(n_sample, diff_net, vae_net, diff_latent_dim, noise_divider=1.0, timesteps=None,
-                        n_timesteps=None, *, seed, group=None, gather=False, sparsity=None, sampler=None, out_dtype=None):
+                        n_timesteps=None, *, seed, group=None, gather=False, sparsity=None, sampler=None, out_dtype=None,
+                        sampling_steps=None, eta=None):
     """Each rank samples its contiguous block of the n_sample rows (same `seed` on every rank; the Philox streams are keyed
     by the global row id, so in full-resolution mode the union of the blocks is bit-identical to a single-GPU run).
 
@@ -43,6 +44,7 @@ def sample_ddpm_sharded(n_sample, diff_net, vae_net, diff_latent_dim, noise_divi
     out_dtype=torch.bfloat16 samples bfloat16 rows (the rounded float32 rows, sample_ddpm's out_dtype): gather=False / True then
     return / gather bfloat16 blocks (half the NVLink bytes), and gather="bits" binarises the bfloat16 rows (sparsify.py: ties
     at the threshold can keep a few more ones than the float32 rows would).
+    sampling_steps / eta choose a fewer-step chain (sample_ddpm); multi-resolution rows map their drawn t_j onto its grid.
     An empty block (more ranks than rows) is legal: the rank still takes part in the collectives."""
     import numpy as np
     if sampler is None:
@@ -56,6 +58,8 @@ def sample_ddpm_sharded(n_sample, diff_net, vae_net, diff_latent_dim, noise_divi
         kw["t_rows"] = t_all[lo:hi]
     if out_dtype is not None:
         kw["out_dtype"] = out_dtype
+    if sampling_steps is not None or eta is not None:
+        kw.update(sampling_steps=sampling_steps, eta=eta)
     rows = sampler(hi - lo, diff_net, vae_net, diff_latent_dim, noise_divider, timesteps=timesteps,
                    n_timesteps=n_timesteps, seed=seed, row_offset=lo, **kw)
     if not gather or world == 1:

@@ -29,6 +29,7 @@ class SamplerEngine:
         self._den_key = None
         self._dec_key = None
         self._ws = None
+        self._grid = None          # (timesteps, eta) of the step grid set on the handle; None = the full chain
         self.T = self.L = self.I = None
 
     def __del__(self):
@@ -78,7 +79,34 @@ class SamplerEngine:
         _lib.check(rc, "sdrm_denoiser_pack")
         self._keepalive_den = (ts, sched)
         self._den_key = key
+        self._grid = None          # (the pack resets the handle to the full chain)
         self.T, self.L = T, L
+
+    @property
+    def steps(self):
+        """Reverse steps of the next sample(): S of the step grid, else T."""
+        return self.T if self._grid is None else len(self._grid[0])
+
+    def set_step_grid(self, timesteps=None, eta=None):
+        """Run the chain on the timesteps 1 <= tau_1 < ... < tau_S <= T (a sequence of ints) instead of all T: strided DDPM when
+        eta is None, DDIM with noise scale eta in [0, 1] otherwise (include/sdrm_b200.h, sdrm_set_step_grid).  timesteps=None
+        restores the full chain.  Stays set until the next call or the next pack of the denoiser; a call that repeats the grid
+        already set launches nothing.  t_start entries of sample() are then grid steps in [0, S], and injected z / keep slabs
+        are [S+1, n, L]."""
+        if self._den_key is None:
+            raise _lib.SdrmError("pack_denoiser must be called before set_step_grid")
+        grid = None if timesteps is None else (tuple(int(t) for t in timesteps), None if eta is None else float(eta))
+        if grid == self._grid:
+            return
+        if grid is None:
+            rc = self.lib.sdrm_set_step_grid(self.handle, None, 0, 0, 0.0, _lib.stream_ptr())
+        else:
+            tau, e = grid
+            arr = (C.c_int32 * len(tau))(*tau)
+            rc = self.lib.sdrm_set_step_grid(self.handle, arr, len(tau), 0 if e is None else 1, 0.0 if e is None else e,
+                                             _lib.stream_ptr())
+        _lib.check(rc, "sdrm_set_step_grid")
+        self._grid = grid
 
     def pack_decoder(self, vae_net, force=True):
         W1, b1 = vae_net.decoder[0].weight, vae_net.decoder[0].bias
@@ -121,8 +149,8 @@ class SamplerEngine:
         if t_start is not None:
             if t_start.numel() != n:
                 raise ValueError("t_start must have n entries")
-            if t_start.device.type == "cpu" and t_start.numel() and (int(t_start.min()) < 0 or int(t_start.max()) > self.T):
-                raise ValueError(f"t_start entries must lie in [0, T={self.T}]")   # (device tensors are clamped by the kernel)
+            if t_start.device.type == "cpu" and t_start.numel() and (int(t_start.min()) < 0 or int(t_start.max()) > self.steps):
+                raise ValueError(f"t_start entries must lie in [0, {self.steps}] (the chain's steps)")   # (device tensors are clamped by the kernel)
             t_start = t_start.to(self.device, torch.int32).contiguous()
         if row_ids is not None:
             row_ids = row_ids.to(self.device, torch.int32).contiguous()

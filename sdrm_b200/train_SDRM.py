@@ -6,6 +6,7 @@ hyperparameter_search.py and the SVD / MLP / NeuMF benchmarks can switch by chan
     train_SDRM(dl, N_ITEMS, ..., verbose=False) -> (DIFF, variational_ae)       (train_SDRM.py:271-340)
     sample_ddpm(n_sample, diff_net, vae_net, diff_latent_dim, noise_divider=1.0,
                 timesteps=None, n_timesteps=None, verbose=False) -> Tensor[n, N_ITEMS] on the device   (27-63)
+                (keyword-only extras, among them sampling_steps / eta for a fewer-step chain)
     SDRM, VAE, train_variational_autoencoder, perturb_input, denoise_add_noise, checkpoint, resume
 
 The sampling chain and the diffusion training step run in hand-written sm_100a kernels through the C ABI
@@ -98,6 +99,52 @@ def _resolve_steps(diff_net, timesteps, n_timesteps):
     return T, random_mode
 
 
+def step_grid(T, sampling_steps):
+    """Timesteps 1 <= tau_1 < ... < tau_S <= T of a fewer-step chain over the T-step schedule, as an int32 array.
+
+    An int S in [1, T] gives tau_j = ceil(j T / S), so tau_S = T and S = T is the full chain; a sequence of ints is taken as an
+    explicit grid and must increase strictly within [1, T]."""
+    T = int(T)
+    if isinstance(sampling_steps, (bool, np.bool_)):
+        raise ValueError(f"sampling_steps must be an int or a sequence of ints, got {sampling_steps!r}")
+    if isinstance(sampling_steps, (int, np.integer)):
+        S = int(sampling_steps)
+        if not 1 <= S <= T:
+            raise ValueError(f"sampling_steps={S} must lie in [1, T={T}]")
+        j = np.arange(1, S + 1, dtype=np.int64)
+        return ((j * T + S - 1) // S).astype(np.int32)
+    if isinstance(sampling_steps, torch.Tensor):
+        sampling_steps = sampling_steps.tolist()
+    try:
+        vals = list(sampling_steps)
+    except TypeError:
+        raise ValueError(f"sampling_steps must be an int or a sequence of ints, got {sampling_steps!r}") from None
+    if not vals or not all(isinstance(v, (int, np.integer)) and not isinstance(v, (bool, np.bool_)) for v in vals):
+        raise ValueError("an explicit sampling_steps grid must be a non-empty sequence of ints")
+    tau = np.asarray(vals, dtype=np.int64)
+    if tau[0] < 1 or tau[-1] > T or (np.diff(tau) <= 0).any():
+        raise ValueError(f"an explicit sampling_steps grid must increase strictly within [1, T={T}], got {vals}")
+    return tau.astype(np.int32)
+
+
+def grid_start_steps(t, timesteps):
+    """Grid step at which a multi-resolution row with start timestep t_j enters a fewer-step chain: s_j = #{k >= 1 : tau_k <= t_j},
+    the index of the largest grid timestep not above t_j (0: the row runs no step and decodes x_T).  On the full grid s_j = t_j."""
+    return np.searchsorted(np.asarray(timesteps), np.asarray(t), side="right").astype(np.int32)
+
+
+def resolve_step_grid(T, sampling_steps=None, eta=None):
+    """sample_ddpm's sampling_steps / eta -> (timesteps, eta) for SamplerEngine.set_step_grid; (None, None) is the reference
+    chain on all T steps.  eta=None is strided DDPM; eta in [0, 1] is DDIM, on the full grid when sampling_steps is None."""
+    if eta is not None:
+        if isinstance(eta, (bool, np.bool_)) or not isinstance(eta, (int, float, np.integer, np.floating)) or not 0.0 <= float(eta) <= 1.0:
+            raise ValueError(f"eta must be a number in [0, 1], got {eta!r}")
+        eta = float(eta)
+    if sampling_steps is None:
+        return (None, None) if eta is None else (step_grid(T, T), eta)
+    return step_grid(T, sampling_steps), eta
+
+
 def _resolve_schedule(diff_net, T, device):
     sched = getattr(diff_net, "sdrm_schedule", None)
     if sched is None and b_t is not None and b_t.numel() == T + 1:
@@ -126,7 +173,7 @@ def _check_out_dtype(out_dtype, out):
 @torch.no_grad()
 def sample_ddpm(n_sample, diff_net, vae_net, diff_latent_dim, noise_divider=1.0, timesteps=None, n_timesteps=None,
                 verbose=False, *, seed=None, row_offset=0, out=None, return_latent=False, reuse_packed=False, t_rows=None,
-                out_dtype=torch.float32):
+                out_dtype=torch.float32, sampling_steps=None, eta=None):
     """Reverse diffusion in the VAE latent space + decode -> float32 logits [n_sample, N_ITEMS] on the GPU.
 
     timesteps='random' is the multi-resolution mode: row j runs only t_j ~ U{1..T-1} steps, t_j drawn from
@@ -139,6 +186,17 @@ def sample_ddpm(n_sample, diff_net, vae_net, diff_latent_dim, noise_divider=1.0,
     `out_dtype=torch.bfloat16` returns bfloat16 logits: each one the round-to-nearest-even bfloat16 of the float32 logit the
     default would return for the same seed (half the bytes to keep, copy or gather; the latent stays float32).  An `out` tensor
     must have dtype `out_dtype`.
+
+    Fewer-step sampling (the defaults run the reference's chain on all T steps):
+      `sampling_steps=S` (an int in [1, T]) runs S reverse steps on the timesteps tau_j = ceil(j T / S); a sequence of ints is
+      an explicit grid 1 <= tau_1 < ... < tau_S <= T.  Step j feeds the denoiser the time embedding of tau_j.
+      `eta=None` (strided DDPM) applies denoise_add_noise with the jump's schedule: a' = prod a_t over (tau_{j-1}, tau_j],
+      x' = (x - (1 - a') / sqrt(1 - ab_{tau_j}) eps) / sqrt(a') + sqrt(1 - a') noise_divider z.
+      `eta` in [0, 1] takes the DDIM update instead (eta = 0: no noise added; eta alone runs DDIM on all T steps).
+      Both read the denoiser's output as the noise eps, as the reference's denoise_add_noise does.  SDRM's denoiser applies
+      dropout on every forward, so even eta = 0 is random through the keep masks.  With timesteps='random' the drawn t_j maps
+      to grid step s_j = #{k : tau_k <= t_j} (grid_start_steps).  Step j draws the random streams of step index j, so x_T is
+      the default call's.  Sample quality against S and eta is not characterised here.
     """
     start_time = time.time()
     out_dtype = _check_out_dtype(out_dtype, out)
@@ -148,6 +206,7 @@ def sample_ddpm(n_sample, diff_net, vae_net, diff_latent_dim, noise_divider=1.0,
     if dev.type != "cuda":
         raise _lib.SdrmError("sample_ddpm: the denoiser must live on a CUDA device (no CPU fallback)")
     T, random_mode = _resolve_steps(diff_net, timesteps, n_timesteps)
+    grid = resolve_step_grid(T, sampling_steps, eta)
     lt = diff_net.layer_tensors()
     L = lt["W0"].shape[1] - T
     if int(diff_latent_dim) != L:
@@ -155,6 +214,7 @@ def sample_ddpm(n_sample, diff_net, vae_net, diff_latent_dim, noise_divider=1.0,
     eng = engine_for(diff_net, dev)
     eng.pack_denoiser(diff_net, _resolve_schedule(diff_net, T, dev), noise_divider, force=not reuse_packed)
     eng.pack_decoder(vae_net, force=not reuse_packed)
+    eng.set_step_grid(*grid)
     if seed is None:
         seed = int(torch.randint(0, 2 ** 62, (1,)).item())
     t_start = row_ids = None
@@ -164,6 +224,8 @@ def sample_ddpm(n_sample, diff_net, vae_net, diff_latent_dim, noise_divider=1.0,
         t_np = (np.random.randint(1, T, size=int(n_sample)) if t_rows is None else np.asarray(t_rows)).astype(np.int32)
         if t_np.shape != (int(n_sample),):
             raise ValueError("t_rows must have n_sample entries")
+        if grid[0] is not None:
+            t_np = grid_start_steps(t_np, grid[0])
         order = np.argsort(-t_np, kind="stable").astype(np.int32)  # long chains first: tiles finish together
         t_start = torch.from_numpy(t_np[order])
         row_ids = torch.from_numpy(order)
@@ -183,13 +245,15 @@ def sample_ddpm(n_sample, diff_net, vae_net, diff_latent_dim, noise_divider=1.0,
 
 @torch.no_grad()
 def sample_ddpm_host(n_sample, diff_net, vae_net, diff_latent_dim, noise_divider=1.0, timesteps=None, n_timesteps=None,
-                     verbose=False, *, seed=None, row_offset=0, host_out=None, chunk_rows=None, out_dtype=None):
+                     verbose=False, *, seed=None, row_offset=0, host_out=None, chunk_rows=None, out_dtype=None,
+                     sampling_steps=None, eta=None):
     """Full-resolution sample_ddpm whose result is delivered in (pinned) HOST memory — what main.py's
     `.detach().cpu().numpy()` consumes (main.py:171,175).  Rows are generated in chunks of whole CTA waves; the
     device->host copy of chunk c runs on a side stream while chunk c+1 is being computed, so the 4*I bytes per
     user never wait for the chain.  Row content is identical to sample_ddpm(seed=..., row_offset=...).
     A bfloat16 `host_out` or `out_dtype=torch.bfloat16` delivers bfloat16 rows (2*I bytes per user), identical to
-    sample_ddpm(..., out_dtype=torch.bfloat16); out_dtype defaults to host_out's dtype, else float32."""
+    sample_ddpm(..., out_dtype=torch.bfloat16); out_dtype defaults to host_out's dtype, else float32.
+    `sampling_steps` / `eta` choose a fewer-step chain exactly as in sample_ddpm."""
     if out_dtype is None:
         out_dtype = host_out.dtype if host_out is not None else torch.float32
     out_dtype = _check_out_dtype(out_dtype, host_out)
@@ -201,12 +265,14 @@ def sample_ddpm_host(n_sample, diff_net, vae_net, diff_latent_dim, noise_divider
     T, random_mode = _resolve_steps(diff_net, timesteps, n_timesteps)
     if random_mode:
         raise NotImplementedError("sample_ddpm_host streams full-resolution rows; use sample_ddpm for timesteps='random'")
+    grid = resolve_step_grid(T, sampling_steps, eta)
     L = diff_net.layer_tensors()["W0"].shape[1] - T
     if int(diff_latent_dim) != L:
         raise ValueError(f"diff_latent_dim={diff_latent_dim} but the denoiser works on {L} latent columns")
     eng = engine_for(diff_net, dev)
     eng.pack_denoiser(diff_net, _resolve_schedule(diff_net, T, dev), noise_divider)
     eng.pack_decoder(vae_net)
+    eng.set_step_grid(*grid)
     if seed is None:
         seed = int(torch.randint(0, 2 ** 62, (1,)).item())
     n_sample = int(n_sample)

@@ -1,4 +1,7 @@
-"""End-to-end quality run of THIS repo on the GPU: same loop, hyper-parameters and evaluator settings as tools/ref_e2e.py."""
+"""End-to-end quality run of THIS repo on the GPU: same loop, hyper-parameters and evaluator settings as tools/ref_e2e.py.
+
+  python tools/our_e2e.py [runs] [only_synth] [out] [json overrides] [--sampling-steps S] [--eta X]
+--sampling-steps / --eta sample F-SDRM and M-SDRM on a fewer-step chain (sample_ddpm's sampling_steps / eta); default: all T steps."""
 import json, os, sys, time
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, pandas as pd, torch
@@ -7,6 +10,12 @@ from sdrm_b200 import evaluators
 from sdrm_b200.data import SparseDataset, load_data, sparse_batch_collate
 from sdrm_b200.train_SDRM import sample_ddpm, train_SDRM
 
+GRID = {}
+for flag, key, conv in (("--sampling-steps", "sampling_steps", int), ("--eta", "eta", float)):
+    if flag in sys.argv:
+        i = sys.argv.index(flag)
+        GRID[key] = conv(sys.argv[i + 1])
+        del sys.argv[i:i + 2]
 runs = int(sys.argv[1]) if len(sys.argv) > 1 else 5
 only_synth = (sys.argv[2] == "1") if len(sys.argv) > 2 else True
 out_path = sys.argv[3] if len(sys.argv) > 3 else "gpurun_out/e2e_ours_ml100k.jsonl"
@@ -26,12 +35,12 @@ for run in range(runs):
                            noise_divider=A["nd"], VAE_DIR_PATH="/tmp/our_temp_vae", TRAIN_PARTIAL_VALID_DATA=TPV, VALID_DATA=VALID,
                            OPTIMIZATION_OBJECTIVE="Recall@10", verbose=False)
     torch.cuda.synchronize()
-    res = {"impl": "sdrm_b200", "run": run, "train_s": round(time.time() - t0, 1), "only_synthetic": only_synth}
+    res = {"impl": "sdrm_b200", "run": run, "train_s": round(time.time() - t0, 1), "only_synthetic": only_synth, **GRID}
     t1 = time.time()
     from sdrm_b200.sparsify import equal_sparsity_device
-    M = sample_ddpm(N_USERS, DIFF, VAE, A["L"], A["nd"], timesteps="random", n_timesteps=A["T"])
+    M = sample_ddpm(N_USERS, DIFF, VAE, A["L"], A["nd"], timesteps="random", n_timesteps=A["T"], **GRID)
     torch.cuda.synchronize(); res["sample_random_s"] = round(time.time() - t1, 4); t1 = time.time()
-    F = sample_ddpm(N_USERS, DIFF, VAE, A["L"], A["nd"], n_timesteps=A["T"])
+    F = sample_ddpm(N_USERS, DIFF, VAE, A["L"], A["nd"], n_timesteps=A["T"], **GRID)
     torch.cuda.synchronize(); res["sample_full_s"] = round(time.time() - t1, 4)
     V = VAE.sample(N_USERS)
     for name, S in (("F-SDRM", F), ("M-SDRM", M), ("MultiVAE++", V)):
