@@ -21,7 +21,7 @@ import torch
 import torch.optim as optim
 from torch.nn import functional as F
 
-from . import _lib, metrics, training
+from . import _lib, metrics, recommend, training
 from .engine import SamplerEngine
 from .models import SDRM, VAE, default_device, make_schedule  # noqa: F401  (re-exported)
 
@@ -173,7 +173,7 @@ def _check_out_dtype(out_dtype, out):
 @torch.no_grad()
 def sample_ddpm(n_sample, diff_net, vae_net, diff_latent_dim, noise_divider=1.0, timesteps=None, n_timesteps=None,
                 verbose=False, *, seed=None, row_offset=0, out=None, return_latent=False, reuse_packed=False, t_rows=None,
-                out_dtype=torch.float32, sampling_steps=None, eta=None):
+                out_dtype=torch.float32, sampling_steps=None, eta=None, topk=None, exclude=None):
     """Reverse diffusion in the VAE latent space + decode -> float32 logits [n_sample, N_ITEMS] on the GPU.
 
     timesteps='random' is the multi-resolution mode: row j runs only t_j ~ U{1..T-1} steps, t_j drawn from
@@ -197,9 +197,19 @@ def sample_ddpm(n_sample, diff_net, vae_net, diff_latent_dim, noise_divider=1.0,
       dropout on every forward, so even eta = 0 is random through the keep masks.  With timesteps='random' the drawn t_j maps
       to grid step s_j = #{k : tau_k <= t_j} (grid_start_steps).  Step j draws the random streams of step index j, so x_T is
       the default call's.  Sample quality against S and eta is not characterised here.
+
+    Top-K recommendation (the default returns the dense rows):
+      `topk=k` (an int in [1, min(256, N_ITEMS)]) returns `(values [n_sample, k], indices int64 [n_sample, k])` instead of the
+      dense logits: per row the k highest logits by descending score, ties to the lower item index, computed on the device from
+      the rows this call samples (recommend.recommend_topk; `out` / `out_dtype` still choose the dense buffer and the dtype of
+      the values).  `exclude=(indptr, indices)` is the users' history in CSR form (int64[n_sample + 1], int32[nnz], on the
+      denoiser's device): row j never recommends an item of indices[indptr[j]:indptr[j + 1]].  With return_latent the result is
+      `((values, indices), latent)`.  A row with fewer than k items outside its history raises ValueError after the sampling.
     """
     start_time = time.time()
     out_dtype = _check_out_dtype(out_dtype, out)
+    if topk is None and exclude is not None:
+        raise ValueError("exclude= needs topk=")
     diff_net.eval()
     vae_net.eval()
     dev = next(diff_net.parameters()).device
@@ -215,6 +225,15 @@ def sample_ddpm(n_sample, diff_net, vae_net, diff_latent_dim, noise_divider=1.0,
     eng.pack_denoiser(diff_net, _resolve_schedule(diff_net, T, dev), noise_divider, force=not reuse_packed)
     eng.pack_decoder(vae_net, force=not reuse_packed)
     eng.set_step_grid(*grid)
+    if topk is not None:
+        topk = recommend.check_k(topk, eng.I)
+        if exclude is None:
+            exclude = (torch.zeros(int(n_sample) + 1, dtype=torch.int64, device=dev), torch.empty(0, dtype=torch.int32, device=dev))
+        if not isinstance(exclude, (tuple, list)) or len(exclude) != 2:
+            raise TypeError("exclude must be a pair (indptr int64[n_sample + 1], indices int32[nnz])")
+        exclude = recommend.check_history(exclude[0], exclude[1], int(n_sample))
+        if exclude[0].device != dev or exclude[1].device != dev:
+            raise ValueError(f"exclude tensors must be on {dev}, the denoiser's device")
     if seed is None:
         seed = int(torch.randint(0, 2 ** 62, (1,)).item())
     t_start = row_ids = None
@@ -232,11 +251,15 @@ def sample_ddpm(n_sample, diff_net, vae_net, diff_latent_dim, noise_divider=1.0,
     latent = torch.empty((n_sample, L), dtype=torch.float32, device=dev) if return_latent else None
     if int(n_sample) == 0:
         empty = torch.empty((0, eng.I), dtype=out_dtype, device=dev)
+        if topk is not None:
+            empty = (torch.empty((0, topk), dtype=out_dtype, device=dev), torch.empty((0, topk), dtype=torch.int64, device=dev))
         return (empty, latent) if return_latent else empty
     if out is None and out_dtype != torch.float32:
         out = torch.empty((int(n_sample), eng.I), dtype=out_dtype, device=dev)
     samples = eng.sample(int(n_sample), row_offset=int(row_offset), t_start=t_start, row_ids=row_ids, seed=seed,
                          out=out, latent_out=latent)
+    if topk is not None:
+        samples = recommend.recommend_topk(samples[: int(n_sample), : eng.I], exclude[0], exclude[1], topk)
     if verbose:
         torch.cuda.synchronize(dev)
         print(f"Sampling {n_sample}/{n_sample}, Sampling took {np.round((time.time() - start_time) / 60, 2)} minutes")
