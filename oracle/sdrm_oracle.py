@@ -57,7 +57,9 @@ def denoiser_forward(sd, x, t, keep_mask):
     """eps = SDRM.forward(x, t) with the dropout keep-mask given explicitly (F.dropout p=.5, line 100)."""
     T = sd["emb_layer.weight"].shape[0]
     nh = n_hidden_of(sd)
-    emb = F.linear(timestep_embedding(t, T), sd["emb_layer.weight"], sd["emb_layer.bias"])
+    w_emb = sd["emb_layer.weight"]
+    # the sinusoid is fp32 like the model's; widened to the weights' dtype so that a float64 state_dict runs in float64
+    emb = F.linear(timestep_embedding(t, T).to(w_emb.dtype), w_emb, sd["emb_layer.bias"])
     h = torch.cat([x * keep_mask.to(x.dtype) * 2.0, emb], dim=-1)
     h = prelu(F.linear(h, sd["dnn.0.weight"], sd["dnn.0.bias"]), sd["dnn.1.weight"])
     for _ in range(nh):  # the SAME Linear + PReLU nh times (train_SDRM.py:94)

@@ -200,36 +200,56 @@ __device__ __forceinline__ double warp_sum(double v) {
 }
 
 // stats += {sum r, sum r^2, sum (sd-r)^2, sum (r-sx)^2, count};  r = pred - mu, sd = (psx - sx)/mu_coef^2
-// float4 loads (the four arrays are flat and 16-byte aligned in every caller; otherwise the scalar loop takes all of it);
-// the four terms of a quad are summed in fp32 and promoted to fp64 once per quad: B200 runs FP64 at a fraction of the fp32
-// rate, and one DADD per element and statistic made this kernel ALU-bound.
+// The four terms of a quad are summed in fp32 and promoted to fp64 once per quad: B200 runs FP64 at a fraction of the fp32
+// rate, and one DADD per element and statistic made this kernel ALU-bound.  Quads are read as float4 when all four arrays are
+// 16-byte aligned and as four scalars otherwise (ScoreMatchingLoss passes sx and psx as row slices of one [3B, L] buffer, so
+// B*L % 4 != 0 misaligns them): both give the same fp32 partials, in the same threads.
+// r is accumulated about a shift K = r[0] and turned back into sum r and sum r^2 in fp64 once per thread: the fp32 partials
+// then hold (r - K)^2 ~ var(r) instead of r^2, so the variance (sum r^2 - N mean^2) / (N - 1) that loss_seeds_kernel forms
+// keeps its precision when the mean of r is large next to its spread (mean 3, std 0.05: 3600 x N var in sum r^2).
 __global__ void __launch_bounds__(256) loss_stats_kernel(const float* __restrict__ pred, const float* __restrict__ sx,
                                                          const float* __restrict__ psx, const float* __restrict__ mu,
                                                          long long count, float mu2, double* __restrict__ stats) {
   double s0 = 0, s1 = 0, s2 = 0, s3 = 0;
+  long long n = 0;                                     // elements this thread summed
   const long long tid = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x;
   const long long nth = static_cast<long long>(gridDim.x) * blockDim.x;
   const bool vec = (((reinterpret_cast<uintptr_t>(pred) | reinterpret_cast<uintptr_t>(sx) | reinterpret_cast<uintptr_t>(psx) |
                       reinterpret_cast<uintptr_t>(mu)) & 15) == 0);
-  const long long n4 = vec ? (count >> 2) : 0;
+  const long long n4 = count >> 2;
+  const float K = __ldg(pred) - __ldg(mu);
   auto term = [&](float p, float s, float q, float m, float& a0, float& a1, float& a2, float& a3) {
-    const float r = p - m;
+    const float r = p - m, rk = r - K;
     const float sd = (q - s) / mu2;
     const float d1 = sd - r, d2 = r - s;
-    a0 += r; a1 = fmaf(r, r, a1); a2 = fmaf(d1, d1, a2); a3 = fmaf(d2, d2, a3);
+    a0 += rk; a1 = fmaf(rk, rk, a1); a2 = fmaf(d1, d1, a2); a3 = fmaf(d2, d2, a3);
   };
   for (long long i = tid; i < n4; i += nth) {
-    const float4 p = __ldcs(reinterpret_cast<const float4*>(pred) + i), s = __ldcs(reinterpret_cast<const float4*>(sx) + i);
-    const float4 q = __ldcs(reinterpret_cast<const float4*>(psx) + i), m = __ldcs(reinterpret_cast<const float4*>(mu) + i);
+    float4 p, s, q, m;
+    if (vec) {
+      p = __ldcs(reinterpret_cast<const float4*>(pred) + i); s = __ldcs(reinterpret_cast<const float4*>(sx) + i);
+      q = __ldcs(reinterpret_cast<const float4*>(psx) + i); m = __ldcs(reinterpret_cast<const float4*>(mu) + i);
+    } else {
+      const long long e = i << 2;
+      p = make_float4(pred[e], pred[e + 1], pred[e + 2], pred[e + 3]); s = make_float4(sx[e], sx[e + 1], sx[e + 2], sx[e + 3]);
+      q = make_float4(psx[e], psx[e + 1], psx[e + 2], psx[e + 3]); m = make_float4(mu[e], mu[e + 1], mu[e + 2], mu[e + 3]);
+    }
     float a0 = 0.f, a1 = 0.f, a2 = 0.f, a3 = 0.f;
     term(p.x, s.x, q.x, m.x, a0, a1, a2, a3); term(p.y, s.y, q.y, m.y, a0, a1, a2, a3);
     term(p.z, s.z, q.z, m.z, a0, a1, a2, a3); term(p.w, s.w, q.w, m.w, a0, a1, a2, a3);
     s0 += a0; s1 += a1; s2 += a2; s3 += a3;
+    n += 4;
   }
   for (long long i = (n4 << 2) + tid; i < count; i += nth) {
     float a0 = 0.f, a1 = 0.f, a2 = 0.f, a3 = 0.f;
     term(pred[i], sx[i], psx[i], mu[i], a0, a1, a2, a3);
     s0 += a0; s1 += a1; s2 += a2; s3 += a3;
+    ++n;
+  }
+  {  // sums about K -> sums of r and r^2
+    const double k = K, nd = static_cast<double>(n);
+    s1 += k * (2.0 * s0 + nd * k);
+    s0 += nd * k;
   }
   __shared__ double sh[4][8];
   s0 = warp_sum(s0); s1 = warp_sum(s1); s2 = warp_sum(s2); s3 = warp_sum(s3);

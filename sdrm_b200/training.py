@@ -113,7 +113,10 @@ class FrozenEncoder:
         if dev.type != "cuda":
             raise _lib.SdrmError("FrozenEncoder: the VAE must live on a CUDA device (no CPU fallback)")
         if x.layout == torch.sparse_csr:
-            csr = x
+            # a torch CSR tensor may store one column twice in a row; to_dense() adds such entries, and the kernel's L2 norm
+            # must be that of the sum, so the entries are summed first (to_sparse_coo() marks its result coalesced as is)
+            coo = x.to_sparse_coo()
+            csr = torch.sparse_coo_tensor(coo.indices(), coo.values(), coo.shape).coalesce().to_sparse_csr()
         elif x.layout == torch.sparse_coo:
             csr = x.coalesce().to_sparse_csr()
         else:
@@ -291,6 +294,9 @@ class DeviceCSR:
 
     def __init__(self, csr, device):
         csr = csr.tocsr()
+        if not csr.has_canonical_format:   # repeated (row, column) entries are summed once here, like to_dense() would
+            csr = csr.copy()
+            csr.sum_duplicates()
         self.shape = csr.shape
         self.host_indptr = csr.indptr.astype("int64")
         self.indptr = torch.from_numpy(self.host_indptr).to(device)

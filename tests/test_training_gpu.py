@@ -161,3 +161,15 @@ def test_multinomial_nll_matches_torch_autograd(rows, items):
     v = wide[:, :items].clone().requires_grad_(True)
     loss2 = multinomial_nll(v, X)
     assert abs(loss2.item() - loss.item()) <= 1e-6 * max(1.0, abs(loss.item()))
+    # large-magnitude logits (scale 50, |logit| up to ~250): a softmax without the max shift overflows fp32 here.  The fp32
+    # row lse of that magnitude carries ~1.5e-5 of rounding, which every softmax term of the gradient inherits.
+    big = (torch.randn(rows, items, generator=g) * 50).cuda().requires_grad_(True)
+    loss_b = multinomial_nll(big, X)
+    (loss_b * 1.7).backward()
+    ref_b_in = big.detach().double().cpu().requires_grad_(True)
+    ref_b = -torch.mean(torch.sum(torch.nn.functional.log_softmax(ref_b_in, dim=1) * X.double().cpu(), dim=1))
+    (ref_b * 1.7).backward()
+    assert torch.isfinite(loss_b).item() and torch.isfinite(big.grad).all().item()
+    assert abs(loss_b.item() - ref_b.item()) <= 2e-6 * max(1.0, abs(ref_b.item()))
+    gscale_b = ref_b_in.grad.abs().max().item() + 1e-30
+    assert (big.grad.double().cpu() - ref_b_in.grad).abs().max().item() <= 4e-5 * gscale_b
