@@ -41,6 +41,8 @@ def build_parser():
     p.add_argument("--runs", type=int, default=5, help="number of independent runs (reference: 5)")
     p.add_argument("--data-dir", type=str, default="./data", help="directory holding <dataset>/<dataset>_*.pkl")
     p.add_argument("--seed", type=int, default=None, help="seed torch / numpy for a reproducible run")
+    p.add_argument("--privacy-audit", action="store_true", default=False,
+                   help="after each run, print how close the binarised synthetic rows come to the training rows (privacy_audit)")
     return p
 
 
@@ -50,11 +52,44 @@ def equal_sparsity(scores, sparsity):
     CUDA score matrices never leave the GPU as floats: kernel K4 finds np.quantile's threshold with an exact radix select
     and ships 1 bit per entry (sdrm_b200/sparsify.py); the result is identical to the reference's host-side lines.
     Host arrays (VAE.sample returns a NumPy array in the reference too, main.py:183) take the reference's own two lines."""
+    return binarise(scores, sparsity)[0]
+
+
+def binarise(scores, sparsity):
+    """equal_sparsity, returning (dense 0/1 rows, the device PackedMatrix of CUDA scores or None for host arrays), so that the
+    privacy audit searches the bits already on the GPU instead of uploading the dense frame again."""
     import torch
     if isinstance(scores, torch.Tensor):
         from sdrm_b200.sparsify import equal_sparsity_device
-        return equal_sparsity_device(scores.detach(), sparsity).numpy(int)
-    return (scores >= np.quantile(scores.flatten(), sparsity)).astype(int)
+        pm = equal_sparsity_device(scores.detach(), sparsity)
+        return pm.numpy(int), pm
+    return (scores >= np.quantile(scores.flatten(), sparsity)).astype(int), None
+
+
+AUDIT_COLS = ["DCR mean", "DCR p5", "DCR p50", "DCR p95", "exact copies", "copy share", "NNDR median"]
+
+
+def privacy_audit(binarised, real, baseline=None):
+    """Distance to the closest record of every binarised synthetic row set against `real` (the rows the generator was trained
+    on, TRAIN_PARTIAL_VALID_DATA), with the real rows against themselves (each row's own index excluded) as the baseline line.
+    DCR = 1 - Jaccard similarity of the nearest real row; exact copies have Hamming distance 0; NNDR = DCR of the nearest over
+    DCR of the second nearest real row (sdrm_b200.privacy.NearestRows.summary).  Returns (table, baseline summary).
+
+    Read the synthetic lines against the baseline line, not against 0.  Equal sparsity keeps 1 - SPARSITY of the entries, and
+    SPARSITY counts the training matrix's explicit stored zeros as interactions, so synthetic rows carry more ones than real
+    rows do (10.07 % against 5.75 % of the entries at ml-100k).  That alone lowers their Jaccard similarity to any real row."""
+    import pandas as pd
+
+    from sdrm_b200.privacy import nearest_rows
+    if baseline is None:
+        baseline = nearest_rows(real, real, k=2, exclude_same_index=True).summary()
+    rows = {}
+    for name, (dense, packed) in binarised.items():
+        rows[name] = nearest_rows(packed if packed is not None else dense, real, k=2).summary()
+    rows["real vs real (baseline)"] = baseline
+    keys = ["dcr_mean", "dcr_p5", "dcr_p50", "dcr_p95", "exact_copies", "exact_copy_share", "nndr_median"]
+    table = pd.DataFrame([[s[k] for k in keys] for s in rows.values()], index=list(rows), columns=AUDIT_COLS)
+    return table, baseline
 
 
 def main(argv=None):
@@ -84,6 +119,7 @@ def main(argv=None):
 
     model = args.model.lower()
     results = {c: [] for c in COLS}
+    audit_baseline = None
     for run_n in range(args.runs):
         start_time = time.time()
         print(10 * "#", "Starting run", run_n + 1, 10 * "#")
@@ -103,11 +139,15 @@ def main(argv=None):
         F_SDRM = sample_ddpm(N_USERS, SDRM, VAE, args.MLP_latent_neurons, args.SDRM_noise_variance_diminisher,
                              n_timesteps=args.SDRM_timesteps, verbose=True,
                              sampling_steps=args.SDRM_sampling_steps, eta=args.SDRM_eta)
-        synth = {
-            "M-SDRM": pd.DataFrame(equal_sparsity(M_SDRM, SPARSITY)),
-            "F-SDRM": pd.DataFrame(equal_sparsity(F_SDRM, SPARSITY)),
-            "MultiVAE++": pd.DataFrame(equal_sparsity(VAE.sample(N_USERS), SPARSITY)),
+        binarised = {
+            "M-SDRM": binarise(M_SDRM, SPARSITY),
+            "F-SDRM": binarise(F_SDRM, SPARSITY),
+            "MultiVAE++": binarise(VAE.sample(N_USERS), SPARSITY),
         }
+        synth = {name: pd.DataFrame(dense) for name, (dense, _) in binarised.items()}
+        if args.privacy_audit:
+            audit, audit_baseline = privacy_audit({c: binarised[c] for c in COLS}, TRAIN_PARTIAL_VALID_DATA, audit_baseline)
+            print(f"\nPrivacy audit (run {run_n + 1}): distance to the closest training row\n{audit.round(4).to_markdown()}")
         for name, frame in synth.items():
             if model == "svd":
                 # NOTE: the flag is passed as only_synthetic=, exactly like the reference (main.py:189-194)

@@ -70,6 +70,12 @@ SIGNATURES = {
     "sdrm_select_walk_bf16": (C.c_int, [_P, _P, C.c_int, C.c_double, C.c_int, _P]),
     "sdrm_select_threshold_pack_bf16": (C.c_int, [_P, C.c_int64, C.c_int, C.c_int64, _P, C.c_int, _P, C.c_int64, _P, _P]),
     "sdrm_loss_grad_seeds": (C.c_int, [_P, _P, _P, _P, C.c_int64, C.c_double, _P, _P, _P, _P, _P, _P]),
+    "sdrm_privacy_image_pitch": (C.c_int64, [C.c_int]),
+    "sdrm_privacy_image_bits": (C.c_int, [_P, C.c_int64, C.c_int64, C.c_int, _P, C.c_int64, _P, _P]),
+    "sdrm_privacy_image_csr": (C.c_int, [_P, _P, _P, C.c_int64, C.c_int64, C.c_int, _P, C.c_int64, _P, _P, _P]),
+    "sdrm_privacy_workspace_bytes": (C.c_size_t, [C.c_int64, C.c_int64, C.c_int, C.c_int]),
+    "sdrm_privacy_nearest": (C.c_int, [_P, _P, C.c_int64, _P, _P, C.c_int64, C.c_int, C.c_int64, C.c_int, C.c_int, C.c_int64,
+                                       C.c_int, _P, _P, _P, _P, C.c_size_t, _P]),
 }
 
 

@@ -271,6 +271,22 @@ __device__ __forceinline__ void umma_bf16_ss(uint32_t d_tmem, uint64_t a_desc, u
       ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
       : "memory");
 }
+// Instruction descriptor for kind::i8: D=s32, A=B=u8 (unsigned), both K-major, M x N tile.
+__host__ __device__ constexpr uint32_t umma_idesc_u8(int M, int N) {
+  return (2u << 4) | (static_cast<uint32_t>(N >> 3) << 17) | (static_cast<uint32_t>(M >> 4) << 24);
+}
+// one K = 32 step (32 bytes of each K-major row): exact integer products, s32 accumulate
+__device__ __forceinline__ void umma_u8_ss(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc,
+                                          uint32_t accumulate) {
+  asm volatile(
+      "{\n"
+      ".reg .pred p;\n"
+      "setp.ne.b32 p, %4, 0;\n"
+      "tcgen05.mma.cta_group::1.kind::i8 [%0], %1, %2, %3, p;\n"
+      "}\n"
+      ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
 // all previously issued UMMAs of this thread arrive on `bar` when they retire
 __device__ __forceinline__ void umma_commit(uint32_t bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
