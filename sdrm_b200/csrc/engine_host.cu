@@ -248,6 +248,13 @@ __global__ void grid_bias_kernel(const float* __restrict__ src, int ld, const in
   for (int c = threadIdx.x; c < ld; c += blockDim.x) d[c] = s[c];
 }
 
+static void launch_pack_weight(const float* W, int N, int K, long long ldw, int col_off, uint8_t* hi, uint8_t* lo,
+                               const Geom& g, cudaStream_t st) {
+  const long long total = static_cast<long long>(g.NCH) * g.KB * g.NC * 8;
+  const int blocks = static_cast<int>(std::min<long long>((total + 255) / 256, 4096));
+  pack_weight_kernel<<<blocks, 256, 0, st>>>(W, N, K, ldw, col_off, hi, lo, g.NCH, g.NC, g.KB);
+}
+
 }  // namespace sdrm
 
 // ------------------------------------------------------------------------------------------------
@@ -255,11 +262,34 @@ __global__ void grid_bias_kernel(const float* __restrict__ src, int ld, const in
 // ------------------------------------------------------------------------------------------------
 using namespace sdrm;
 
+// One dense layer packed for the engine, in the normal geometry [0] and in the 8-chunk geometry of the column split [1].
+// img[1] stays null when the split set is not packed or its geometry is the normal one; img[0] then serves.
+struct PackedLayer {
+  Geom g[2];
+  uint8_t* img[2] = {nullptr, nullptr};
+  int np = 0;                 // padded bias width (both geometries fit)
+  float* bias = nullptr;      // [np]; the first layer's is the per-step table [T+1][np]
+  const uint8_t* image(bool split_geom) const { return split_geom && img[1] ? img[1] : img[0]; }
+};
+enum { LAYER_FIRST, LAYER_HIDDEN, LAYER_OUT, LAYER_DEC1, LAYER_DEC2, N_LAYERS };   // denoiser: FIRST .. OUT, decoder: DEC1, DEC2
+
+// How one sdrm_sample launch runs (every data flow gives bit-identical rows); plan_launch chooses it
+struct LaunchPlan {
+  bool k6 = false;              // the small-chain kernel instead of the tcgen05 layer engine (K1)
+  int cluster = 1;              // K1: CTAs of a tcgen05 tile (1 or 2; 1 for the column split); 0 for K6
+  int split = 0;                // K1 column split: CTAs per row tile (8 / 4 / 2), 0 = not split
+  bool split_geom = false;      // the column split runs on the 8-chunk images
+  int grid = 0;                 // K1 CTAs
+  int n_sub = 1;                // row tiles a CTA pair interleaves
+  int resident = 0, res_nstg = 0, discard_kb = 0;
+  uint32_t split_stage_bytes = 0;
+};
+
 struct sdrm_handle {
   int device = 0;
   int num_sms = 0;
   int last_launches = 0;
-  int last_cluster = 1;
+  LaunchPlan last;              // what the last sdrm_sample launch did
   int resident[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};  // resident CTAs per cluster size (1, 2, 4, 8)
   int* err_word = nullptr;        // device view of the watchdog word
   volatile int* err_host = nullptr;   // host view: the word lives in mapped pinned host memory, so it survives a device trap
@@ -270,23 +300,15 @@ struct sdrm_handle {
   int no_resident = 0;          // 1 = never keep the chain's activation tile in shared memory (A/B of the resident mode)
   int no_split = 0;             // 1 = never split a row tile's N chunks over a cluster (A/B of the column-split mode)
   int split_resident[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};   // resident CTAs of the column-split kernel per cluster size (2, 4, 8)
-  int last_split = 0;           // cluster size of the last launch's column split (0: not split)
-  int last_resident = 0;        // what the last sdrm_sample launch did
   int grid_limit = 0;           // cap on the CTAs of an sdrm_sample launch (tests: small inputs exercise the multi-tile loops)
   int debug_flags = 0;          // -DSDRM_PERF_DEBUG builds only
   unsigned long long* trace = nullptr;   // -DSDRM_TRACE builds only
+  PackedLayer layer[N_LAYERS];
   // denoiser
   bool have_den = false;
   int T = 0, L = 0, D = 0, nh = 0;
   float nd = 1.0f;
-  Geom g0, gh, go;
-  uint8_t *w0 = nullptr, *wh = nullptr, *wo = nullptr;
-  // column-split geometry (8 chunks per layer) and its weight images; packed for every denoiser the tcgen05 engine takes (> 64 wide)
-  Geom s0, sh, so, s1, s2;
-  uint8_t *w0s = nullptr, *whs = nullptr, *wos = nullptr, *w1s = nullptr, *w2s = nullptr;
-  bool split_den = false, split_dec = false;
-  int np0 = 0, nph = 0, npo = 0, np1 = 0, np2 = 0;   // padded bias widths (both geometries fit)
-  float *bias0 = nullptr, *bh = nullptr, *bo = nullptr, *slopes = nullptr, *coef = nullptr;
+  float *slopes = nullptr, *coef = nullptr;
   // K6 (small denoisers, small_chain_kernel.cuh): zero-padded bf16 images and 64-wide bias rows, packed when every width <= 64
   bool small_den = false, small_dec = false;
   __nv_bfloat16 *s_den = nullptr;   // w0 | wh | wo, each [64][SMALL_KP]
@@ -300,82 +322,79 @@ struct sdrm_handle {
   int grid_S = 0;
   float* sched = nullptr;           // the packed schedule b | a | ab [3 (T+1)]
   int32_t* grid_tau = nullptr;      // tau_0 = 0, tau_1 .. tau_S
-  float *grid_bias0 = nullptr, *grid_coef = nullptr;   // bias0 rows tau_j [T+1][np0]; coefficients [T+1][4]
+  float *grid_bias0 = nullptr, *grid_coef = nullptr;   // first-layer bias rows tau_j [T+1][np]; coefficients [T+1][4]
   float* grid_s_bias = nullptr;     // K6: bias0 rows tau_j [T+1][64]
   // decoder
   bool have_dec = false;
   int H = 0, I = 0;
-  Geom g1, g2;
-  uint8_t *w1 = nullptr, *w2 = nullptr;
-  float *b1 = nullptr, *b2 = nullptr;
 };
 
+static void free_layers(sdrm_handle* h, int first, int last) {
+  for (int l = first; l <= last; ++l) {
+    PackedLayer& p = h->layer[l];
+    cudaFree(p.img[0]); cudaFree(p.img[1]); cudaFree(p.bias);
+    p = PackedLayer();
+  }
+}
 static void free_den(sdrm_handle* h) {
-  cudaFree(h->w0); cudaFree(h->wh); cudaFree(h->wo);
-  cudaFree(h->w0s); cudaFree(h->whs); cudaFree(h->wos);
-  h->w0s = h->whs = h->wos = nullptr; h->split_den = false;
-  cudaFree(h->bias0); cudaFree(h->bh); cudaFree(h->bo); cudaFree(h->slopes); cudaFree(h->coef);
+  free_layers(h, LAYER_FIRST, LAYER_OUT);
+  cudaFree(h->slopes); cudaFree(h->coef);
   cudaFree(h->s_den); cudaFree(h->s_bias);
   h->s_den = nullptr; h->s_bias = nullptr; h->small_den = false;
   cudaFree(h->sched); cudaFree(h->grid_tau); cudaFree(h->grid_bias0); cudaFree(h->grid_coef); cudaFree(h->grid_s_bias);
   h->sched = h->grid_bias0 = h->grid_coef = h->grid_s_bias = nullptr; h->grid_tau = nullptr; h->grid_S = 0;
-  h->w0 = h->wh = h->wo = nullptr;
-  h->bias0 = h->bh = h->bo = h->slopes = h->coef = nullptr;
+  h->slopes = h->coef = nullptr;
   h->have_den = false;
 }
 static void free_dec(sdrm_handle* h) {
-  cudaFree(h->w1); cudaFree(h->w2); cudaFree(h->b1); cudaFree(h->b2);
-  cudaFree(h->w1s); cudaFree(h->w2s);
-  h->w1s = h->w2s = nullptr; h->split_dec = false;
+  free_layers(h, LAYER_DEC1, LAYER_DEC2);
   cudaFree(h->s_dec1); cudaFree(h->s_dec2); cudaFree(h->s_b1);
   h->s_dec1 = h->s_dec2 = nullptr; h->s_b1 = nullptr; h->small_dec = false;
-  h->w1 = h->w2 = nullptr;
-  h->b1 = h->b2 = nullptr;
   h->have_dec = false;
 }
 
+// The 8-chunk images are packed for a denoiser wider than 64 (narrower ones run on the small-chain kernel) whose layers they
+// re-cut, and for a decoder behind a latent wider than 64 (the denoiser it follows may take the column split)
+static bool split_set_packed(const sdrm_handle* h, bool decoder) {
+  if (decoder) return h->layer[LAYER_DEC1].g[0].K > SMALL_MAX;
+  if (std::max(h->L, h->D) <= SMALL_MAX) return false;
+  for (int l = LAYER_FIRST; l <= LAYER_OUT; ++l)
+    if (!same_geom(h->layer[l].g[0], h->layer[l].g[1])) return true;
+  return false;
+}
 
-// run-time watchdog limit of this translation unit's kernels (ptx_sm100.cuh): SDRM_WATCHDOG_MS in the environment, 0 = none
-static int apply_watchdog_env_k1() {
-  static bool done = false;
-  if (done) return SDRM_OK;
-  done = true;
-  const char* e = getenv("SDRM_WATCHDOG_MS");
-  if (!e || !*e) return SDRM_OK;
-  const unsigned long long ns = strtoull(e, nullptr, 10) * 1000000ull;
-  SDRM_CUDA(cudaMemcpyToSymbol(sdrm::g_sdrm_watchdog_ns, &ns, sizeof ns));
+// Layers first .. last, of N x K weights: both geometries, the images (bf16x3: a lo image after the hi one) and the padded bias
+// (the first layer's has T + 1 rows).  The 8-chunk image only where the set is packed and the geometry differs.
+static int alloc_layers(sdrm_handle* h, int first, int last, const int (*NK)[2], bool bf16x3, int first_bias_rows) {
+  for (int l = first; l <= last; ++l) {
+    PackedLayer& p = h->layer[l];
+    p.g[0] = make_geom(NK[l - first][0], NK[l - first][1]);
+    p.g[1] = make_geom_split(NK[l - first][0], NK[l - first][1]);
+    p.np = std::max(p.g[0].Np, p.g[1].Np);
+  }
+  const bool split_set = split_set_packed(h, first == LAYER_DEC1);
+  for (int l = first; l <= last; ++l) {
+    PackedLayer& p = h->layer[l];
+    SDRM_CUDA(cudaMalloc(&p.img[0], (bf16x3 ? 2 : 1) * p.g[0].img_bytes()));
+    if (split_set && !same_geom(p.g[0], p.g[1])) SDRM_CUDA(cudaMalloc(&p.img[1], (bf16x3 ? 2 : 1) * p.g[1].img_bytes()));
+    SDRM_CUDA(cudaMalloc(&p.bias, sizeof(float) * (l == LAYER_FIRST ? first_bias_rows : 1) * p.np));
+  }
   return SDRM_OK;
 }
 
-static int engine_set_smem_attr() {
-  { int wrc = apply_watchdog_env_k1(); if (wrc) return wrc; }
-  static bool done[64] = {false};
-  int dev = 0;
-  SDRM_CUDA(cudaGetDevice(&dev));
-  if (dev < 64 && done[dev]) return SDRM_OK;
-  SDRM_CUDA(cudaFuncSetAttribute(sdrm_layer_engine_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, ENGINE_SMEM_BYTES));
-  SDRM_CUDA(cudaFuncSetAttribute(sdrm_layer_engine_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, ENGINE_SMEM_BYTES));
-  SDRM_CUDA(cudaFuncSetAttribute((sdrm_layer_engine_kernel<2, true>), cudaFuncAttributeMaxDynamicSharedMemorySize, ENGINE_SMEM_BYTES));
-  SDRM_CUDA(cudaFuncSetAttribute((sdrm_layer_engine_kernel<1, false, true>), cudaFuncAttributeMaxDynamicSharedMemorySize, ENGINE_SMEM_BYTES));
-  if (dev < 64) done[dev] = true;
-  return SDRM_OK;
+// W fp32 [N, ldw] (columns 0 .. K) -> the layer's images
+static void pack_layer(const PackedLayer& p, const float* W, long long ldw, bool bf16x3, cudaStream_t st) {
+  for (int s = 0; s < 2; ++s)
+    if (p.img[s]) launch_pack_weight(W, p.g[s].N, p.g[s].K, ldw, 0, p.img[s], bf16x3 ? p.img[s] + p.g[s].img_bytes() : nullptr, p.g[s], st);
 }
 
 // resident CTAs for a cluster size (1 CTA per SM; clusters must fit inside a GPC)
 static int max_resident_ctas(int cluster, int num_sms, bool split = false) {
   if (cluster == 1) return num_sms;
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(static_cast<unsigned>(num_sms / cluster * cluster));
-  cfg.blockDim = dim3(ENGINE_THREADS);
-  cfg.dynamicSmemBytes = ENGINE_SMEM_BYTES;
-  cudaLaunchAttribute attr;
-  attr.id = cudaLaunchAttributeClusterDimension;
-  attr.val.clusterDim.x = cluster; attr.val.clusterDim.y = 1; attr.val.clusterDim.z = 1;
-  cfg.attrs = &attr; cfg.numAttrs = 1;
-  int n = 0;
   if (!split && cluster != 2) return 0;
-  cudaError_t e = split ? cudaOccupancyMaxActiveClusters(&n, (sdrm_layer_engine_kernel<1, false, true>), &cfg)
-                        : cudaOccupancyMaxActiveClusters(&n, sdrm_layer_engine_kernel<2>, &cfg);
+  const EngineClusterConfig c(num_sms / cluster * cluster, cluster, nullptr);
+  int n = 0;
+  cudaError_t e = cudaOccupancyMaxActiveClusters(&n, engine_kernel<false>(cluster, false, split), &c.cfg);
   if (e != cudaSuccess) { cudaGetLastError(); return 0; }
   return n * cluster;
 }
@@ -383,24 +402,9 @@ static int max_resident_ctas(int cluster, int num_sms, bool split = false) {
 // ---- TMA tensor maps: a blob of `rows` x 128 bytes, box = `box_rows` rows x `box_bytes`.  Weight maps (pair mode) take no
 // swizzle: the weight images are pre-swizzled in global memory, so a box lands in shared memory byte-for-byte like the bulk
 // copies of single mode.  The activation load map swizzles (SWIZZLE_128B), the activation store map does not.
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-static EncodeTiledFn get_encode_fn() {
-  static EncodeTiledFn fn = nullptr;
-  if (fn) return fn;
-  void* p = nullptr;
-  cudaDriverEntryPointQueryResult q;
-  if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) != cudaSuccess || q != cudaDriverEntryPointSuccess) {
-    cudaGetLastError();
-    return nullptr;
-  }
-  fn = reinterpret_cast<EncodeTiledFn>(p);
-  return fn;
-}
 static int make_rows_map(CUtensorMap* map, const void* base, unsigned long long rows, unsigned box_rows, unsigned box_bytes = 128,
                          bool swizzle128 = false) {
-  EncodeTiledFn fn = get_encode_fn();
+  EncodeTiledFn fn = encode_tiled_fn();
   if (!fn) return sdrm_fail(SDRM_ERR_CUDA, "cuTensorMapEncodeTiled entry point not available");
   const cuuint64_t dims[2] = {128, rows};
   const cuuint64_t strides[1] = {128};
@@ -423,7 +427,7 @@ static int fill_act_maps(ChainParams& P, size_t workspace_bytes) {
   if (rc) return rc;
   return make_rows_map(&P.tm_act_st, P.scratch, workspace_bytes / 128, 32, 32, false);
 }
-static int fill_pair_maps(ChainParams& P, size_t workspace_bytes, int cluster) {
+static int fill_pair_maps(ChainParams& P, int cluster) {
   auto w_rows = [](const LayerDesc& d) {
     return static_cast<unsigned long long>(d.passes == 3 ? 2 : 1) * d.NCH * d.KB * d.NC;
   };
@@ -435,7 +439,6 @@ static int fill_pair_maps(ChainParams& P, size_t workspace_bytes, int cluster) {
     int rc = make_rows_map(&P.tm_dec_w[l], P.dec[l].w_img, w_rows(P.dec[l]), P.dec[l].NC / cluster);
     if (rc) return rc;
   }
-  (void)workspace_bytes;
   return SDRM_OK;
 }
 
@@ -443,13 +446,6 @@ static int fill_pair_maps(ChainParams& P, size_t workspace_bytes, int cluster) {
 // perturb how the compiler optimises the fp32 kernels, whose code stays as it is.
 static int launch_engine(const ChainParams& P, int grid, int cluster, cudaStream_t st, int split = 0, bool bf16 = false) {
   return bf16 ? launch_engine_bf16(P, grid, cluster, st, split) : launch_engine_t<false>(P, grid, cluster, st, split);
-}
-
-static void launch_pack_weight(const float* W, int N, int K, long long ldw, int col_off, uint8_t* hi, uint8_t* lo,
-                               const Geom& g, cudaStream_t st) {
-  const long long total = static_cast<long long>(g.NCH) * g.KB * g.NC * 8;
-  const int blocks = static_cast<int>(std::min<long long>((total + 255) / 256, 4096));
-  pack_weight_kernel<<<blocks, 256, 0, st>>>(W, N, K, ldw, col_off, hi, lo, g.NCH, g.NC, g.KB);
 }
 
 extern "C" {
@@ -481,7 +477,7 @@ int sdrm_create(sdrm_handle** out, int device) {
     h->err_host = static_cast<volatile int*>(hp);
     h->err_word = static_cast<int*>(dp);
   }
-  if (engine_set_smem_attr() != SDRM_OK) { delete h; return SDRM_ERR_CUDA; }
+  if (engine_setup<false>() != SDRM_OK) { delete h; return SDRM_ERR_CUDA; }
   h->resident[1] = h->num_sms;
   h->resident[2] = max_resident_ctas(2, h->num_sms);
   for (int cs = 2; cs <= 8; cs *= 2) h->split_resident[cs] = max_resident_ctas(cs, h->num_sms, true);
@@ -516,48 +512,26 @@ int sdrm_denoiser_pack(sdrm_handle* h, const float* d_We, const float* d_be, con
   if (!same) {
     free_den(h);
     h->T = T; h->L = L; h->D = D; h->nh = nh;
-    h->g0 = make_geom(D, L);
-    h->gh = make_geom(D, D);
-    h->go = make_geom(L, D);
-    h->s0 = make_geom_split(D, L);
-    h->sh = make_geom_split(D, D);
-    h->so = make_geom_split(L, D);
-    h->np0 = std::max(h->g0.Np, h->s0.Np); h->nph = std::max(h->gh.Np, h->sh.Np); h->npo = std::max(h->go.Np, h->so.Np);
-    SDRM_CUDA(cudaMalloc(&h->w0, h->g0.img_bytes()));
-    SDRM_CUDA(cudaMalloc(&h->wh, h->gh.img_bytes()));
-    SDRM_CUDA(cudaMalloc(&h->wo, h->go.img_bytes()));
-    // a second set of images in the column-split geometry (every layer re-cut into 8 chunks), unless it is the normal one
-    h->split_den = std::max(L, D) > SMALL_MAX &&   // (narrower denoisers run on the small-chain kernel)
-                   !(same_geom(h->g0, h->s0) && same_geom(h->gh, h->sh) && same_geom(h->go, h->so));
-    if (h->split_den) {
-      SDRM_CUDA(cudaMalloc(&h->w0s, h->s0.img_bytes()));
-      SDRM_CUDA(cudaMalloc(&h->whs, h->sh.img_bytes()));
-      SDRM_CUDA(cudaMalloc(&h->wos, h->so.img_bytes()));
-    }
-    SDRM_CUDA(cudaMalloc(&h->bias0, sizeof(float) * (T + 1) * h->np0));
-    SDRM_CUDA(cudaMalloc(&h->bh, sizeof(float) * h->nph));
-    SDRM_CUDA(cudaMalloc(&h->bo, sizeof(float) * h->npo));
+    const int NK[3][2] = {{D, L}, {D, D}, {L, D}};   // first, hidden, out
+    int rc = alloc_layers(h, LAYER_FIRST, LAYER_OUT, NK, false, T + 1);
+    if (rc) return rc;
     SDRM_CUDA(cudaMalloc(&h->slopes, sizeof(float) * 2));
     SDRM_CUDA(cudaMalloc(&h->coef, sizeof(float) * 4 * (T + 1)));
     SDRM_CUDA(cudaMalloc(&h->sched, sizeof(float) * 3 * (T + 1)));
     SDRM_CUDA(cudaMalloc(&h->grid_tau, sizeof(int32_t) * (T + 1)));
-    SDRM_CUDA(cudaMalloc(&h->grid_bias0, sizeof(float) * (T + 1) * h->np0));
+    SDRM_CUDA(cudaMalloc(&h->grid_bias0, sizeof(float) * (T + 1) * h->layer[LAYER_FIRST].np));
     SDRM_CUDA(cudaMalloc(&h->grid_coef, sizeof(float) * 4 * (T + 1)));
   }
   h->grid_S = 0;   // new weights or schedule: the full chain until a grid is set again
   h->nd = noise_divider;
   SDRM_CUDA(cudaMemcpyAsync(h->sched, d_sched, sizeof(float) * 3 * (T + 1), cudaMemcpyDeviceToDevice, st));
-  launch_pack_weight(d_W0, D, L, L + T, 0, h->w0, nullptr, h->g0, st);
-  if (nh > 0) launch_pack_weight(d_Wh, D, D, D, 0, h->wh, nullptr, h->gh, st);
-  launch_pack_weight(d_Wo, L, D, D, 0, h->wo, nullptr, h->go, st);
-  if (h->split_den) {
-    launch_pack_weight(d_W0, D, L, L + T, 0, h->w0s, nullptr, h->s0, st);
-    if (nh > 0) launch_pack_weight(d_Wh, D, D, D, 0, h->whs, nullptr, h->sh, st);
-    launch_pack_weight(d_Wo, L, D, D, 0, h->wos, nullptr, h->so, st);
-  }
-  bias_table_kernel<<<T + 1, 256, sizeof(float) * 2 * T, st>>>(d_We, d_be, d_W0, d_b0, T, L, D, h->bias0, h->np0);
-  pad_bias_kernel<<<(h->nph + 255) / 256, 256, 0, st>>>(nh > 0 ? d_bh : nullptr, D, h->bh, h->nph);
-  pad_bias_kernel<<<(h->npo + 255) / 256, 256, 0, st>>>(d_bo, L, h->bo, h->npo);
+  const PackedLayer &first = h->layer[LAYER_FIRST], &hidden = h->layer[LAYER_HIDDEN], &out = h->layer[LAYER_OUT];
+  pack_layer(first, d_W0, L + T, false, st);
+  if (nh > 0) pack_layer(hidden, d_Wh, D, false, st);
+  pack_layer(out, d_Wo, D, false, st);
+  bias_table_kernel<<<T + 1, 256, sizeof(float) * 2 * T, st>>>(d_We, d_be, d_W0, d_b0, T, L, D, first.bias, first.np);
+  pad_bias_kernel<<<(hidden.np + 255) / 256, 256, 0, st>>>(nh > 0 ? d_bh : nullptr, D, hidden.bias, hidden.np);
+  pad_bias_kernel<<<(out.np + 255) / 256, 256, 0, st>>>(d_bo, L, out.bias, out.np);
   SDRM_CUDA(cudaMemcpyAsync(h->slopes, d_a0, sizeof(float), cudaMemcpyDeviceToDevice, st));
   if (nh > 0) SDRM_CUDA(cudaMemcpyAsync(h->slopes + 1, d_ah, sizeof(float), cudaMemcpyDeviceToDevice, st));
   coef_kernel<<<(T + 1 + 127) / 128, 128, 0, st>>>(d_sched, T, noise_divider, h->coef);
@@ -572,7 +546,7 @@ int sdrm_denoiser_pack(sdrm_handle* h, const float* d_We, const float* d_be, con
     pack_small_weight_kernel<<<18, 256, 0, st>>>(d_W0, D, L, L + T, 0, 64, h->s_den, nullptr);
     pack_small_weight_kernel<<<18, 256, 0, st>>>(nh > 0 ? d_Wh : d_Wo, nh > 0 ? D : 0, nh > 0 ? D : 0, D, 0, 64, h->s_den + img, nullptr);
     pack_small_weight_kernel<<<18, 256, 0, st>>>(d_Wo, L, D, D, 0, 64, h->s_den + 2 * img, nullptr);
-    pad_rows64_kernel<<<(64 * (T + 1) + 255) / 256, 256, 0, st>>>(h->bias0, h->np0, D, T + 1, h->s_bias);
+    pad_rows64_kernel<<<(64 * (T + 1) + 255) / 256, 256, 0, st>>>(first.bias, first.np, D, T + 1, h->s_bias);
     pad_rows64_kernel<<<1, 64, 0, st>>>(nh > 0 ? d_bh : nullptr, 0, D, 1, h->s_bias + 64 * (T + 1));
     pad_rows64_kernel<<<1, 64, 0, st>>>(d_bo, 0, L, 1, h->s_bias + 64 * (T + 2));
     SDRM_CUDA(cudaGetLastError());
@@ -591,31 +565,19 @@ int sdrm_decoder_pack(sdrm_handle* h, const float* d_W1, const float* d_b1, cons
   if (H > MAX_ACT_CHUNKS * MAX_NC) return sdrm_fail(SDRM_ERR_UNSUPPORTED, "sdrm_decoder_pack: VAE hidden width above 8 x 256");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   SDRM_CUDA(cudaSetDevice(h->device));
-  const bool same = h->have_dec && h->g1.K == L && h->H == H && h->I == I;
+  const bool same = h->have_dec && h->layer[LAYER_DEC1].g[0].K == L && h->H == H && h->I == I;
   if (!same) {
     free_dec(h);
     h->H = H; h->I = I;
-    h->g1 = make_geom(H, L);
-    h->g2 = make_geom(I, H);
-    h->s1 = make_geom_split(H, L);
-    h->s2 = make_geom_split(I, H);
-    h->np1 = std::max(h->g1.Np, h->s1.Np); h->np2 = std::max(h->g2.Np, h->s2.Np);
-    SDRM_CUDA(cudaMalloc(&h->w1, 2 * h->g1.img_bytes()));
-    SDRM_CUDA(cudaMalloc(&h->w2, 2 * h->g2.img_bytes()));
-    h->split_dec = L > SMALL_MAX;   // the denoiser this decoder follows may take the column split
-    if (h->split_dec) {
-      if (!same_geom(h->g1, h->s1)) SDRM_CUDA(cudaMalloc(&h->w1s, 2 * h->s1.img_bytes()));
-      if (!same_geom(h->g2, h->s2)) SDRM_CUDA(cudaMalloc(&h->w2s, 2 * h->s2.img_bytes()));
-    }
-    SDRM_CUDA(cudaMalloc(&h->b1, sizeof(float) * h->np1));
-    SDRM_CUDA(cudaMalloc(&h->b2, sizeof(float) * h->np2));
+    const int NK[2][2] = {{H, L}, {I, H}};
+    int rc = alloc_layers(h, LAYER_DEC1, LAYER_DEC2, NK, true, 1);
+    if (rc) return rc;
   }
-  launch_pack_weight(d_W1, H, L, L, 0, h->w1, h->w1 + h->g1.img_bytes(), h->g1, st);
-  launch_pack_weight(d_W2, I, H, H, 0, h->w2, h->w2 + h->g2.img_bytes(), h->g2, st);
-  if (h->w1s) launch_pack_weight(d_W1, H, L, L, 0, h->w1s, h->w1s + h->s1.img_bytes(), h->s1, st);
-  if (h->w2s) launch_pack_weight(d_W2, I, H, H, 0, h->w2s, h->w2s + h->s2.img_bytes(), h->s2, st);
-  pad_bias_kernel<<<(h->np1 + 255) / 256, 256, 0, st>>>(d_b1, H, h->b1, h->np1);
-  pad_bias_kernel<<<(h->np2 + 255) / 256, 256, 0, st>>>(d_b2, I, h->b2, h->np2);
+  const PackedLayer &dec1 = h->layer[LAYER_DEC1], &dec2 = h->layer[LAYER_DEC2];
+  pack_layer(dec1, d_W1, L, true, st);
+  pack_layer(dec2, d_W2, H, true, st);
+  pad_bias_kernel<<<(dec1.np + 255) / 256, 256, 0, st>>>(d_b1, H, dec1.bias, dec1.np);
+  pad_bias_kernel<<<(dec2.np + 255) / 256, 256, 0, st>>>(d_b2, I, dec2.bias, dec2.np);
   SDRM_CUDA(cudaGetLastError());
   if (L <= SMALL_MAX && H <= SMALL_MAX) {   // K6 images
     const size_t img = static_cast<size_t>(64) * SMALL_KP;
@@ -639,16 +601,20 @@ int sdrm_decoder_pack(sdrm_handle* h, const float* d_W1, const float* d_b1, cons
   return SDRM_OK;
 }
 
+// the column split may run on the 8-chunk images when both the denoiser's and the decoder's are packed
+static bool geom8_packed(const sdrm_handle* h) { return split_set_packed(h, false) && split_set_packed(h, true); }
+
+// k-blocks of the widest activation image: every layer's input, every output but the logits
 static int kb_max_of(const sdrm_handle* h) {
+  const bool geom8 = geom8_packed(h);
   int kb = 1;
-  const Geom* gs[5] = {&h->g0, &h->gh, &h->go, &h->g1, &h->g2};
-  const Geom* ss[4] = {&h->s0, &h->sh, &h->so, &h->s1};
-  for (int i = 0; i < 4; ++i) {  // g2 writes logits, not activations
-    kb = std::max(kb, gs[i]->KB);
-    kb = std::max(kb, (gs[i]->Np + KBLK - 1) / KBLK);
-    if (h->split_den && h->split_dec) kb = std::max(kb, (ss[i]->Np + KBLK - 1) / KBLK);   // (the column-split geometry pads wider)
+  for (int l = 0; l < N_LAYERS; ++l) {
+    const Geom *g = h->layer[l].g;
+    kb = std::max(kb, g[0].KB);
+    if (l == LAYER_DEC2) continue;   // writes logits, not activations
+    kb = std::max(kb, (g[0].Np + KBLK - 1) / KBLK);
+    if (geom8) kb = std::max(kb, (g[1].Np + KBLK - 1) / KBLK);   // (the column-split geometry pads wider)
   }
-  kb = std::max(kb, h->g2.KB);
   return kb;
 }
 
@@ -679,24 +645,145 @@ size_t sdrm_sample_workspace_bytes(const sdrm_handle* h, int64_t n) {
 
 }  // extern "C"
 
+static void fill_desc(LayerDesc& d, const uint8_t* w, const Geom& g, const float* bias, const float* slope, int bstride, int passes,
+                      int kind, int in_hi, int in_lo, int out_hi, int out_lo) {
+  d.w_img = w; d.bias = bias; d.slope = slope; d.bias_step_stride = bstride;
+  d.KB = g.KB; d.kmma_last = g.kmma_last; d.passes = passes; d.NCH = g.NCH; d.NC = g.NC; d.kind = kind;
+  d.in_hi = in_hi; d.in_lo = in_lo; d.out_hi = out_hi; d.out_lo = out_lo; d.n_valid = g.N;
+}
+
+// the small-chain kernel (K6) takes models whose every width is <= 64
+static bool small_ok(const sdrm_handle* h) { return h->small_den && h->small_dec && h->D <= SMALL_MAX && h->H <= SMALL_MAX; }
+
+// The kernel and data flow of a launch of n rows (multires: per-row start steps; steps: reverse steps of the chain), from the
+// packed geometries and the handle's options.
+static LaunchPlan plan_launch(const sdrm_handle* h, int64_t n, bool multires, int steps) {
+  LaunchPlan p;
+  // small denoisers (every width <= 64): the register / shared-memory resident chain (K6) instead of the tcgen05 engine
+  if (small_ok(h) && h->engine_choice != 1) {
+    p.k6 = true;
+    p.cluster = 0;   // 0 = not the cluster engine
+    return p;
+  }
+  // the chain's layers (first, hidden when nh > 0, out) in geometry s (1 = 8-chunk)
+  auto chain = [h](int s, auto f) {
+    for (int l = LAYER_FIRST; l <= LAYER_OUT; ++l)
+      if (l != LAYER_HIDDEN || h->nh > 0) f(h->layer[l].g[s]);
+  };
+  // Column-split mode (see the kernel): launches of a FEW row tiles (the dataset-sized calls of the reference: the latency
+  // regime).  A cluster of S CTAs per tile, CTA j computes the chunks c = j (mod S); one tile per cluster, all clusters resident
+  // at once.  Preferred: S = 8 in the 8-chunk geometry (second set of weight images); when 8 CTAs per tile do not fit, the largest
+  // S = 4 / 2 that does, in the normal geometry (denoisers of >= 2 chunks).  Measured against the pair flows on every BASELINE
+  // configuration and on mid-size launches up to 74 tiles (profiles/k1_split_r02.txt): always faster.
+  const long long n_tiles = (n + TILE_M - 1) / TILE_M;
+  {
+    int nch_min = 1 << 30, nch_max = 0;
+    chain(0, [&](const Geom& g) { nch_min = std::min(nch_min, g.NCH); nch_max = std::max(nch_max, g.NCH); });
+    const int ov = h->cluster_override;
+    auto fits = [&](int S) {
+      return h->split_resident[S] > 0 && n_tiles * S <= h->split_resident[S] && (h->grid_limit == 0 || n_tiles * S <= h->grid_limit);
+    };
+    // (multi-resolution chains too: the tile's start step is the maximum over its rows in every CTA of the cluster alike)
+    if (!h->no_split && (ov == 0 || ov >= 4) && std::max(h->L, h->D) > SMALL_MAX) {
+      const bool geom8 = geom8_packed(h);
+      const int s_norm = nch_max <= 2 ? 2 : nch_max <= 4 ? 4 : 8;   // cluster size that gives every chunk of the normal geometry its CTA
+      if ((ov == 0 || ov == 8) && fits(8) && (geom8 || nch_max > 4)) { p.split = 8; p.split_geom = geom8; }
+      else if (ov == 4 && fits(4)) p.split = 4;
+      else if (ov == 0 && nch_min >= 2) {
+        // more tiles than clusters of that size fit: smaller clusters, each CTA takes several chunks of a layer (c = j, j + S, ...)
+        for (int S = std::min(s_norm, 4); S >= 2 && !p.split; S >>= 1)
+          if (fits(S)) p.split = S;
+      }
+    }
+  }
+  if (p.split) {
+    p.cluster = 1;
+    p.grid = static_cast<int>(n_tiles) * p.split;
+    int nc_max = 16;
+    for (int l = 0; l < N_LAYERS; ++l)
+      if (l != LAYER_HIDDEN || h->nh > 0) nc_max = std::max(nc_max, h->layer[l].g[p.split_geom].NC);
+    p.split_stage_bytes = static_cast<uint32_t>(A_TILE_BYTES + (nc_max * 128 + 1023) / 1024 * 1024);
+    p.res_nstg = std::max(1, std::min(6, static_cast<int>(4u * STAGE_BYTES / p.split_stage_bytes)));
+    return p;
+  }
+  // full-resolution chains run on tcgen05 cta_group::2 CTA pairs (fewer weight bytes and more k-blocks in flight per SM);
+  // multi-resolution chains (per-tile step counts) and single-tile calls use single-CTA mode
+  // (multi-resolution chains too since the third r02 session: a pair runs the longer of its two tiles' chains)
+  int cluster = n_tiles >= 2 ? 2 : 1;
+  if (h->cluster_override == 1 || h->cluster_override == 2) cluster = h->cluster_override;
+  for (; cluster >= 1; cluster >>= 1) {
+    const int resident = h->resident[cluster];
+    if (resident <= 0) continue;
+    const long long want = (n_tiles + cluster - 1) / cluster * cluster;
+    p.grid = static_cast<int>(std::min<long long>(want, resident));
+    if (h->grid_limit > 0) p.grid = std::min(p.grid, std::max(cluster, h->grid_limit / cluster * cluster));
+    break;
+  }
+  p.cluster = cluster;
+  if (p.grid <= 0) return p;
+  // Sub-tiles: a pair that owns two or more row tiles interleaves two of them layer by layer (see the kernel)
+  const long long n_local = (n_tiles + p.grid - 1) / p.grid;
+  // Which of the three data flows a pair-mode launch takes (all bit-identical), measured on B200 with tools/shape_probe.py:
+  //   * two interleaved sub-tiles per CTA (streaming through the L2): narrow denoisers with several tiles per CTA.  A layer's UMMAs
+  //     are short there and the hand-off of a tile's layer hides behind the other tile's work: L = 96 / 128 / 200 / 264 / 300 at
+  //     80 000 - 150 000 users: +21 / +18 / +10 / +6.5 / +2.5 % over the best single-tile flow.  From ~320 columns on it loses (the
+  //     second tile doubles the scratch and the L2 traffic: cfg-2 widths -5 %, cfg 5 -8 % with the L2 hit rate down from 80 to 67 %);
+  //   * resident mode (below): everything else that fits it, except one-tile-per-CTA launches of very narrow denoisers (<= 128
+  //     columns: 0.798 vs 0.824 ms, the tile hand-off through the L2 is as fast and the weight stream keeps all 6 stages);
+  //   * one streaming tile per CTA: the wide denoisers (cfg 1, cfg 5).
+  int w_max = 0;
+  chain(0, [&](const Geom& g) { w_max = std::max(w_max, std::max(g.KB * KBLK, g.Np)); });
+  if (cluster == 2 && n_local >= 2 && !multires &&   // (multi-resolution pairs: one tile at a time)
+      (h->subtile_override == 2 || (h->subtile_override == 0 && w_max <= 320)))
+    p.n_sub = 2;
+  // Dead-buffer discard (pair mode, see the kernel's discard warp): whole k-blocks of a chain layer's input image that EVERY
+  // chain layer's epilogue rewrites completely (64-column blocks below the narrowest written width), so a partly written
+  // last k-block keeps the zero padding it got at kernel start.
+  if (cluster >= 2 && !h->no_discard && steps >= 2 && !multires) {   // (the discard warp counts P.T steps per tile)
+    int written = (h->L + 15) / 16 * 16, kb_read = 1 << 30;
+    chain(0, [&](const Geom& g) { written = std::min(written, g.Np); kb_read = std::min(kb_read, g.KB); });
+    p.discard_kb = std::max(0, std::min(written / KBLK, kb_read));
+  }
+  // Resident mode (see the kernel): every chain layer fits one pass of the accumulators (N <= 2 chunks = 512 TMEM columns) and
+  // the part of the stage ring the weight stream can spare (<= 8 k-blocks).  Built for the latency regime (one row tile per CTA:
+  // cfg 4 1.40 -> 1.31 ms), it also wins when a CTA owns several tiles: at these widths the streaming path is bound by L2 bandwidth
+  // (~9 TB/s of activation re-reads, weights, stores and state at 148 CTAs), and the resident tile removes the activation half of it
+  // (cfg-2 widths, 100 000 users: 14.91 -> 14.39 ms; cfg-4 widths, 60 000 users: 5.55 -> 5.26 ms).
+  if (cluster == 2 && p.n_sub == 1 && h->no_resident != 1 && !multires && (n_local >= 2 || w_max > 128)) {
+    int kb_max = 0;
+    bool ok = true;
+    chain(0, [&](const Geom& g) {
+      ok = ok && g.NCH <= 2;
+      kb_max = std::max(kb_max, std::max(g.KB, (g.Np + KBLK - 1) / KBLK));
+    });
+    if (ok && kb_max <= 8) {
+      p.resident = 1;
+      p.res_nstg = kb_max <= 6 ? 3 : 2;
+      p.discard_kb = 0;
+    }
+  }
+  return p;
+}
+
 // sdrm_sample and sdrm_sample_bf16: d_logits holds fp32 or (bf16) bfloat16 logits, ld_logits counts elements either way
 static int sample_impl(sdrm_handle* h, int64_t n, int64_t row_offset, const int32_t* d_t_start, const int32_t* d_row_ids,
                        uint64_t seed, float* d_x0_out, void* d_logits, int64_t ld_logits, bool bf16, const float* d_inj_xT,
                        const float* d_inj_z, const uint8_t* d_inj_mask, void* d_workspace, size_t workspace_bytes, void* stream) {
   if (!h) return sdrm_fail(SDRM_ERR_BAD_ARG, "sdrm_sample: null handle");
   if (!h->have_den || !h->have_dec) return sdrm_fail(SDRM_ERR_STATE, "sdrm_sample: pack denoiser and decoder first");
-  if (h->g1.K != h->L) return sdrm_fail(SDRM_ERR_STATE, "sdrm_sample: decoder latent dim != denoiser latent dim");
+  if (h->layer[LAYER_DEC1].g[0].K != h->L) return sdrm_fail(SDRM_ERR_STATE, "sdrm_sample: decoder latent dim != denoiser latent dim");
   if (n <= 0) return SDRM_OK;
   if (!d_logits || ld_logits < h->I) return sdrm_fail(SDRM_ERR_BAD_ARG, "sdrm_sample: logits buffer / ld");
   if (!d_workspace) return sdrm_fail(SDRM_ERR_BAD_ARG, "sdrm_sample: null workspace");
+  if (h->engine_choice == 2 && !small_ok(h)) return sdrm_fail(SDRM_ERR_UNSUPPORTED, "sdrm_sample: the small-chain kernel needs every width <= 64");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   SDRM_CUDA(cudaSetDevice(h->device));
   const bool on_grid = h->grid_S > 0;
   const int steps = on_grid ? h->grid_S : h->T;   // reverse steps of this launch (t_start entries are clamped to [0, steps])
-  // ---- small denoisers (every width <= 64): the register / shared-memory resident chain (K6) instead of the tcgen05 engine
-  const bool small_ok = h->small_den && h->small_dec && h->D <= SMALL_MAX && h->H <= SMALL_MAX;
-  if (h->engine_choice == 2 && !small_ok) return sdrm_fail(SDRM_ERR_UNSUPPORTED, "sdrm_sample: the small-chain kernel needs every width <= 64");
-  if (small_ok && h->engine_choice != 1) {
+  const LaunchPlan plan = plan_launch(h, n, d_t_start != nullptr, steps);
+  if (plan.k6) {
+    const long long ctas = (n + 16 * SMALL_WARPS - 1) / (16 * SMALL_WARPS);
+    if (ctas > 0x7fffffffLL) return sdrm_fail(SDRM_ERR_UNSUPPORTED, "sdrm_sample: too many rows for one launch");
     SmallParams S;
     memset(&S, 0, sizeof S);
     const size_t img = static_cast<size_t>(64) * SMALL_KP;
@@ -711,86 +798,42 @@ static int sample_impl(sdrm_handle* h, int64_t n, int64_t row_offset, const int3
     S.n_rows = n; S.row_offset = row_offset; S.ld_logits = ld_logits;
     S.t_start = d_t_start; S.row_ids = d_row_ids; S.x0_out = d_x0_out; S.logits = d_logits;
     S.inj_xT = d_inj_xT; S.inj_z = d_inj_z; S.inj_mask = d_inj_mask; S.seed = seed;
-    const int widest = std::max(std::max(h->L, h->D), h->H);
-    const int nt = (widest + 7) / 8;
-    const long long ctas = (n + 16 * SMALL_WARPS - 1) / (16 * SMALL_WARPS);
-    if (ctas > 0x7fffffffLL) return sdrm_fail(SDRM_ERR_UNSUPPORTED, "sdrm_sample: too many rows for one launch");
-    auto launch = [&](auto kernel, int smem) -> int {
-      SDRM_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-      kernel<<<static_cast<unsigned>(ctas), SMALL_THREADS, smem, st>>>(S);
-      SDRM_CUDA(cudaGetLastError());
-      return SDRM_OK;
-    };
-    int rc_s;
-    if (bf16) {
-      rc_s = launch_small_chain_bf16(S, nt, static_cast<unsigned>(ctas), st);
-    } else {
-      if (nt <= 3) rc_s = launch(sdrm_small_chain_kernel<3>, SmallGeom<3>::SMEM_BYTES);
-      else if (nt <= 5) rc_s = launch(sdrm_small_chain_kernel<5>, SmallGeom<5>::SMEM_BYTES);
-      else rc_s = launch(sdrm_small_chain_kernel<8>, SmallGeom<8>::SMEM_BYTES);
-    }
-    if (rc_s) return rc_s;
+    const int nt = (std::max(std::max(h->L, h->D), h->H) + 7) / 8;
+    const int rc = bf16 ? launch_small_chain_bf16(S, nt, static_cast<unsigned>(ctas), st)
+                        : launch_small_chain_t<false>(S, nt, static_cast<unsigned>(ctas), st);
+    if (rc) return rc;
+    h->last = plan;
     h->last_launches = 1;
-    h->last_cluster = 0;   // 0 = not the cluster engine
     return SDRM_OK;
   }
   int grid, mask_pitch; size_t act, stride, mask_off;
   sample_geometry(h, n, &grid, &act, &stride, &mask_off, &mask_pitch);
   if (workspace_bytes < static_cast<size_t>(grid) * stride) return sdrm_fail(SDRM_ERR_WORKSPACE, "sdrm_sample: workspace too small");
-  int rc = engine_set_smem_attr();
-  if (rc) return rc;
+  const long long n_tiles = (n + TILE_M - 1) / TILE_M;
+  if (plan.grid <= 0 || (plan.split ? n_tiles > grid : plan.grid > grid)) return sdrm_fail(SDRM_ERR_CUDA, "sdrm_sample: no launchable grid");
+  if (static_cast<size_t>(plan.split ? n_tiles : plan.grid) * plan.n_sub * stride > workspace_bytes)
+    return sdrm_fail(SDRM_ERR_WORKSPACE, "sdrm_sample: workspace too small for the sub-tile scratch slots");
 
   ChainParams P;
   memset(&P, 0, sizeof P);
-  auto fill = [](LayerDesc& d, const uint8_t* w, const float* bias, const float* slope, int bstride, const Geom& g,
-                 int passes, int kind, int in_hi, int in_lo, int out_hi, int out_lo) {
-    d.w_img = w; d.bias = bias; d.slope = slope; d.bias_step_stride = bstride;
-    d.KB = g.KB; d.kmma_last = g.kmma_last; d.passes = passes; d.NCH = g.NCH; d.NC = g.NC; d.kind = kind;
-    d.in_hi = in_hi; d.in_lo = in_lo; d.out_hi = out_hi; d.out_lo = out_lo; d.n_valid = g.N;
-  };
-  // chain layers ping-pong between activation buffers 0/1 (the kernel derives the parity); decoder descriptors name
-  // their hi buffers RELATIVE to the chain's last output (0 = that buffer, 1 = the other), lo buffers are 2 and 3
-  // Column-split mode (see the kernel): launches of a FEW row tiles (the dataset-sized calls of the reference: the latency
-  // regime).  A cluster of S CTAs per tile, CTA j computes the chunks c = j (mod S); one tile per cluster, all clusters resident
-  // at once.  Preferred: S = 8 in the 8-chunk geometry (second set of weight images); when 8 CTAs per tile do not fit, the largest
-  // S = 4 / 2 that does, in the normal geometry (denoisers of >= 2 chunks).  Measured against the pair flows on every BASELINE
-  // configuration and on mid-size launches up to 74 tiles (profiles/k1_split_r02.txt): always faster.
-  const long long n_tiles = (n + TILE_M - 1) / TILE_M;
-  int split = 0;
-  bool split_geom = false;
-  {
-    int nch_min = std::min(h->g0.NCH, h->go.NCH), nch_max = std::max(h->g0.NCH, h->go.NCH);
-    if (h->nh > 0) { nch_min = std::min(nch_min, h->gh.NCH); nch_max = std::max(nch_max, h->gh.NCH); }
-    const int ov = h->cluster_override;
-    auto fits = [&](int S) {
-      return h->split_resident[S] > 0 && n_tiles * S <= h->split_resident[S] && (h->grid_limit == 0 || n_tiles * S <= h->grid_limit);
-    };
-    // (multi-resolution chains too: the tile's start step is the maximum over its rows in every CTA of the cluster alike)
-    if (!h->no_split && (ov == 0 || ov >= 4) && std::max(h->L, h->D) > SMALL_MAX) {
-      const bool geom8 = h->split_den && h->split_dec;
-      const int s_norm = nch_max <= 2 ? 2 : nch_max <= 4 ? 4 : 8;   // cluster size that gives every chunk of the normal geometry its CTA
-      if ((ov == 0 || ov == 8) && fits(8) && (geom8 || nch_max > 4)) { split = 8; split_geom = geom8; }
-      else if (ov == 4 && fits(4)) split = 4;
-      else if (ov == 0 && nch_min >= 2) {
-        // more tiles than clusters of that size fit: smaller clusters, each CTA takes several chunks of a layer (c = j, j + S, ...)
-        for (int S = std::min(s_norm, 4); S >= 2 && !split; S >>= 1)
-          if (fits(S)) split = S;
-      }
-    }
+  // chain layers (first, nh x the shared hidden one, out) ping-pong between activation buffers 0/1 (the kernel derives the
+  // parity); decoder descriptors name their hi buffers RELATIVE to the chain's last output (0 = that buffer, 1 = the other),
+  // lo buffers are 2 and 3
+  const bool sg = plan.split_geom;
+  P.n_step = 2 + h->nh;
+  for (int j = 0; j < P.n_step; ++j) {
+    const int l = j == 0 ? LAYER_FIRST : j <= h->nh ? LAYER_HIDDEN : LAYER_OUT;
+    const PackedLayer& q = h->layer[l];
+    if (l == LAYER_FIRST)
+      fill_desc(P.step[j], q.image(sg), q.g[sg], on_grid ? h->grid_bias0 : q.bias, h->slopes, q.np, 1, EPI_PRELU, 0, 0, 0, 0);
+    else if (l == LAYER_HIDDEN)
+      fill_desc(P.step[j], q.image(sg), q.g[sg], q.bias, h->slopes + 1, 0, 1, EPI_PRELU, 0, 0, 0, 0);
+    else
+      fill_desc(P.step[j], q.image(sg), q.g[sg], q.bias, nullptr, 0, 1, EPI_POSTERIOR, 0, 0, 0, 0);
   }
-  h->last_split = split;
-  const Geom& G0 = split_geom ? h->s0 : h->g0;
-  const Geom& GH = split_geom ? h->sh : h->gh;
-  const Geom& GO = split_geom ? h->so : h->go;
-  const Geom& G1 = split_geom ? h->s1 : h->g1;
-  const Geom& G2 = split_geom ? h->s2 : h->g2;
-  int l = 0;
-  fill(P.step[l++], split_geom ? h->w0s : h->w0, on_grid ? h->grid_bias0 : h->bias0, h->slopes, h->np0, G0, 1, EPI_PRELU, 0, 0, 0, 0);
-  for (int j = 0; j < h->nh; ++j) fill(P.step[l++], split_geom ? h->whs : h->wh, h->bh, h->slopes + 1, 0, GH, 1, EPI_PRELU, 0, 0, 0, 0);
-  fill(P.step[l++], split_geom ? h->wos : h->wo, h->bo, nullptr, 0, GO, 1, EPI_POSTERIOR, 0, 0, 0, 0);
-  P.n_step = l;
-  fill(P.dec[0], (split_geom && h->w1s) ? h->w1s : h->w1, h->b1, nullptr, 0, G1, 3, EPI_TANH_SPLIT, 0, 2, 1, 3);
-  fill(P.dec[1], (split_geom && h->w2s) ? h->w2s : h->w2, h->b2, nullptr, 0, G2, 3, EPI_LINEAR_OUT, 1, 3, 0, 0);
+  const PackedLayer &dec1 = h->layer[LAYER_DEC1], &dec2 = h->layer[LAYER_DEC2];
+  fill_desc(P.dec[0], dec1.image(sg), dec1.g[sg], dec1.bias, nullptr, 0, 3, EPI_TANH_SPLIT, 0, 2, 1, 3);
+  fill_desc(P.dec[1], dec2.image(sg), dec2.g[sg], dec2.bias, nullptr, 0, 3, EPI_LINEAR_OUT, 1, 3, 0, 0);
   P.n_dec = 2;
   P.T = steps; P.L = h->L; P.Lg16 = (h->L + 15) / 16;
   P.preloaded_input = 0;
@@ -810,87 +853,19 @@ static int sample_impl(sdrm_handle* h, int64_t n, int64_t row_offset, const int3
   P.err_word = h->err_word;
   P.trace = h->trace;
   P.debug_flags = h->debug_flags;
-  int cluster = 1;
-  // full-resolution chains run on tcgen05 cta_group::2 CTA pairs (fewer weight bytes and more k-blocks in flight per SM);
-  // multi-resolution chains (per-tile step counts) and single-tile calls use single-CTA mode
-  // (multi-resolution chains too since the third r02 session: a pair runs the longer of its two tiles' chains)
-  if (n_tiles >= 2) cluster = 2;
-  if (h->cluster_override == 1 || h->cluster_override == 2) cluster = h->cluster_override;
-  int launch_grid = 0;
-  if (split) { cluster = 1; launch_grid = static_cast<int>(n_tiles) * split; }
-  else
-  for (; cluster >= 1; cluster >>= 1) {
-    const int resident = h->resident[cluster];
-    if (resident <= 0) continue;
-    const long long want = (n_tiles + cluster - 1) / cluster * cluster;
-    launch_grid = static_cast<int>(std::min<long long>(want, resident));
-    if (h->grid_limit > 0) launch_grid = std::min(launch_grid, std::max(cluster, h->grid_limit / cluster * cluster));
-    break;
-  }
-  if (launch_grid <= 0 || (split ? n_tiles > grid : launch_grid > grid)) return sdrm_fail(SDRM_ERR_CUDA, "sdrm_sample: no launchable grid");
-  h->last_cluster = cluster;
-  rc = fill_act_maps(P, static_cast<size_t>(grid) * stride);
+  P.n_sub = plan.n_sub;
+  P.resident = plan.resident;
+  P.res_nstg = plan.res_nstg;
+  P.discard_kb = plan.discard_kb;
+  P.split_stage_bytes = plan.split_stage_bytes;
+  int rc = fill_act_maps(P, static_cast<size_t>(grid) * stride);
   if (rc) return rc;
-  if (cluster >= 2) {
-    rc = fill_pair_maps(P, static_cast<size_t>(grid) * stride, cluster);
+  if (plan.cluster >= 2) {
+    rc = fill_pair_maps(P, plan.cluster);
     if (rc) return rc;
   }
-  // Sub-tiles: a pair that owns two or more row tiles interleaves two of them layer by layer (see the kernel)
-  const long long n_local = split ? 1 : (n_tiles + launch_grid - 1) / launch_grid;
-  // Which of the three data flows a pair-mode launch takes (all bit-identical), measured on B200 with tools/shape_probe.py:
-  //   * two interleaved sub-tiles per CTA (streaming through the L2): narrow denoisers with several tiles per CTA.  A layer's UMMAs
-  //     are short there and the hand-off of a tile's layer hides behind the other tile's work: L = 96 / 128 / 200 / 264 / 300 at
-  //     80 000 - 150 000 users: +21 / +18 / +10 / +6.5 / +2.5 % over the best single-tile flow.  From ~320 columns on it loses (the
-  //     second tile doubles the scratch and the L2 traffic: cfg-2 widths -5 %, cfg 5 -8 % with the L2 hit rate down from 80 to 67 %);
-  //   * resident mode (below): everything else that fits it, except one-tile-per-CTA launches of very narrow denoisers (<= 128
-  //     columns: 0.798 vs 0.824 ms, the tile hand-off through the L2 is as fast and the weight stream keeps all 6 stages);
-  //   * one streaming tile per CTA: the wide denoisers (cfg 1, cfg 5).
-  int w_max = 0;
-  for (int j = 0; j < P.n_step; ++j) w_max = std::max(w_max, std::max(P.step[j].KB * KBLK, P.step[j].NCH * P.step[j].NC));
-  P.n_sub = 1;
-  if (cluster == 2 && n_local >= 2 && P.n_step > 0 && d_t_start == nullptr &&   // (multi-resolution pairs: one tile at a time)
-      (h->subtile_override == 2 || (h->subtile_override == 0 && w_max <= 320)))
-    P.n_sub = 2;
-  // Dead-buffer discard (pair mode, see the kernel's discard warp): whole k-blocks of a chain layer's input image that EVERY
-  // chain layer's epilogue rewrites completely (64-column blocks below the narrowest written width), so a partly written
-  // last k-block keeps the zero padding it got at kernel start.
-  P.discard_kb = 0;
-  if (cluster >= 2 && !h->no_discard && steps >= 2 && d_t_start == nullptr) {   // (the discard warp counts P.T steps per tile)
-    const int written = std::min(std::min(h->g0.Np, h->nh > 0 ? h->gh.Np : h->g0.Np), std::min(h->go.Np, P.Lg16 * 16));
-    const int kb_read = std::min(std::min(h->g0.KB, h->nh > 0 ? h->gh.KB : h->g0.KB), h->go.KB);
-    P.discard_kb = std::max(0, std::min(written / KBLK, kb_read));
-  }
-  // Resident mode (see the kernel): every chain layer fits one pass of the accumulators (N <= 2 chunks = 512 TMEM columns) and
-  // the part of the stage ring the weight stream can spare (<= 8 k-blocks).  Built for the latency regime (one row tile per CTA:
-  // cfg 4 1.40 -> 1.31 ms), it also wins when a CTA owns several tiles: at these widths the streaming path is bound by L2 bandwidth
-  // (~9 TB/s of activation re-reads, weights, stores and state at 148 CTAs), and the resident tile removes the activation half of it
-  // (cfg-2 widths, 100 000 users: 14.91 -> 14.39 ms; cfg-4 widths, 60 000 users: 5.55 -> 5.26 ms).
-  P.resident = 0; P.res_nstg = 0;
-  if (cluster == 2 && P.n_sub == 1 && P.n_step > 0 && h->no_resident != 1 && d_t_start == nullptr && (n_local >= 2 || w_max > 128)) {
-    int kb_max = 0;
-    bool ok = true;
-    for (int j = 0; j < P.n_step; ++j) {
-      const LayerDesc& d = P.step[j];
-      ok = ok && d.NCH <= 2 && d.passes == 1;
-      kb_max = std::max(kb_max, std::max(d.KB, (d.NCH * d.NC + KBLK - 1) / KBLK));
-    }
-    if (ok && kb_max <= 8) {
-      P.resident = 1;
-      P.res_nstg = kb_max <= 6 ? 3 : 2;
-      P.discard_kb = 0;
-    }
-  }
-  h->last_resident = P.resident;
-  if (split) {
-    int nc_max = 16;
-    for (int j = 0; j < P.n_step; ++j) nc_max = std::max(nc_max, P.step[j].NC);
-    for (int j = 0; j < P.n_dec; ++j) nc_max = std::max(nc_max, P.dec[j].NC);
-    P.split_stage_bytes = static_cast<uint32_t>(A_TILE_BYTES + (nc_max * 128 + 1023) / 1024 * 1024);
-    P.res_nstg = std::max(1, std::min(6, static_cast<int>(4u * STAGE_BYTES / P.split_stage_bytes)));
-  }
-  if (static_cast<size_t>(split ? n_tiles : launch_grid) * P.n_sub * stride > workspace_bytes)
-    return sdrm_fail(SDRM_ERR_WORKSPACE, "sdrm_sample: workspace too small for the sub-tile scratch slots");
-  rc = launch_engine(P, launch_grid, cluster, st, split, bf16);
+  h->last = plan;
+  rc = launch_engine(P, plan.grid, plan.cluster, st, plan.split, bf16);
   if (rc) return rc;
   h->last_launches = 1;
   return SDRM_OK;
@@ -932,7 +907,8 @@ int sdrm_set_step_grid(sdrm_handle* h, const int32_t* timesteps, int S, int mode
   // (pageable source: the copy is staged before this call returns)
   SDRM_CUDA(cudaMemcpyAsync(h->grid_tau, tau.data(), sizeof(int32_t) * (S + 1), cudaMemcpyHostToDevice, st));
   grid_coef_kernel<<<(S + 1 + 127) / 128, 128, 0, st>>>(h->sched, h->T, h->grid_tau, S, mode, eta, h->nd, h->grid_coef);
-  grid_bias_kernel<<<S + 1, 256, 0, st>>>(h->bias0, h->np0, h->grid_tau, h->grid_bias0);
+  const PackedLayer& first = h->layer[LAYER_FIRST];
+  grid_bias_kernel<<<S + 1, 256, 0, st>>>(first.bias, first.np, h->grid_tau, h->grid_bias0);
   if (h->small_den) grid_bias_kernel<<<S + 1, 64, 0, st>>>(h->s_bias, 64, h->grid_tau, h->grid_s_bias);
   SDRM_CUDA(cudaGetLastError());
   h->grid_S = S;
@@ -942,8 +918,8 @@ int sdrm_set_step_grid(sdrm_handle* h, const int32_t* timesteps, int S, int mode
 int sdrm_step_grid_size(const sdrm_handle* h) { return h ? h->grid_S : 0; }
 
 int sdrm_last_launch_count(const sdrm_handle* h) { return h ? h->last_launches : 0; }
-int sdrm_last_resident_mode(const sdrm_handle* h) { return h ? h->last_resident : 0; }
-int sdrm_last_split_size(const sdrm_handle* h) { return h ? h->last_split : 0; }
+int sdrm_last_resident_mode(const sdrm_handle* h) { return h ? h->last.resident : 0; }
+int sdrm_last_split_size(const sdrm_handle* h) { return h ? h->last.split : 0; }
 
 int sdrm_check_device_error(sdrm_handle* h, void* stream) {
   if (!h) return sdrm_fail(SDRM_ERR_BAD_ARG, "null handle");
@@ -1020,7 +996,7 @@ int sdrm_set_option(sdrm_handle* h, int option, int64_t value) {
   }
 }
 int sdrm_resident_ctas(const sdrm_handle* h, int cluster) { return (h && cluster >= 1 && cluster <= 8) ? h->resident[cluster] : 0; }
-int sdrm_last_cluster_size(const sdrm_handle* h) { return h ? h->last_cluster : 0; }
+int sdrm_last_cluster_size(const sdrm_handle* h) { return h ? h->last.cluster : 0; }
 
 int sdrm_layer_geometry(int N, int K, int column_split, int* n_chunks, int* chunk_cols, int* k_blocks) {
   if (N < 1 || K < 1 || !n_chunks || !chunk_cols || !k_blocks) return sdrm_fail(SDRM_ERR_BAD_ARG, "sdrm_layer_geometry: bad argument");
@@ -1044,8 +1020,6 @@ int sdrm_probe_linear(const float* d_A, const float* d_W, const float* d_bias, f
   probe_geometry(M, K, N, &g, &act, &w_off, &b_off, &s_off, &total);
   if (workspace_bytes < total) return sdrm_fail(SDRM_ERR_WORKSPACE, "sdrm_probe_linear: workspace too small");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  int rc = engine_set_smem_attr();
-  if (rc) return rc;
   int dev = 0, sms = 0;
   SDRM_CUDA(cudaGetDevice(&dev));
   SDRM_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
@@ -1061,18 +1035,14 @@ int sdrm_probe_linear(const float* d_A, const float* d_W, const float* d_bias, f
   }
   ChainParams P;
   memset(&P, 0, sizeof P);
-  LayerDesc& d = P.dec[0];
-  d.w_img = ws + w_off; d.bias = reinterpret_cast<const float*>(ws + b_off); d.slope = nullptr;
-  d.bias_step_stride = 0; d.KB = g.KB; d.kmma_last = g.kmma_last; d.passes = split3 ? 3 : 1;
-  d.NCH = g.NCH; d.NC = g.NC; d.kind = EPI_LINEAR_OUT; d.in_hi = 0; d.in_lo = 1; d.out_hi = 0; d.out_lo = 0;
-  d.n_valid = N;
+  fill_desc(P.dec[0], ws + w_off, g, reinterpret_cast<const float*>(ws + b_off), nullptr, 0, split3 ? 3 : 1, EPI_LINEAR_OUT, 0, 1, 0, 0);
   P.n_step = 0; P.n_dec = 1; P.T = 0; P.L = K; P.Lg16 = 0; P.preloaded_input = 1; P.n_sub = 1;
   P.n_rows = M; P.row_offset = 0;
   P.logits = d_out; P.ld_logits = N;
   P.scratch = ws + s_off; P.scratch_stride = 2 * act; P.act_buf_bytes = act;
   P.err_word = reinterpret_cast<int*>(ws);
   const int grid = static_cast<int>(std::max<long long>(1, std::min<long long>(n_tiles, sms)));
-  rc = fill_act_maps(P, static_cast<size_t>(n_tiles) * 2 * act);
+  const int rc = fill_act_maps(P, static_cast<size_t>(n_tiles) * 2 * act);
   if (rc) return rc;
   return launch_engine(P, grid, 1, st);
 }

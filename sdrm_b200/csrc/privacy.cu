@@ -385,24 +385,9 @@ __global__ void __launch_bounds__(PREP_THREADS) csr_image_kernel(const int64_t* 
 // ---------------------------------------------------------------------------------------------------------------------
 // host side
 // ---------------------------------------------------------------------------------------------------------------------
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-static EncodeTiledFn encode_fn() {
-  static EncodeTiledFn fn = nullptr;
-  if (fn) return fn;
-  void* p = nullptr;
-  cudaDriverEntryPointQueryResult q;
-  if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) != cudaSuccess || q != cudaDriverEntryPointSuccess) {
-    cudaGetLastError();
-    return nullptr;
-  }
-  fn = reinterpret_cast<EncodeTiledFn>(p);
-  return fn;
-}
 // uint8 image [rows, pitch]: box = 128 columns x box_rows rows, SWIZZLE_128B
 static int make_u8_map(CUtensorMap* map, const void* base, long long rows, long long pitch, unsigned box_rows) {
-  EncodeTiledFn fn = encode_fn();
+  EncodeTiledFn fn = encode_tiled_fn();
   if (!fn) return sdrm_fail(SDRM_ERR_CUDA, "cuTensorMapEncodeTiled entry point not available");
   const cuuint64_t dims[2] = {static_cast<cuuint64_t>(pitch), static_cast<cuuint64_t>(rows)};
   const cuuint64_t strides[1] = {static_cast<cuuint64_t>(pitch)};
@@ -415,17 +400,6 @@ static int make_u8_map(CUtensorMap* map, const void* base, long long rows, long 
     snprintf(msg, sizeof msg, "cuTensorMapEncodeTiled (u8) failed (%d) rows=%lld pitch=%lld box_rows=%u", static_cast<int>(r), rows, pitch, box_rows);
     return sdrm_fail(SDRM_ERR_CUDA, msg);
   }
-  return SDRM_OK;
-}
-
-static int apply_watchdog_env_k8() {
-  static bool done = false;
-  if (done) return SDRM_OK;
-  done = true;
-  const char* e = getenv("SDRM_WATCHDOG_MS");
-  if (!e || !*e) return SDRM_OK;
-  const unsigned long long ns = strtoull(e, nullptr, 10) * 1000000ull;
-  SDRM_CUDA(cudaMemcpyToSymbol(sdrm::g_sdrm_watchdog_ns, &ns, sizeof ns));
   return SDRM_OK;
 }
 
@@ -545,7 +519,7 @@ int sdrm_privacy_nearest(const uint8_t* d_q_image, const int32_t* d_q_ones, int6
   if ((reinterpret_cast<uintptr_t>(d_q_image) | reinterpret_cast<uintptr_t>(d_r_image) | reinterpret_cast<uintptr_t>(d_r_ones) |
        reinterpret_cast<uintptr_t>(d_workspace)) & 15)
     return sdrm_fail(SDRM_ERR_BAD_ARG, "sdrm_privacy_nearest: images, reference ones and workspace must be 16-byte aligned");
-  { int wrc = apply_watchdog_env_k8(); if (wrc) return wrc; }
+  { int wrc = sdrm::apply_watchdog_env(); if (wrc) return wrc; }
   int s = 0;
   { int rc = resolve_splits(n, m, splits, &s); if (rc) return rc; }
   const size_t need = sdrm_privacy_workspace_bytes(n, m, k, s);

@@ -5,6 +5,9 @@
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
+#include <stdlib.h>
+
+#include "host_util.h"
 
 namespace sdrm {
 
@@ -64,13 +67,27 @@ __device__ __forceinline__ uint64_t globaltimer_ns() {
 }
 
 // Watchdog: a protocol bug must become an error code, never a hung GPU box.  The limit is a run-time value (per translation
-// unit: sdrm_set_watchdog_* in the host files copy it in; environment variable SDRM_WATCHDOG_MS, 0 = no limit), because the
+// unit: apply_watchdog_env below copies it in; environment variable SDRM_WATCHDOG_MS, 0 = no limit), because the
 // global timer keeps running while a context is preempted (time-sliced GPU, debugger, profiler replay) and a healthy run must
 // not be killed there.
 #ifndef SDRM_WATCHDOG_NS
 #define SDRM_WATCHDOG_NS 4000000000ull
 #endif
 static __constant__ unsigned long long g_sdrm_watchdog_ns = SDRM_WATCHDOG_NS;
+// Copies SDRM_WATCHDOG_MS into the calling translation unit's g_sdrm_watchdog_ns (static, so each unit's module has its own
+// copy) on the current device, once per device: every device a process uses gets the limit.
+static inline int apply_watchdog_env() {
+  static bool done[64] = {false};
+  int dev = 0;
+  SDRM_CUDA(cudaGetDevice(&dev));
+  if (dev < 64 && done[dev]) return 0;
+  if (dev < 64) done[dev] = true;
+  const char* e = getenv("SDRM_WATCHDOG_MS");
+  if (!e || !*e) return 0;
+  const unsigned long long ns = strtoull(e, nullptr, 10) * 1000000ull;
+  SDRM_CUDA(cudaMemcpyToSymbol(g_sdrm_watchdog_ns, &ns, sizeof ns));
+  return 0;
+}
 // try_wait with a suspend-time hint: the waiting thread is parked by the hardware until the phase completes or the hint
 // (ns) expires, so a waiter neither issues poll instructions nor wakes up late.  (The polling loops with __nanosleep were
 // 45 % of all executed warp instructions of the engine kernel — ncu source page, r01 — and every epilogue warp woke up

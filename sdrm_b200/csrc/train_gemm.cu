@@ -133,24 +133,9 @@ static thread_local long long g_train_launches = 0;   // kernels of this file la
 // ------------------------------------------------------------------------------------------------
 // launch helpers
 // ------------------------------------------------------------------------------------------------
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-static EncodeTiledFn gemm_encode_fn() {
-  static EncodeTiledFn fn = nullptr;
-  if (fn) return fn;
-  void* p = nullptr;
-  cudaDriverEntryPointQueryResult q;
-  if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) != cudaSuccess || q != cudaDriverEntryPointSuccess) {
-    cudaGetLastError();
-    return nullptr;
-  }
-  fn = reinterpret_cast<EncodeTiledFn>(p);
-  return fn;
-}
 // bf16 matrix [rows, cols] with row pitch ld (elements, multiple of 8): box = 64 columns x box_rows rows, SWIZZLE_128B
 static int make_bf16_map(CUtensorMap* map, const void* base, long long rows, long long cols, long long ld, unsigned box_rows) {
-  EncodeTiledFn fn = gemm_encode_fn();
+  EncodeTiledFn fn = encode_tiled_fn();
   if (!fn) return sdrm_fail(SDRM_ERR_CUDA, "cuTensorMapEncodeTiled entry point not available");
   const cuuint64_t dims[2] = {static_cast<cuuint64_t>(cols), static_cast<cuuint64_t>(rows)};
   const cuuint64_t strides[1] = {static_cast<cuuint64_t>(ld) * 2};
@@ -173,20 +158,8 @@ struct Bf16Mat {   // hi / lo images of one fp32 matrix
 };
 
 
-// run-time watchdog limit of this translation unit's kernels (ptx_sm100.cuh): SDRM_WATCHDOG_MS in the environment, 0 = none
-static int apply_watchdog_env_k5() {
-  static bool done = false;
-  if (done) return SDRM_OK;
-  done = true;
-  const char* e = getenv("SDRM_WATCHDOG_MS");
-  if (!e || !*e) return SDRM_OK;
-  const unsigned long long ns = strtoull(e, nullptr, 10) * 1000000ull;
-  SDRM_CUDA(cudaMemcpyToSymbol(sdrm::g_sdrm_watchdog_ns, &ns, sizeof ns));
-  return SDRM_OK;
-}
-
 static int gemm_clusters(int* out) {
-  { int wrc = apply_watchdog_env_k5(); if (wrc) return wrc; }
+  { int wrc = apply_watchdog_env(); if (wrc) return wrc; }
   static int cached[64];
   static bool have[64] = {false};
   int dev = 0;

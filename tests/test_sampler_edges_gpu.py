@@ -14,9 +14,8 @@ from test_sampler_gpu import TOL, TOL_MAX, _engine
 pytestmark = pytest.mark.gpu
 
 # flow -> (options that force it, (sdrm_last_cluster_size, sdrm_last_split_size, sdrm_last_resident_mode) that prove it ran).
-# K6 leaves the split / resident words of the handle alone (None: not checked).
 FLOWS = {
-    "k6": ({_lib.OPT_ENGINE: 2}, (0, None, None)),
+    "k6": ({_lib.OPT_ENGINE: 2}, (0, 0, 0)),
     "single": ({_lib.OPT_ENGINE: 1, _lib.OPT_CLUSTER: 1, _lib.OPT_NO_SPLIT: 1}, (1, 0, 0)),
     "pair": ({_lib.OPT_ENGINE: 1, _lib.OPT_CLUSTER: 2, _lib.OPT_NO_SPLIT: 1, _lib.OPT_RESIDENT: 1}, (2, 0, 0)),
     # one CTA pair for the whole launch: every CTA runs several row tiles one after the other
