@@ -43,6 +43,8 @@ def build_parser():
     p.add_argument("--seed", type=int, default=None, help="seed torch / numpy for a reproducible run")
     p.add_argument("--privacy-audit", action="store_true", default=False,
                    help="after each run, print how close the binarised synthetic rows come to the training rows (privacy_audit)")
+    p.add_argument("--fidelity-audit", action="store_true", default=False,
+                   help="after each run, print how closely the binarised synthetic rows resemble the training rows (fidelity_audit)")
     return p
 
 
@@ -92,6 +94,36 @@ def privacy_audit(binarised, real, baseline=None):
     return table, baseline
 
 
+FIDELITY_COLS = ["ones/user", "activity KS", "item freq r", "item freq rho", "item TV", "item coverage", "phi PCD",
+                 "phi RMSE", "phi corr", "neighbour recall@k"]
+FIDELITY_SPLIT_SEED = 123
+
+
+def fidelity_audit(binarised, real, baseline=None):
+    """Fidelity of every binarised synthetic row set to `real` (TRAIN_PARTIAL_VALID_DATA): user activity, item frequencies, the
+    pairwise item correlation (phi) and item-neighbour recall (sdrm_b200.fidelity.FidelityReport.summary), with k = 10 nearest
+    items (fewer when there are fewer items).  The baseline line compares two random halves of the real rows, split by a
+    private generator so the run's global random state is untouched: it is the metrics' noise floor at that sample size.
+    Returns (table, baseline summary)."""
+    import pandas as pd
+
+    from sdrm_b200.fidelity import compare
+    n_items = real.shape[1]
+    k = min(10, n_items - 1) if n_items > 1 else None
+    if baseline is None:
+        perm = np.random.default_rng(FIDELITY_SPLIT_SEED).permutation(real.shape[0])
+        half = real.shape[0] // 2
+        baseline = compare(real[np.sort(perm[:half])], real[np.sort(perm[half:])], k=k).summary()
+    rows = {}
+    for name, (dense, packed) in binarised.items():
+        rows[name] = compare(real, packed if packed is not None else dense, k=k).summary()
+    rows["real split-half (baseline)"] = baseline
+    keys = ["ones_per_user_synth", "activity_ks", "item_freq_pearson", "item_freq_spearman", "item_tv", "item_coverage",
+            "phi_pcd", "phi_rmse", "phi_corr", "neighbour_recall_at_k"]
+    table = pd.DataFrame([[s[k] for k in keys] for s in rows.values()], index=list(rows), columns=FIDELITY_COLS)
+    return table, baseline
+
+
 def main(argv=None):
     args = build_parser().parse_args(argv)
     import pandas as pd
@@ -120,6 +152,7 @@ def main(argv=None):
     model = args.model.lower()
     results = {c: [] for c in COLS}
     audit_baseline = None
+    fidelity_baseline = None
     for run_n in range(args.runs):
         start_time = time.time()
         print(10 * "#", "Starting run", run_n + 1, 10 * "#")
@@ -148,6 +181,9 @@ def main(argv=None):
         if args.privacy_audit:
             audit, audit_baseline = privacy_audit({c: binarised[c] for c in COLS}, TRAIN_PARTIAL_VALID_DATA, audit_baseline)
             print(f"\nPrivacy audit (run {run_n + 1}): distance to the closest training row\n{audit.round(4).to_markdown()}")
+        if args.fidelity_audit:
+            fid, fidelity_baseline = fidelity_audit({c: binarised[c] for c in COLS}, TRAIN_PARTIAL_VALID_DATA, fidelity_baseline)
+            print(f"\nFidelity audit (run {run_n + 1}): synthetic rows against the training rows\n{fid.round(4).to_markdown()}")
         for name, frame in synth.items():
             if model == "svd":
                 # NOTE: the flag is passed as only_synthetic=, exactly like the reference (main.py:189-194)

@@ -76,6 +76,11 @@ SIGNATURES = {
     "sdrm_privacy_workspace_bytes": (C.c_size_t, [C.c_int64, C.c_int64, C.c_int, C.c_int]),
     "sdrm_privacy_nearest": (C.c_int, [_P, _P, C.c_int64, _P, _P, C.c_int64, C.c_int, C.c_int64, C.c_int, C.c_int, C.c_int64,
                                        C.c_int, _P, _P, _P, _P, C.c_size_t, _P]),
+    "sdrm_fidelity_item_image_bits": (C.c_int, [_P, C.c_int64, C.c_int64, C.c_int, _P, C.c_int64, _P, _P, _P]),
+    "sdrm_fidelity_item_image_csr": (C.c_int, [_P, _P, _P, C.c_int64, C.c_int64, C.c_int, _P, C.c_int64, _P, _P, _P, _P]),
+    "sdrm_fidelity_workspace_bytes": (C.c_size_t, [C.c_int]),
+    "sdrm_fidelity_pair_stats": (C.c_int, [_P, _P, C.c_int64, C.c_int64, _P, _P, C.c_int64, C.c_int64, C.c_int, _P, _P,
+                                           C.c_size_t, _P]),
 }
 
 

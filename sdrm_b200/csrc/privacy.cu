@@ -385,23 +385,7 @@ __global__ void __launch_bounds__(PREP_THREADS) csr_image_kernel(const int64_t* 
 // ---------------------------------------------------------------------------------------------------------------------
 // host side
 // ---------------------------------------------------------------------------------------------------------------------
-// uint8 image [rows, pitch]: box = 128 columns x box_rows rows, SWIZZLE_128B
-static int make_u8_map(CUtensorMap* map, const void* base, long long rows, long long pitch, unsigned box_rows) {
-  EncodeTiledFn fn = encode_tiled_fn();
-  if (!fn) return sdrm_fail(SDRM_ERR_CUDA, "cuTensorMapEncodeTiled entry point not available");
-  const cuuint64_t dims[2] = {static_cast<cuuint64_t>(pitch), static_cast<cuuint64_t>(rows)};
-  const cuuint64_t strides[1] = {static_cast<cuuint64_t>(pitch)};
-  const cuuint32_t box[2] = {static_cast<cuuint32_t>(KB), box_rows};
-  const cuuint32_t estr[2] = {1, 1};
-  CUresult r = fn(map, CU_TENSOR_MAP_DATA_TYPE_UINT8, 2, const_cast<void*>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                  CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) {
-    char msg[160];
-    snprintf(msg, sizeof msg, "cuTensorMapEncodeTiled (u8) failed (%d) rows=%lld pitch=%lld box_rows=%u", static_cast<int>(r), rows, pitch, box_rows);
-    return sdrm_fail(SDRM_ERR_CUDA, msg);
-  }
-  return SDRM_OK;
-}
+static_assert(KB == 128, "make_u8_map (host_util.h) loads boxes of 128 columns");
 
 static int k_lists(int k) { return k <= 1 ? 1 : k <= 2 ? 2 : k <= 4 ? 4 : k <= 8 ? 8 : 16; }
 

@@ -129,9 +129,9 @@ def _device_of(x):
     return None
 
 
-def _csr_image(indptr, indices, values, rows, n_cols, dev):
-    """Operand image from CSR arrays (any integer / value dtypes; values None = every stored entry is an interaction)."""
-    lib = _lib.load()
+def _csr_device(indptr, indices, values, rows, dev):
+    """CSR arrays (any integer / value dtypes; values None = every stored entry is an interaction) as the prep kernels take
+    them: int64 indptr and indices, float32 values or None, contiguous on `dev`."""
     indptr = torch.as_tensor(indptr).to(device=dev, dtype=torch.int64).contiguous()
     indices = torch.as_tensor(indices).to(device=dev, dtype=torch.int64).contiguous()
     if values is not None:
@@ -143,6 +143,37 @@ def _csr_image(indptr, indices, values, rows, n_cols, dev):
         raise ValueError(f"CSR indptr must have rows + 1 = {rows + 1} entries, got shape {tuple(indptr.shape)}")
     if values is not None and values.numel() != indices.numel():
         raise ValueError("CSR values and indices must have the same length")
+    return indptr, indices, values
+
+
+def _csr_arrays(x, kind, rows, dev):
+    """The CSR arrays of a sparse or dense row set (every kind but "bits")."""
+    if kind == "device_csr":
+        return _csr_device(x.indptr, x.indices, x.values, rows, dev)
+    if kind == "torch_csr":
+        return _csr_device(x.crow_indices(), x.col_indices(), x.values(), rows, dev)
+    if kind == "scipy":
+        x = x.tocsr()
+        return _csr_device(torch.from_numpy(x.indptr.astype(np.int64)), torch.from_numpy(x.indices.astype(np.int64)),
+                           torch.from_numpy(np.asarray(x.data != 0, dtype=np.float32)), rows, dev)
+    t = torch.as_tensor(np.ascontiguousarray(x)) if isinstance(x, np.ndarray) else x
+    csr = (t.to(dev) != 0).to(torch.float32).to_sparse_csr()   # dense rows: nonzero = 1
+    return _csr_device(csr.crow_indices(), csr.col_indices(), None, rows, dev)
+
+
+def _raise_csr_status(status, nnz, n_cols):
+    """ValueError for the sdrm_privacy_status bits a CSR prep kernel set (reading them synchronises with the stream)."""
+    st = int(status.item())
+    if st & _BAD_INDPTR:
+        raise ValueError(f"CSR indptr must be non-decreasing within [0, {nnz}] (the number of stored entries)")
+    if st & _BAD_INDEX:
+        raise ValueError(f"CSR indices has entries outside [0, {n_cols})")
+
+
+def _csr_image(indptr, indices, values, rows, n_cols, dev):
+    """Operand image from CSR arrays (any integer / value dtypes; values None = every stored entry is an interaction)."""
+    lib = _lib.load()
+    indptr, indices, values = _csr_device(indptr, indices, values, rows, dev)
     pitch = int(lib.sdrm_privacy_image_pitch(n_cols))
     img = torch.empty((rows, pitch), dtype=torch.uint8, device=dev)
     ones = torch.empty(rows, dtype=torch.int32, device=dev)
@@ -152,11 +183,8 @@ def _csr_image(indptr, indices, values, rows, n_cols, dev):
                                           _lib.ptr(values) if values is not None and nnz else None, nnz, rows, n_cols,
                                           _lib.ptr(img), pitch, _lib.ptr(ones), _lib.ptr(status), _lib.stream_ptr()),
                "sdrm_privacy_image_csr")
-    st = int(status.item()) if rows else 0
-    if st & _BAD_INDPTR:
-        raise ValueError(f"CSR indptr must be non-decreasing within [0, {nnz}] (the number of stored entries)")
-    if st & _BAD_INDEX:
-        raise ValueError(f"CSR indices has entries outside [0, {n_cols})")
+    if rows:
+        _raise_csr_status(status, nnz, n_cols)
     return img, ones
 
 
@@ -174,17 +202,7 @@ def _image(x, kind, rows, n_cols, dev):
                                                _lib.ptr(img), pitch, _lib.ptr(ones), _lib.stream_ptr()),
                    "sdrm_privacy_image_bits")
         return img, ones
-    if kind == "device_csr":
-        return _csr_image(x.indptr, x.indices, x.values, rows, n_cols, dev)
-    if kind == "torch_csr":
-        return _csr_image(x.crow_indices(), x.col_indices(), x.values(), rows, n_cols, dev)
-    if kind == "scipy":
-        x = x.tocsr()
-        return _csr_image(torch.from_numpy(x.indptr.astype(np.int64)), torch.from_numpy(x.indices.astype(np.int64)),
-                          torch.from_numpy(np.asarray(x.data != 0, dtype=np.float32)), rows, n_cols, dev)
-    t = torch.as_tensor(np.ascontiguousarray(x)) if isinstance(x, np.ndarray) else x
-    csr = (t.to(dev) != 0).to(torch.float32).to_sparse_csr()   # dense rows: nonzero = 1
-    return _csr_image(csr.crow_indices(), csr.col_indices(), None, rows, n_cols, dev)
+    return _csr_image(*_csr_arrays(x, kind, rows, dev), rows, n_cols, dev)
 
 
 def _search(q_img, q_ones, r_img, r_ones, n_items, k, exclude_same_index=False, q_index_offset=0, splits=0):
