@@ -530,7 +530,9 @@ __global__ void __launch_bounds__(ENGINE_THREADS, 1) sdrm_layer_engine_kernel(co
           const int KB = ldref.KB, NCH = ldref.NCH, passes = ldref.passes, kmma_last = ldref.kmma_last;
           const uint32_t idesc = umma_idesc_bf16(PAIR ? 256 : 128, ldref.NC);
           const bool res_layer = RES && chain;
-          const int half_kb = (ldref.NC - 1) >> 6;   // last k-block under the first chunk's output columns
+          // last input k-block under the first chunk's output columns: every input k-block when the output is the wider image
+          // (a layer whose hidden width D differs from its latent width L, e.g. N = 2 x 256 over K = 128)
+          const int half_kb = min((ldref.NC - 1) >> 6, KB - 1);
           if (res_layer) {
             // both halves of the M = 256 input tile are in place (and the previous layer's accumulators have been read)
             mbar_wait(bar_a_ready, a_par, err, WD_MMA_AREADY);
@@ -585,6 +587,9 @@ __global__ void __launch_bounds__(ENGINE_THREADS, 1) sdrm_layer_engine_kernel(co
                     if (nk > 2) umma_bf16_ss_pair(d_tmem, a_desc + 4u, b_desc + 4u, idesc, 1u);
                     if (nk > 3) umma_bf16_ss_pair(d_tmem, a_desc + 6u, b_desc + 6u, idesc, 1u);
                     umma_commit_pair(bar_empty(stage), static_cast<uint16_t>((1u << CS) - 1u));   // every CTA of the cluster
+                    // (a resident layer of odd KB ends on a lone k-block: the first chunk's columns may end there)
+                    if (res_layer && NCH == 2 && c == 1 && kb == half_kb)
+                      umma_commit_pair(bar_half_read, static_cast<uint16_t>(0x3u << leader_rank));
                   } else {
 #ifdef SDRM_PERF_DEBUG
                     if (!(P.debug_flags & 2048))   // (experiment: no UMMAs, only the commits -- the pace of the barrier machinery alone)
