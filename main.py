@@ -45,6 +45,10 @@ def build_parser():
                    help="after each run, print how close the binarised synthetic rows come to the training rows (privacy_audit)")
     p.add_argument("--fidelity-audit", action="store_true", default=False,
                    help="after each run, print how closely the binarised synthetic rows resemble the training rows (fidelity_audit)")
+    p.add_argument("--save-generator", type=str, default=None, metavar="DIR",
+                   help="write each run's trained denoiser + VAE to DIR/run{n}_generator.pt (python -m sdrm_b200.synthesize reads it)")
+    p.add_argument("--save-synthetic", type=str, default=None, metavar="DIR",
+                   help="write each run's binarised synthetic rows to DIR/run{n}_{F-SDRM,M-SDRM,MultiVAE++}.npz (scipy sparse CSR)")
     return p
 
 
@@ -124,6 +128,18 @@ def fidelity_audit(binarised, real, baseline=None):
     return table, baseline
 
 
+def save_synthetic(binarised, out_dir, run):
+    """Each binarised row set as DIR/run{run}_{name}.npz: the GPU rows through K10 (PackedMatrix.to_sparse, no dense host copy),
+    host rows through csr_matrix.  Draws from no random generator."""
+    import os
+
+    import scipy.sparse as sp
+    os.makedirs(out_dir, exist_ok=True)
+    for name, (dense, packed) in binarised.items():
+        mat = packed.to_sparse().to_scipy() if packed is not None else sp.csr_matrix(dense)
+        sp.save_npz(os.path.join(out_dir, f"run{run}_{name}.npz"), mat)
+
+
 def main(argv=None):
     args = build_parser().parse_args(argv)
     import pandas as pd
@@ -163,6 +179,13 @@ def main(argv=None):
             TIMESTEPS=args.SDRM_timesteps, noise_divider=args.SDRM_noise_variance_diminisher, VAE_DIR_PATH="./temp_vae",
             TRAIN_PARTIAL_VALID_DATA=TRAIN_PARTIAL_VALID_DATA, VALID_DATA=VALID_DATA,
             OPTIMIZATION_OBJECTIVE="Recall@10", verbose=True)
+        if args.save_generator:
+            import os
+
+            from sdrm_b200.synthesize import save_generator
+            os.makedirs(args.save_generator, exist_ok=True)
+            save_generator(os.path.join(args.save_generator, f"run{run_n + 1}_generator.pt"), SDRM, VAE,
+                           noise_divider=args.SDRM_noise_variance_diminisher, sparsity=SPARSITY)
 
         print("Sampling Multi-resolution Data")
         M_SDRM = sample_ddpm(N_USERS, SDRM, VAE, args.MLP_latent_neurons, args.SDRM_noise_variance_diminisher,
@@ -178,6 +201,8 @@ def main(argv=None):
             "MultiVAE++": binarise(VAE.sample(N_USERS), SPARSITY),
         }
         synth = {name: pd.DataFrame(dense) for name, (dense, _) in binarised.items()}
+        if args.save_synthetic:
+            save_synthetic({c: binarised[c] for c in COLS}, args.save_synthetic, run_n + 1)
         if args.privacy_audit:
             audit, audit_baseline = privacy_audit({c: binarised[c] for c in COLS}, TRAIN_PARTIAL_VALID_DATA, audit_baseline)
             print(f"\nPrivacy audit (run {run_n + 1}): distance to the closest training row\n{audit.round(4).to_markdown()}")

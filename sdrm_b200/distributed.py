@@ -41,12 +41,18 @@ def sample_ddpm_sharded(n_sample, diff_net, vae_net, diff_latent_dim, noise_divi
     gather="bits"     -> equal-sparsity binarisation with the GLOBAL np.quantile threshold (sparsity = the reference's SPARSITY,
                          main.py:177-178) and an all_gather of the BIT-PACKED rows (32x less NVLink traffic: 312 MB per GPU at the
                          scale-up shape); returns (PackedMatrix of all n_sample rows, (0, n_sample))
+    gather="csr"      -> the same binarisation, each rank's shard converted to CSR on the device (kernel K10), then an all_gather of
+                         the per-rank nnz and of the shards' indices padded to the largest one; the indptr blocks are rebased on
+                         the device.  Returns (SparseRows of all n_sample rows, (0, n_sample)).  At 1 % ones a row costs 4 bytes per
+                         one + 8 as CSR against I / 8 as bits: fewer bytes to gather and to copy to the host when the rows are sparse
     out_dtype=torch.bfloat16 samples bfloat16 rows (the rounded float32 rows, sample_ddpm's out_dtype): gather=False / True then
     return / gather bfloat16 blocks (half the NVLink bytes), and gather="bits" binarises the bfloat16 rows (sparsify.py: ties
     at the threshold can keep a few more ones than the float32 rows would).
     sampling_steps / eta choose a fewer-step chain (sample_ddpm); multi-resolution rows map their drawn t_j onto its grid.
     An empty block (more ranks than rows) is legal: the rank still takes part in the collectives."""
     import numpy as np
+    if isinstance(gather, str) and gather == "csr" and sparsity is None:
+        raise ValueError("gather='csr' needs the sparsity of the binarisation")
     if sampler is None:
         from .train_SDRM import sample_ddpm as sampler
     rank = dist.get_rank(group) if dist.is_initialized() else 0
@@ -66,7 +72,12 @@ def sample_ddpm_sharded(n_sample, diff_net, vae_net, diff_latent_dim, noise_divi
         if gather == "bits":
             from .sparsify import equal_sparsity_device
             return equal_sparsity_device(rows, sparsity), (0, n_sample)
+        if gather == "csr":
+            from .sparsify import equal_sparsity_device
+            return equal_sparsity_device(rows, sparsity).to_sparse(), (0, n_sample)
         return rows, (lo, hi)
+    if gather == "csr":
+        return _gather_csr(rows, sparsity, n_sample, world, group), (0, n_sample)
     cap = shard_bounds(n_sample, 0, world)[1]  # largest block
     if gather == "bits":
         from .sparsify import PackedMatrix, equal_sparsity_device
@@ -90,6 +101,34 @@ def sample_ddpm_sharded(n_sample, diff_net, vae_net, diff_latent_dim, noise_divi
     out = torch.cat([p[: shard_bounds(n_sample, r, world)[1] - shard_bounds(n_sample, r, world)[0]]
                      for r, p in enumerate(parts)], dim=0)
     return out, (0, n_sample)
+
+
+def _gather_csr(rows, sparsity, n_sample, world, group):
+    """gather='csr' over `world` ranks: global-threshold binarisation and K10 on this rank's block, then two all_gathers (per-rank
+    nnz; indptr blocks and indices padded to the largest block) and the rebase of each indptr block by the nnz before it."""
+    from .sparsify import SparseRows, equal_sparsity_device
+    pm = equal_sparsity_device(rows, sparsity, group=group if group is not None else dist.group.WORLD)
+    local = pm.to_sparse()
+    dev = local.indptr.device
+    nnz = torch.tensor([local.nnz], dtype=torch.int64, device=dev)
+    nnzs = [torch.empty_like(nnz) for _ in range(world)]
+    dist.all_gather(nnzs, nnz, group=group)
+    counts = torch.cat(nnzs).tolist()
+    sizes = [shard_bounds(n_sample, r, world)[1] - shard_bounds(n_sample, r, world)[0] for r in range(world)]
+    ends = local.indptr.new_zeros(max(1, max(sizes)))   # indptr[1:] of the block, padded
+    ends[: sizes[dist.get_rank(group)]] = local.indptr[1:]
+    idx = local.indices.new_zeros(max(1, max(counts)))  # (NCCL gets at least one element)
+    idx[: local.nnz] = local.indices
+    ends_all = [torch.empty_like(ends) for _ in range(world)]
+    idx_all = [torch.empty_like(idx) for _ in range(world)]
+    dist.all_gather(ends_all, ends, group=group)
+    dist.all_gather(idx_all, idx, group=group)
+    base, blocks = 0, [local.indptr.new_zeros(1)]
+    for r in range(world):
+        blocks.append(ends_all[r][: sizes[r]] + base)
+        base += counts[r]
+    indices = torch.cat([idx_all[r][: counts[r]] for r in range(world)])
+    return SparseRows(torch.cat(blocks), indices, local.n_cols, pm.threshold)
 
 
 def unique_parameters(module):

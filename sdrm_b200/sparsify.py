@@ -197,6 +197,75 @@ class PackedMatrix:
         dense = np.unpackbits(words.view(np.uint8), axis=1, bitorder="little")[:, : self.n_cols]
         return dense.astype(dtype)
 
+    def to_sparse(self):
+        """The same rows as CSR on the device (kernel K10): a SparseRows.  Reads back one value, nnz, to size `indices`."""
+        return packed_to_csr(self.bits, self.n_cols, threshold=self.threshold)
+
+
+class SparseRows:
+    """Binary rows in CSR form on the device: `indptr` int64[rows + 1], `indices` int32[nnz] (ascending within each row), all
+    values 1.  `threshold` is the binarisation threshold when the rows come from equal_sparsity_device (else None)."""
+
+    def __init__(self, indptr, indices, n_cols, threshold=None):
+        self.indptr, self.indices, self.n_cols, self.threshold = indptr, indices, int(n_cols), threshold
+
+    @property
+    def shape(self):
+        return (self.indptr.shape[0] - 1, self.n_cols)
+
+    @property
+    def nnz(self):
+        return int(self.indices.shape[0])
+
+    def to_scipy(self, dtype=np.int64):
+        """scipy.sparse.csr_matrix of ones (default int64, like `(S >= thr).astype(int)`), copied through pinned host buffers with
+        one synchronisation.  Canonical: sorted indices, no duplicates."""
+        import scipy.sparse as sp
+        indptr = torch.empty(self.indptr.shape, dtype=torch.int64, pin_memory=True)
+        indices = torch.empty(self.indices.shape, dtype=torch.int32, pin_memory=True)
+        indptr.copy_(self.indptr, non_blocking=True)
+        indices.copy_(self.indices, non_blocking=True)
+        torch.cuda.current_stream(self.indptr.device).synchronize()
+        data = np.ones(self.nnz, dtype=dtype)
+        return sp.csr_matrix((data, indices.numpy(), indptr.numpy()), shape=self.shape)
+
+
+def _check_bits(bits, n_cols):
+    if not isinstance(bits, torch.Tensor):
+        raise TypeError(f"bits must be a torch.Tensor, got {type(bits).__name__}")
+    if bits.dtype != torch.int32 or bits.dim() != 2 or (bits.shape[1] > 1 and bits.stride(1) != 1):
+        raise ValueError("bits must be int32 [rows, words] with unit word stride")
+    if isinstance(n_cols, (bool, np.bool_)) or not isinstance(n_cols, (int, np.integer)):
+        raise TypeError(f"n_cols must be an int, got {n_cols!r}")
+    if not 1 <= int(n_cols) <= 2 ** 31 - 1:
+        raise ValueError(f"n_cols={n_cols} must lie in [1, 2^31 - 1]")
+    if bits.shape[1] < (int(n_cols) + 31) // 32:
+        raise ValueError(f"bits has {bits.shape[1]} words per row; {n_cols} columns need {(int(n_cols) + 31) // 32}")
+    if bits.device.type != "cuda":
+        raise _lib.SdrmError("packed_to_csr: bits must be a CUDA tensor (no CPU fallback)")
+
+
+def packed_to_csr(bits, n_cols, threshold=None):
+    """Bit-packed rows (sdrm_threshold_pack's layout: bit j of word w is column 32 w + j; bits at or past n_cols are ignored) ->
+    SparseRows on the same device, with kernel K10.  `bits` may be a row slice of a wider or longer matrix (any row stride)."""
+    _check_bits(bits, n_cols)
+    lib = _lib.load()
+    rows, n_cols = bits.shape[0], int(n_cols)
+    ld = bits.stride(0) if rows > 1 else bits.shape[1]
+    dev = bits.device
+    st = _lib.stream_ptr()
+    indptr = torch.empty(rows + 1, dtype=torch.int64, device=dev)
+    ws_bytes = lib.sdrm_packed_csr_workspace_bytes(rows)
+    ws = torch.empty(max(1, (ws_bytes + 7) // 8), dtype=torch.int64, device=dev)
+    _lib.check(lib.sdrm_packed_csr_indptr(_lib.ptr(bits), ld, rows, n_cols, _lib.ptr(indptr), _lib.ptr(ws), ws_bytes, st),
+               "sdrm_packed_csr_indptr")
+    nnz = int(indptr[-1].item())          # the only read-back: it sizes `indices`
+    indices = torch.empty(nnz, dtype=torch.int32, device=dev)
+    if nnz:
+        _lib.check(lib.sdrm_packed_csr_indices(_lib.ptr(bits), ld, rows, n_cols, _lib.ptr(indptr), _lib.ptr(indices), st),
+                   "sdrm_packed_csr_indices")
+    return SparseRows(indptr, indices, n_cols, threshold)
+
 
 def threshold_pack(scores, threshold, lower=False):
     """(S >= threshold) — or (S <= threshold) with lower=True — as a PackedMatrix (float32 or bfloat16 scores, compared as
