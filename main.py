@@ -49,6 +49,9 @@ def build_parser():
                    help="write each run's trained denoiser + VAE to DIR/run{n}_generator.pt (python -m sdrm_b200.synthesize reads it)")
     p.add_argument("--save-synthetic", type=str, default=None, metavar="DIR",
                    help="write each run's binarised synthetic rows to DIR/run{n}_{F-SDRM,M-SDRM,MultiVAE++}.npz (scipy sparse CSR)")
+    p.add_argument("--svd-on-gpu", action="store_true", default=False,
+                   help="--model svd: run the SVD evaluator's randomized SVD on the GPU from the binarised rows where they are "
+                        "(evaluators.compute_mf_results_gpu) instead of sklearn on dense host rows")
     return p
 
 
@@ -210,7 +213,11 @@ def main(argv=None):
             fid, fidelity_baseline = fidelity_audit({c: binarised[c] for c in COLS}, TRAIN_PARTIAL_VALID_DATA, fidelity_baseline)
             print(f"\nFidelity audit (run {run_n + 1}): synthetic rows against the training rows\n{fid.round(4).to_markdown()}")
         for name, frame in synth.items():
-            if model == "svd":
+            if model == "svd" and args.svd_on_gpu:
+                dense, packed = binarised[name]
+                rec, ndcg = evaluators.compute_mf_results_gpu(TRAIN_DATA, VALID_DATA, packed if packed is not None else dense,
+                                                              only_synthetic=args.augment_training_data)
+            elif model == "svd":
                 # NOTE: the flag is passed as only_synthetic=, exactly like the reference (main.py:189-194)
                 rec, ndcg = evaluators.compute_mf_results(TRAIN_DATA, VALID_DATA, synthetic_data=frame, nnmf=False,
                                                           only_synthetic=args.augment_training_data)

@@ -84,6 +84,9 @@ SIGNATURES = {
     "sdrm_packed_csr_workspace_bytes": (C.c_size_t, [C.c_int64]),
     "sdrm_packed_csr_indptr": (C.c_int, [_P, C.c_int64, C.c_int64, C.c_int, _P, _P, C.c_size_t, _P]),
     "sdrm_packed_csr_indices": (C.c_int, [_P, C.c_int64, C.c_int64, C.c_int, _P, _P, _P]),
+    "sdrm_spmm_binary_workspace_bytes": (C.c_size_t, [C.c_int64, C.c_int]),
+    "sdrm_spmm_binary": (C.c_int, [_P, _P, C.c_int64, C.c_int64, _P, C.c_int64, C.c_int, C.c_int64, _P, C.c_int64, _P, _P,
+                                   C.c_size_t, _P]),
 }
 
 

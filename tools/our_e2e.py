@@ -1,7 +1,9 @@
 """End-to-end quality run of THIS repo on the GPU: same loop, hyper-parameters and evaluator settings as tools/ref_e2e.py.
 
-  python tools/our_e2e.py [runs] [only_synth] [out] [json overrides] [--sampling-steps S] [--eta X]
---sampling-steps / --eta sample F-SDRM and M-SDRM on a fewer-step chain (sample_ddpm's sampling_steps / eta); default: all T steps."""
+  python tools/our_e2e.py [runs] [only_synth] [out] [json overrides] [--sampling-steps S] [--eta X] [--svd-on-gpu]
+--sampling-steps / --eta sample F-SDRM and M-SDRM on a fewer-step chain (sample_ddpm's sampling_steps / eta); default: all T steps.
+--svd-on-gpu scores with evaluators.compute_mf_results_gpu from the device bits instead of sklearn; each record names the
+evaluator that ran ("svd_evaluator")."""
 import json, os, sys, time
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, pandas as pd, torch
@@ -16,6 +18,9 @@ for flag, key, conv in (("--sampling-steps", "sampling_steps", int), ("--eta", "
         i = sys.argv.index(flag)
         GRID[key] = conv(sys.argv[i + 1])
         del sys.argv[i:i + 2]
+SVD_ON_GPU = "--svd-on-gpu" in sys.argv
+if SVD_ON_GPU:
+    sys.argv.remove("--svd-on-gpu")
 runs = int(sys.argv[1]) if len(sys.argv) > 1 else 5
 only_synth = (sys.argv[2] == "1") if len(sys.argv) > 2 else True
 out_path = sys.argv[3] if len(sys.argv) > 3 else "gpurun_out/e2e_ours_ml100k.jsonl"
@@ -35,7 +40,8 @@ for run in range(runs):
                            noise_divider=A["nd"], VAE_DIR_PATH="/tmp/our_temp_vae", TRAIN_PARTIAL_VALID_DATA=TPV, VALID_DATA=VALID,
                            OPTIMIZATION_OBJECTIVE="Recall@10", verbose=False)
     torch.cuda.synchronize()
-    res = {"impl": "sdrm_b200", "run": run, "train_s": round(time.time() - t0, 1), "only_synthetic": only_synth, **GRID}
+    res = {"impl": "sdrm_b200", "run": run, "train_s": round(time.time() - t0, 1), "only_synthetic": only_synth, **GRID,
+           "svd_evaluator": "compute_mf_results_gpu" if SVD_ON_GPU else "compute_mf_results"}
     t1 = time.time()
     from sdrm_b200.sparsify import equal_sparsity_device
     M = sample_ddpm(N_USERS, DIFF, VAE, A["L"], A["nd"], timesteps="random", n_timesteps=A["T"], **GRID)
@@ -51,8 +57,14 @@ for run in range(runs):
             assert pm.threshold == np.quantile(host.flatten(), SPARSITY) and (dense == (host >= pm.threshold)).all()
             syn = pd.DataFrame(dense)
         else:
+            pm = None
             syn = pd.DataFrame((S >= np.quantile(S.flatten(), SPARSITY)).astype(int))
-        rec, ndcg = evaluators.compute_mf_results(TRAIN, VALID, synthetic_data=syn, nnmf=False, only_synthetic=only_synth)
+        t1 = time.time()
+        if SVD_ON_GPU:
+            rec, ndcg = evaluators.compute_mf_results_gpu(TRAIN, VALID, pm if pm is not None else syn, only_synthetic=only_synth)
+        else:
+            rec, ndcg = evaluators.compute_mf_results(TRAIN, VALID, synthetic_data=syn, nnmf=False, only_synthetic=only_synth)
+        res[f"{name}_svd_s"] = round(time.time() - t1, 3)
         res[name] = {"recall@10": float(rec[3]), "ndcg@10": float(ndcg[3])}
     print(json.dumps(res), flush=True)
     with open(out_path, "a") as fh:
