@@ -52,6 +52,9 @@ def build_parser():
     p.add_argument("--svd-on-gpu", action="store_true", default=False,
                    help="--model svd: run the SVD evaluator's randomized SVD on the GPU from the binarised rows where they are "
                         "(evaluators.compute_mf_results_gpu) instead of sklearn on dense host rows")
+    p.add_argument("--binarise", choices=["equal-sparsity", "activity"], default="equal-sparsity",
+                   help="equal-sparsity: the reference's single global threshold; activity: every synthetic row keeps the number "
+                        "of interactions of a training user, at its highest scores (sparsify.activity_matched_device, on the GPU)")
     return p
 
 
@@ -73,6 +76,19 @@ def binarise(scores, sparsity):
         pm = equal_sparsity_device(scores.detach(), sparsity)
         return pm.numpy(int), pm
     return (scores >= np.quantile(scores.flatten(), sparsity)).astype(int), None
+
+
+def binarise_activity(scores, sparsity, activity):
+    """The activity-matched binarisation (sdrm_b200/sparsify.py activity_matched_device): rows ranked by their equal-sparsity
+    row sums take the training users' activities at the same quantile, at their highest scores.  Host arrays (VAE.sample) are
+    uploaded as float32.  Returns (dense 0/1 rows, the device PackedMatrix) like binarise."""
+    import torch
+
+    from sdrm_b200.sparsify import activity_matched_device
+    if not isinstance(scores, torch.Tensor):
+        scores = torch.as_tensor(np.asarray(scores, dtype=np.float32), device="cuda")
+    pm = activity_matched_device(scores.detach(), sparsity, activity)
+    return pm.numpy(int), pm
 
 
 AUDIT_COLS = ["DCR mean", "DCR p5", "DCR p50", "DCR p95", "exact copies", "copy share", "NNDR median"]
@@ -168,6 +184,16 @@ def main(argv=None):
     dl = DataLoader(ds, batch_size=1, collate_fn=sparse_batch_collate, generator=torch.Generator(device="cpu"),
                     sampler=sampler, shuffle=False)
 
+    if args.binarise == "activity":
+        from sdrm_b200.sparsify import row_activity
+        activity = row_activity(TRAIN_DATA)   # the N_USERS synthetic rows stand in for TRAIN_DATA's users
+
+        def binarise_run(scores, sparsity):
+            return binarise_activity(scores, sparsity, activity)
+    else:
+        def binarise_run(scores, sparsity):
+            return binarise(scores, sparsity)
+
     model = args.model.lower()
     results = {c: [] for c in COLS}
     audit_baseline = None
@@ -199,9 +225,9 @@ def main(argv=None):
                              n_timesteps=args.SDRM_timesteps, verbose=True,
                              sampling_steps=args.SDRM_sampling_steps, eta=args.SDRM_eta)
         binarised = {
-            "M-SDRM": binarise(M_SDRM, SPARSITY),
-            "F-SDRM": binarise(F_SDRM, SPARSITY),
-            "MultiVAE++": binarise(VAE.sample(N_USERS), SPARSITY),
+            "M-SDRM": binarise_run(M_SDRM, SPARSITY),
+            "F-SDRM": binarise_run(F_SDRM, SPARSITY),
+            "MultiVAE++": binarise_run(VAE.sample(N_USERS), SPARSITY),
         }
         synth = {name: pd.DataFrame(dense) for name, (dense, _) in binarised.items()}
         if args.save_synthetic:

@@ -41,6 +41,8 @@ SIGNATURES = {
     "sdrm_recall_ndcg_at_k": (C.c_int, [_P, C.c_int, C.c_int, _P, C.c_int64, C.c_int, C.c_int64, _P, _P, _P, _P]),
     "sdrm_recommend_topk": (C.c_int, [_P, C.c_int64, C.c_int, C.c_int64, _P, _P, C.c_int64, C.c_int, _P, _P, _P, _P]),
     "sdrm_recommend_topk_bf16": (C.c_int, [_P, C.c_int64, C.c_int, C.c_int64, _P, _P, C.c_int64, C.c_int, _P, _P, _P, _P]),
+    "sdrm_topk_pack": (C.c_int, [_P, C.c_int64, C.c_int, C.c_int64, _P, _P, C.c_int64, _P, _P, _P]),
+    "sdrm_topk_pack_bf16": (C.c_int, [_P, C.c_int64, C.c_int, C.c_int64, _P, _P, C.c_int64, _P, _P, _P]),
     "sdrm_noise_inputs": (C.c_int, [_P, _P, _P, C.c_int64, C.c_int, C.c_float, C.c_double, C.c_uint64, C.c_int64,
                                     _P, _P, _P, _P, _P, _P, _P, _P]),
     "sdrm_loss_stats": (C.c_int, [_P, _P, _P, _P, C.c_int64, C.c_double, _P, _P]),

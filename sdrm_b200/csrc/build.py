@@ -6,9 +6,9 @@ import sys
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB = os.path.join(HERE, "libsdrm_b200.so")
-SOURCES = ["errors.cu", "engine_host.cu", "engine_bf16.cu", "metrics.cu", "train_kernels.cu", "train_gemm.cu", "sparsify.cu", "recommend.cu", "privacy.cu", "fidelity.cu", "sparse_rows.cu", "svd.cu"]
+SOURCES = ["errors.cu", "engine_host.cu", "engine_bf16.cu", "metrics.cu", "train_kernels.cu", "train_gemm.cu", "sparsify.cu", "recommend.cu", "privacy.cu", "fidelity.cu", "sparse_rows.cu", "svd.cu", "row_select.cu"]
 HEADERS = ["ptx_sm100.cuh", "philox.cuh", "layer_engine.cuh", "layer_engine_kernel.cuh", "engine_launch.cuh", "gemm_x3_kernel.cuh", "small_chain_kernel.cuh", "host_util.h",
-           "../../include/sdrm_b200.h"]
+           "order_key.cuh", "../../include/sdrm_b200.h"]
 FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
     "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=default", "--expt-relaxed-constexpr",

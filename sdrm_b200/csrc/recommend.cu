@@ -17,6 +17,7 @@
 
 #include "../../include/sdrm_b200.h"
 #include "host_util.h"
+#include "order_key.cuh"
 
 namespace sdrm_rec {
 
@@ -26,19 +27,7 @@ constexpr int MAX_ITEMS = 1 << 20;  // bitmap of 128 KB of shared memory
 constexpr int UNROLL = 4;           // loads in flight per thread and pass
 static_assert(THREADS == 256, "one histogram bin per thread");
 
-// order-preserving unsigned image of a score: 32 bits for fp32, 16 for bf16 (kept as its raw bits)
-__device__ __forceinline__ uint32_t canonical_bits(float v) {
-  v = v + 0.0f;                          // -0.0 -> +0.0: equal scores must have equal keys
-  return __float_as_uint((v != v) ? -CUDART_INF_F : v);   // NaN ranks as -inf
-}
-__device__ __forceinline__ uint32_t score_ord(float x) {
-  const uint32_t u = canonical_bits(x);
-  return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
-}
-__device__ __forceinline__ uint32_t score_ord(uint16_t x) {
-  const uint32_t u = canonical_bits(__uint_as_float(static_cast<uint32_t>(x) << 16)) >> 16;   // (exact: bf16 is fp32's top half)
-  return (u & 0x8000u) ? (~u & 0xFFFFu) : (u | 0x8000u);
-}
+using sdrm_order::score_ord;   // order-preserving unsigned image of a score: 32 bits for fp32, 16 for bf16
 
 __device__ __forceinline__ void store_value(float* p, uint32_t o) {
   *p = __uint_as_float((o & 0x80000000u) ? (o & 0x7FFFFFFFu) : ~o);

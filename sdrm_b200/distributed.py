@@ -27,7 +27,7 @@ def shard_bounds(n, rank, world):
 
 def sample_ddpm_sharded(n_sample, diff_net, vae_net, diff_latent_dim, noise_divider=1.0, timesteps=None,
                         n_timesteps=None, *, seed, group=None, gather=False, sparsity=None, sampler=None, out_dtype=None,
-                        sampling_steps=None, eta=None):
+                        sampling_steps=None, eta=None, activity=None):
     """Each rank samples its contiguous block of the n_sample rows (same `seed` on every rank; the Philox streams are keyed
     by the global row id, so in full-resolution mode the union of the blocks is bit-identical to a single-GPU run).
 
@@ -49,10 +49,14 @@ def sample_ddpm_sharded(n_sample, diff_net, vae_net, diff_latent_dim, noise_divi
     return / gather bfloat16 blocks (half the NVLink bytes), and gather="bits" binarises the bfloat16 rows (sparsify.py: ties
     at the threshold can keep a few more ones than the float32 rows would).
     sampling_steps / eta choose a fewer-step chain (sample_ddpm); multi-resolution rows map their drawn t_j onto its grid.
+    activity (the real rows' sparsify.row_activity; gather="bits" / "csr" only): binarise with sparsify.activity_matched_device
+    instead of equal sparsity, so every synthetic row keeps a real row's number of ones; the bits do not depend on the world size.
     An empty block (more ranks than rows) is legal: the rank still takes part in the collectives."""
     import numpy as np
     if isinstance(gather, str) and gather == "csr" and sparsity is None:
         raise ValueError("gather='csr' needs the sparsity of the binarisation")
+    if activity is not None and not (isinstance(gather, str) and gather in ("bits", "csr")):
+        raise ValueError("activity-matched binarisation needs gather='bits' or gather='csr'")
     if sampler is None:
         from .train_SDRM import sample_ddpm as sampler
     rank = dist.get_rank(group) if dist.is_initialized() else 0
@@ -70,20 +74,18 @@ def sample_ddpm_sharded(n_sample, diff_net, vae_net, diff_latent_dim, noise_divi
                    n_timesteps=n_timesteps, seed=seed, row_offset=lo, **kw)
     if not gather or world == 1:
         if gather == "bits":
-            from .sparsify import equal_sparsity_device
-            return equal_sparsity_device(rows, sparsity), (0, n_sample)
+            return _binarise(rows, sparsity, activity, None), (0, n_sample)
         if gather == "csr":
-            from .sparsify import equal_sparsity_device
-            return equal_sparsity_device(rows, sparsity).to_sparse(), (0, n_sample)
+            return _binarise(rows, sparsity, activity, None).to_sparse(), (0, n_sample)
         return rows, (lo, hi)
     if gather == "csr":
-        return _gather_csr(rows, sparsity, n_sample, world, group), (0, n_sample)
+        return _gather_csr(rows, sparsity, activity, n_sample, world, group), (0, n_sample)
     cap = shard_bounds(n_sample, 0, world)[1]  # largest block
     if gather == "bits":
-        from .sparsify import PackedMatrix, equal_sparsity_device
+        from .sparsify import PackedMatrix
         if sparsity is None:
             raise ValueError("gather='bits' needs the sparsity of the binarisation")
-        pm = equal_sparsity_device(rows, sparsity, group=group if group is not None else dist.group.WORLD)   # (sparsify: None = one process)
+        pm = _binarise(rows, sparsity, activity, group if group is not None else dist.group.WORLD)   # (sparsify: None = one process)
         wpr = pm.bits.shape[1]
         padded = pm.bits.new_zeros((cap, wpr))
         padded[: hi - lo] = pm.bits
@@ -103,11 +105,19 @@ def sample_ddpm_sharded(n_sample, diff_net, vae_net, diff_latent_dim, noise_divi
     return out, (0, n_sample)
 
 
-def _gather_csr(rows, sparsity, n_sample, world, group):
-    """gather='csr' over `world` ranks: global-threshold binarisation and K10 on this rank's block, then two all_gathers (per-rank
-    nnz; indptr blocks and indices padded to the largest block) and the rebase of each indptr block by the nnz before it."""
-    from .sparsify import SparseRows, equal_sparsity_device
-    pm = equal_sparsity_device(rows, sparsity, group=group if group is not None else dist.group.WORLD)
+def _binarise(rows, sparsity, activity, group):
+    """Equal sparsity with the global threshold, or the activity-matched binarisation when `activity` is given."""
+    from .sparsify import activity_matched_device, equal_sparsity_device
+    if activity is not None:
+        return activity_matched_device(rows, sparsity, activity, group=group)
+    return equal_sparsity_device(rows, sparsity, group=group)
+
+
+def _gather_csr(rows, sparsity, activity, n_sample, world, group):
+    """gather='csr' over `world` ranks: global binarisation and K10 on this rank's block, then two all_gathers (per-rank nnz;
+    indptr blocks and indices padded to the largest block) and the rebase of each indptr block by the nnz before it."""
+    from .sparsify import SparseRows
+    pm = _binarise(rows, sparsity, activity, group if group is not None else dist.group.WORLD)
     local = pm.to_sparse()
     dev = local.indptr.device
     nnz = torch.tensor([local.nnz], dtype=torch.int64, device=dev)

@@ -18,6 +18,10 @@ are ranked and compared as float32 values, so the threshold is np.quantile(S.ast
 the bits are S >= thr.  The float32 key of a bfloat16 score has its low 16 bits fixed by the sign, so two histogram passes
 (11 + 5 bits) pin it instead of three.
 
+activity_matched_device is an opt-in alternative that gives every synthetic row a real row's number of interactions: the rows
+are ranked by their equal-sparsity row sums, take the real activities at the same quantile, and kernel K12 (`sdrm_topk_pack`)
+keeps each row's highest scores, reading each score from HBM once.
+
 No CPU fallback: a CPU tensor raises.
 """
 import ctypes as C
@@ -245,6 +249,19 @@ def _check_bits(bits, n_cols):
         raise _lib.SdrmError("packed_to_csr: bits must be a CUDA tensor (no CPU fallback)")
 
 
+def _packed_indptr(bits, n_cols):
+    """int64[rows + 1]: 0 and the running sum of the rows' popcounts (kernel K10's first half, no read-back)."""
+    lib = _lib.load()
+    rows = bits.shape[0]
+    ld = bits.stride(0) if rows > 1 else bits.shape[1]
+    indptr = torch.empty(rows + 1, dtype=torch.int64, device=bits.device)
+    ws_bytes = lib.sdrm_packed_csr_workspace_bytes(rows)
+    ws = torch.empty(max(1, (ws_bytes + 7) // 8), dtype=torch.int64, device=bits.device)
+    _lib.check(lib.sdrm_packed_csr_indptr(_lib.ptr(bits), ld, rows, int(n_cols), _lib.ptr(indptr), _lib.ptr(ws), ws_bytes,
+                                          _lib.stream_ptr()), "sdrm_packed_csr_indptr")
+    return indptr
+
+
 def packed_to_csr(bits, n_cols, threshold=None):
     """Bit-packed rows (sdrm_threshold_pack's layout: bit j of word w is column 32 w + j; bits at or past n_cols are ignored) ->
     SparseRows on the same device, with kernel K10.  `bits` may be a row slice of a wider or longer matrix (any row stride)."""
@@ -254,11 +271,7 @@ def packed_to_csr(bits, n_cols, threshold=None):
     ld = bits.stride(0) if rows > 1 else bits.shape[1]
     dev = bits.device
     st = _lib.stream_ptr()
-    indptr = torch.empty(rows + 1, dtype=torch.int64, device=dev)
-    ws_bytes = lib.sdrm_packed_csr_workspace_bytes(rows)
-    ws = torch.empty(max(1, (ws_bytes + 7) // 8), dtype=torch.int64, device=dev)
-    _lib.check(lib.sdrm_packed_csr_indptr(_lib.ptr(bits), ld, rows, n_cols, _lib.ptr(indptr), _lib.ptr(ws), ws_bytes, st),
-               "sdrm_packed_csr_indptr")
+    indptr = _packed_indptr(bits, n_cols)
     nnz = int(indptr[-1].item())          # the only read-back: it sizes `indices`
     indices = torch.empty(nnz, dtype=torch.int32, device=dev)
     if nnz:
@@ -361,3 +374,125 @@ def equal_sparsity_device(scores, sparsity, group=None, lower=False, host_walk=F
             return pm
     thr = quantile_host_walk(scores, q, group) if host_walk else quantile_device(scores, q, group)
     return threshold_pack(scores, thr, lower=lower)
+
+
+# --------------------------------------------------------------------------------------------------
+# activity-matched binarisation: every synthetic row gets a real row's number of interactions (kernel K12)
+# --------------------------------------------------------------------------------------------------
+MAX_TOPK_COLS = 1 << 20
+_BAD_K = 1   # enum sdrm_topk_pack_status
+
+
+def row_activity(real):
+    """int64[N] host array: the number of distinct columns of each real row that hold a stored value != 0 (explicit stored zeros
+    do not count, a repeated column counts once; fidelity.py's user_ones).  `real`: a scipy sparse matrix or dense rows."""
+    import scipy.sparse as sp
+    if sp.issparse(real):
+        coo = sp.coo_matrix(real)
+        nz = coo.data != 0
+        rows, cols = coo.row[nz].astype(np.int64), coo.col[nz].astype(np.int64)
+        cells = np.unique(rows * coo.shape[1] + cols)
+        return np.bincount(cells // coo.shape[1], minlength=coo.shape[0]).astype(np.int64)
+    dense = np.asarray(real)
+    if dense.ndim != 2:
+        raise ValueError(f"real rows must be 2-D, got shape {dense.shape}")
+    return (dense != 0).sum(axis=1).astype(np.int64)
+
+
+def activity_targets(row_counts, activity, n_cols=None):
+    """The number of ones every synthetic row keeps, on the device of `row_counts` (int64[M]).
+
+    Rows are ranked by (row_counts ascending, row index ascending) and row j of rank r_j takes a_((2 r_j + 1) N // (2 M)) of the
+    N real activities sorted ascending, so with M == N the targets are a permutation of `activity`.  Raises ValueError for an
+    empty activity, a negative one, or one above n_cols (when given)."""
+    c = torch.as_tensor(row_counts)
+    if c.dim() != 1:
+        raise ValueError(f"row_counts must be 1-D, got shape {tuple(c.shape)}")
+    a = torch.as_tensor(np.asarray(activity) if not isinstance(activity, torch.Tensor) else activity)
+    if a.dim() != 1 or a.numel() == 0:
+        raise ValueError("activity must be a non-empty 1-D array of per-user interaction counts")
+    if a.dtype.is_floating_point or a.dtype == torch.bool or a.is_complex():
+        raise ValueError(f"activity must hold integers, got {a.dtype}")
+    a = a.to(device=c.device, dtype=torch.int64)
+    lo, hi = torch.aminmax(a)
+    if int(lo) < 0:
+        raise ValueError("activity holds a negative count")
+    if n_cols is not None and int(hi) > int(n_cols):
+        raise ValueError(f"activity holds a count above the {int(n_cols)} items")
+    m, n = c.numel(), a.numel()
+    order = torch.argsort(c, stable=True)
+    rank = torch.empty_like(order)
+    rank[order] = torch.arange(m, dtype=order.dtype, device=c.device)
+    return torch.sort(a).values[((2 * rank + 1) * n) // (2 * m)]
+
+
+def topk_pack(scores, k):
+    """Row j keeps exactly k[j] ones, at its k[j] highest scores with ties to the lower item index (K7's order: NaN ranks as -inf,
+    -0.0 equals +0.0; bfloat16 scores rank as their float32 values): a PackedMatrix with threshold None, kernel K12.  `k`: one
+    integer per row (any integer dtype, host or device).  Raises ValueError when a k lies outside [0, items]; the check reads one
+    status word back, so the call synchronises with the current stream."""
+    _check(scores)
+    rows, n_cols = scores.shape
+    if not 1 <= n_cols <= MAX_TOPK_COLS:
+        raise ValueError(f"scores must have between 1 and {MAX_TOPK_COLS} items, got {n_cols}")
+    if rows > 1 and scores.stride(0) < n_cols:
+        raise ValueError("scores rows must not overlap (a row-strided view is fine); call .contiguous() first")
+    dev = scores.device
+    k = torch.as_tensor(k, device=dev)
+    if k.dim() != 1 or k.shape[0] != rows:
+        raise ValueError(f"k must hold one count per row ({rows}), got shape {tuple(k.shape)}")
+    if k.dtype.is_floating_point or k.dtype == torch.bool or k.is_complex():
+        raise ValueError(f"k must hold integers, got {k.dtype}")
+    k32 = k.to(torch.int64).clamp(-1, n_cols + 1).to(torch.int32).contiguous()   # out-of-range stays out of range
+    wpr = (n_cols + 31) // 32
+    bits = torch.empty((rows, wpr), dtype=torch.int32, device=dev)
+    count = torch.zeros(1, dtype=torch.int64, device=dev)
+    if rows == 0:
+        return PackedMatrix(bits, n_cols, None, count)
+    status = torch.zeros(1, dtype=torch.int32, device=dev)
+    lib = _lib.load()
+    with torch.cuda.device(dev):
+        entry = lib.sdrm_topk_pack_bf16 if _bf16(scores) else lib.sdrm_topk_pack
+        _lib.check(entry(_lib.ptr(scores), rows, n_cols, scores.stride(0) if rows > 1 else n_cols, _lib.ptr(k32), _lib.ptr(bits),
+                         wpr, _lib.ptr(count), _lib.ptr(status), _lib.stream_ptr()), "sdrm_topk_pack")
+        if int(status.item()) & _BAD_K:
+            raise ValueError(f"k must lie in [0, {n_cols}] (the number of items) in every row")
+    return PackedMatrix(bits, n_cols, None, count)
+
+
+def _gather_blocks(t, group):
+    """All ranks' 1-D blocks of `t` (unequal lengths allowed) concatenated in rank order, and this rank's offset."""
+    dist = _world(group)
+    n = torch.tensor([t.numel()], dtype=torch.int64, device=t.device)
+    sizes = [torch.empty_like(n) for _ in range(dist.get_world_size(group))]
+    dist.all_gather(sizes, n, group=group)
+    sizes = [int(s.item()) for s in sizes]
+    padded = t.new_zeros(max(1, max(sizes)))   # (NCCL gets at least one element)
+    padded[: t.numel()] = t
+    parts = [torch.empty_like(padded) for _ in sizes]
+    dist.all_gather(parts, padded, group=group)
+    rank = dist.get_rank(group)
+    return torch.cat([p[:s] for p, s in zip(parts, sizes)]), sum(sizes[:rank])
+
+
+def activity_matched_device(scores, sparsity, activity, group=None):
+    """Activity-matched binarisation: the model decides which rows are heavy and which items each row gets, `activity` (the real
+    rows' row_activity) decides how many.  c_j = row j's ones under equal_sparsity_device(scores, sparsity) (the reference's
+    global threshold), the rows ranked by c take activity_targets(c, activity) ones each, and topk_pack keeps each row's
+    highest scores.  With M rows and M == len(activity) the row sums are a permutation of `activity`.
+
+    With `group`, `scores` is this rank's row shard: the threshold is the global one, the per-rank counts are all-gathered, so
+    every rank ranks all rows alike and the bits do not depend on the number of ranks.  Returns a PackedMatrix whose threshold
+    is None (no single threshold exists)."""
+    _check(scores)
+    rows, n_cols = scores.shape
+    if not 1 <= n_cols <= MAX_TOPK_COLS:
+        raise ValueError(f"scores must have between 1 and {MAX_TOPK_COLS} items, got {n_cols}")
+    pm = equal_sparsity_device(scores, sparsity, group=group)
+    counts = torch.diff(_packed_indptr(pm.bits, n_cols))
+    if _world(group) is not None:
+        counts, lo = _gather_blocks(counts, group)
+    else:
+        lo = 0
+    k = activity_targets(counts, activity, n_cols)
+    return topk_pack(scores, k[lo: lo + rows])

@@ -2,11 +2,12 @@
 binarises them with the training data's equal-sparsity rule and writes the rows as a sparse CSR matrix (scipy .npz).
 
     python -m sdrm_b200.synthesize --generator G.pt --users N --out X.npz [--seed S] [--multi-resolution]
-        [--sampling-steps S] [--eta E] [--bf16] [--sparsity q]
+        [--sampling-steps S] [--eta E] [--bf16] [--sparsity q] [--activity-from REAL.npz]
     torchrun --nproc_per_node G -m sdrm_b200.synthesize ...      (rows sharded over G GPUs, NCCL set up from the environment)
 
 Every rank samples its block of rows and converts it to CSR on its GPU (sample_ddpm_sharded(gather="csr")); rank 0 writes the
-file.  The rows depend on the seed and the flags, not on the number of processes.
+file.  The rows depend on the seed and the flags, not on the number of processes.  --activity-from gives every synthetic user the
+number of interactions of a user of REAL.npz instead (sparsify.activity_matched_device).
 """
 import argparse
 import os
@@ -74,6 +75,9 @@ def build_parser():
     p.add_argument("--bf16", action="store_true", help="sample bfloat16 rows and binarise those")
     p.add_argument("--sparsity", type=float, default=None,
                    help="share of zeros of the binarised rows, in [0, 1]; default: the training data's, from the checkpoint")
+    p.add_argument("--activity-from", default=None, metavar="REAL.npz",
+                   help="scipy sparse matrix of real users x the generator's items: every synthetic user keeps as many items as a "
+                        "real user has (matched by rank of the equal-sparsity row sums), at its highest scores")
     return p
 
 
@@ -93,17 +97,33 @@ def parse_args(argv=None):
     return args
 
 
+def load_activity(path, n_items):
+    """row_activity of the scipy sparse matrix in `path`, which must have the generator's `n_items` columns."""
+    import scipy.sparse as sp
+
+    from .sparsify import row_activity
+    real = sp.load_npz(path)
+    if real.shape[1] != n_items:
+        raise ValueError(f"{path}: {real.shape[1]} items, the generator samples {n_items}")
+    if real.shape[0] < 1:
+        raise ValueError(f"{path} holds no users")
+    return row_activity(real)
+
+
 def synthesize(args, group=None):
     """Sample, binarise and gather args.users rows on this process's GPU (or this rank's share); returns (SparseRows, meta)."""
     from .distributed import sample_ddpm_sharded
     dev = torch.device("cuda", torch.cuda.current_device())
     diff, vae, meta = load_generator(args.generator, dev)
     sparsity = meta["sparsity"] if args.sparsity is None else args.sparsity
+    activity = None
+    if getattr(args, "activity_from", None):
+        activity = load_activity(args.activity_from, meta["vae_args"]["input_dim"])
     rows, _ = sample_ddpm_sharded(args.users, diff, vae, meta["sdrm_args"]["N_ITEMS"], meta["noise_divider"],
                                   timesteps="random" if args.multi_resolution else None, n_timesteps=meta["T"], seed=args.seed,
                                   group=group, gather="csr", sparsity=sparsity,
                                   out_dtype=torch.bfloat16 if args.bf16 else None,
-                                  sampling_steps=args.sampling_steps, eta=args.eta)
+                                  sampling_steps=args.sampling_steps, eta=args.eta, activity=activity)
     return rows, dict(meta, sparsity_used=sparsity)
 
 
@@ -127,8 +147,9 @@ def main(argv=None):
             mat = rows.to_scipy()
             sp.save_npz(args.out, mat)
             world = dist.get_world_size() if distributed else 1
+            thr = "none (activity-matched)" if rows.threshold is None else repr(float(rows.threshold))
             print(f"synthesize: {mat.shape[0]} users x {mat.shape[1]} items, nnz {mat.nnz} "
-                  f"({mat.nnz / max(1, mat.shape[0] * mat.shape[1]):.4%} ones), threshold {float(rows.threshold)!r}, "
+                  f"({mat.nnz / max(1, mat.shape[0] * mat.shape[1]):.4%} ones), threshold {thr}, "
                   f"sparsity {meta['sparsity_used']}, {world} GPU(s), {time.time() - start:.2f} s -> {args.out}", flush=True)
         if distributed:
             dist.barrier()

@@ -1,9 +1,12 @@
 """End-to-end quality run of THIS repo on the GPU: same loop, hyper-parameters and evaluator settings as tools/ref_e2e.py.
 
   python tools/our_e2e.py [runs] [only_synth] [out] [json overrides] [--sampling-steps S] [--eta X] [--svd-on-gpu]
+                         [--binarise {equal-sparsity,activity}]
 --sampling-steps / --eta sample F-SDRM and M-SDRM on a fewer-step chain (sample_ddpm's sampling_steps / eta); default: all T steps.
 --svd-on-gpu scores with evaluators.compute_mf_results_gpu from the device bits instead of sklearn; each record names the
-evaluator that ran ("svd_evaluator")."""
+evaluator that ran ("svd_evaluator").
+--binarise activity gives every synthetic row a training user's number of interactions (sparsify.activity_matched_device)
+instead of the equal-sparsity threshold; each record names the binarisation ("binarise")."""
 import json, os, sys, time
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, pandas as pd, torch
@@ -18,6 +21,13 @@ for flag, key, conv in (("--sampling-steps", "sampling_steps", int), ("--eta", "
         i = sys.argv.index(flag)
         GRID[key] = conv(sys.argv[i + 1])
         del sys.argv[i:i + 2]
+BINARISE = "equal-sparsity"
+if "--binarise" in sys.argv:
+    i = sys.argv.index("--binarise")
+    BINARISE = sys.argv[i + 1]
+    del sys.argv[i:i + 2]
+    if BINARISE not in ("equal-sparsity", "activity"):
+        sys.exit(f"--binarise must be equal-sparsity or activity, got {BINARISE}")
 SVD_ON_GPU = "--svd-on-gpu" in sys.argv
 if SVD_ON_GPU:
     sys.argv.remove("--svd-on-gpu")
@@ -41,7 +51,7 @@ for run in range(runs):
                            OPTIMIZATION_OBJECTIVE="Recall@10", verbose=False)
     torch.cuda.synchronize()
     res = {"impl": "sdrm_b200", "run": run, "train_s": round(time.time() - t0, 1), "only_synthetic": only_synth, **GRID,
-           "svd_evaluator": "compute_mf_results_gpu" if SVD_ON_GPU else "compute_mf_results"}
+           "svd_evaluator": "compute_mf_results_gpu" if SVD_ON_GPU else "compute_mf_results", "binarise": BINARISE}
     t1 = time.time()
     from sdrm_b200.sparsify import equal_sparsity_device
     M = sample_ddpm(N_USERS, DIFF, VAE, A["L"], A["nd"], timesteps="random", n_timesteps=A["T"], **GRID)
@@ -50,7 +60,12 @@ for run in range(runs):
     torch.cuda.synchronize(); res["sample_full_s"] = round(time.time() - t1, 4)
     V = VAE.sample(N_USERS)
     for name, S in (("F-SDRM", F), ("M-SDRM", M), ("MultiVAE++", V)):
-        if isinstance(S, torch.Tensor):   # K4: threshold identical to np.quantile, 1 bit per entry to the host
+        if BINARISE == "activity":
+            from sdrm_b200.sparsify import activity_matched_device, row_activity
+            S = S if isinstance(S, torch.Tensor) else torch.as_tensor(np.asarray(S, dtype=np.float32), device="cuda")
+            pm = activity_matched_device(S, SPARSITY, row_activity(TRAIN))
+            syn = pd.DataFrame(pm.numpy(int))
+        elif isinstance(S, torch.Tensor):   # K4: threshold identical to np.quantile, 1 bit per entry to the host
             pm = equal_sparsity_device(S, SPARSITY)
             dense = pm.numpy(int)
             host = S.cpu().numpy()
