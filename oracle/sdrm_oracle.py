@@ -41,11 +41,11 @@ def n_hidden_of(sd):
 
 def timestep_embedding(t, dim):
     half = dim // 2
-    freqs = torch.exp(-math.log(10_000) * torch.arange(start=0, end=half, dtype=torch.float32) / half)
+    freqs = torch.exp(-math.log(10_000) * torch.arange(start=0, end=half, dtype=torch.float32, device=t.device) / half)
     args = t[:, None].float() * freqs[None]
     emb = torch.cat([torch.cos(args), torch.sin(args)], dim=-1)
     if dim % 2:
-        emb = torch.cat([emb, torch.zeros(emb.shape[0], 1, dtype=emb.dtype)], dim=-1)   # (dim = 1: emb has no column to copy)
+        emb = torch.cat([emb, torch.zeros(emb.shape[0], 1, dtype=emb.dtype, device=emb.device)], dim=-1)   # (dim = 1: emb has no column to copy)
     return emb
 
 
@@ -176,8 +176,9 @@ def perturb_input(x, t, noise, ab_t):
 
 
 def training_loss(sd, mu, t, noise_scaled, keeps, T, mu_coef=0.1):
-    """Score-matching loss of one minibatch.  keeps = 3 dropout keep masks (pred, sx, psx); autograd-friendly."""
-    _, _, ab_t = make_schedule(T)
+    """Score-matching loss of one minibatch.  keeps = 3 dropout keep masks (pred, sx, psx); autograd-friendly.  Runs on the
+    device of its inputs (a float64 state_dict on the GPU is the oracle at shapes the CPU would take minutes over)."""
+    ab_t = make_schedule(T)[2].to(mu.device)
     x_pert = perturb_input(mu, t, noise_scaled, ab_t)
     pred = denoiser_forward(sd, x_pert, t, keeps[0])
     sx = denoiser_forward(sd, mu, t, keeps[1])

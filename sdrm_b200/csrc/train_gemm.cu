@@ -532,7 +532,9 @@ int sdrm_denoiser_bwd(const float* d_g_out, const float* d_out, const float* d_x
     table_grad_kernel<<<grid, 256, 0, st>>>(Gf, t.Wp, reinterpret_cast<const long long*>(d_order), reinterpret_cast<const long long*>(d_offsets), D, d_gTable, D); ++g_train_launches;
   }
   finish_sums_kernel<<<1, 32, 0, st>>>(slope_g, 1, d_ga0); ++g_train_launches;
-  if (nh > 0) finish_sums_kernel<<<1, 32, 0, st>>>(slope_g + 1, 1, d_gah); ++g_train_launches;
+  if (nh > 0) {
+    finish_sums_kernel<<<1, 32, 0, st>>>(slope_g + 1, 1, d_gah); ++g_train_launches;
+  }
   SDRM_CUDA(cudaGetLastError());
   return SDRM_OK;
 }
